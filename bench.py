@@ -37,6 +37,7 @@ ENV_ID = 'DroneHoverSimpleEnv-v0'
 METRIC = 'env-steps/sec'
 UNIT = 'env-steps/s'
 L2_BYTES = 126 * 1024 * 1024
+DUMP_BYTES = 60 * 1000 * 1000    # --dump-outputs: upper bound of the arrays written
 HBM_FALLBACK_GBS = 6650.0        # /opt/skills/guides/B200_PROFILING.md fallback
 
 
@@ -227,6 +228,21 @@ class Segment:
 
 def ring_slots(bytes_per_segment):
     return max(2, -(-2 * L2_BYTES // bytes_per_segment))
+
+
+def dump_outputs(seg, k, out_dir, max_bytes=DUMP_BYTES):
+    """Writes what segment `k` returned to its caller (obs [inner, S, D], reward / cost / terminated / truncated
+    [inner, S]) as out_dir/<name>.npy in float32, for a fixed, seeded sample of S environments (S as large as
+    `max_bytes` allows, all of them when they fit), so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    outs = seg.seg_outs[k % seg.n_ring]
+    inner, n, d = outs['obs'].shape
+    s = min(n, max(1, max_bytes // (inner * (d + 4) * 4)))
+    idx = torch.randperm(n, generator=torch.Generator().manual_seed(0))[:s].sort().values.to(outs['obs'].device)
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outs.items():
+        np.save(os.path.join(out_dir, name + '.npy'), t.index_select(1, idx).float().cpu().numpy())
 
 
 def time_device(env, seg, K, W, dist_ctx, sampler=None, per_step=1):
@@ -518,6 +534,9 @@ def run_gpu_arm(a):
     sampler = ClockSampler(ctx.local_rank)
     ms, launches = time_device(env, seg, a.steps, a.warmup, ctx, sampler, per_step=a.launches)
     clocks = sampler.stop()
+    if a.dump_outputs and ctx.rank == 0:
+        # the ring still holds the last launch of the timed window: the final `inner` env.steps of the last step
+        dump_outputs(seg, (a.warmup + a.steps) * a.launches - 1, a.dump_outputs)
     env_steps = a.steps * a.launches * a.inner * n * ctx.world
     value = env_steps / (ms * 1e-3)
 
@@ -640,7 +659,14 @@ def main():
     p.add_argument('--e2e-div', type=int, default=4, help='e2e leg times steps/e2e_div segments')
     p.add_argument('--large-envs', type=int, default=4 * 1024 * 1024)
     p.add_argument('--no-ppo-rollout', action='store_true', help='skip the configs[4] companion leg')
+    p.add_argument('--dump-outputs', metavar='DIR',
+                   help='after the timed steps, write what the last launch of the last step returned (obs, reward, cost, '
+                        'terminated, truncated of a fixed, seeded sample of environments) as DIR/<name>.npy, float32')
     a = p.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        p.error('--steps must be at least 1 and --warmup at least 0')
+    if a.dump_outputs and a.impl == 'reference':
+        p.error('--dump-outputs writes the outputs of the CUDA engine (--impl b200)')
     if a.impl == 'reference':
         run_reference_arm(a)
     else:

@@ -343,7 +343,7 @@ def _nccl_worker(rank, world, port, batches, ep, out_q):
     dist.destroy_process_group()
 
 
-@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two GPUs (gpurun --gpus 2)')
+@pytest.mark.skipif(torch.cuda.device_count() < 2, reason='needs two GPUs')
 def test_nccl_world2_running_stats_and_episode_stats():
     """The NCCL branch of OnlineMeanStd._avg and pdx_stats_combine behind one NCCL all-gather, world size 2,
     against the oracle -- the same expectations as the gloo test of tests/test_collector_oracle.py."""
