@@ -29,33 +29,22 @@
 // Global traffic per env-step is the rollout itself: observation row, action, value, log-probability,
 // reward, cost and the two flags.
 #include <cstdio>
-#include <cstdlib>
 #include "pdx_dispatch.cuh"
 #include "pdx_tc.cuh"
 #include "pdx_error.h"
 
-#ifndef PDX_COL_LEADER_WAIT
-// Tuning hooks (tools/build_variant.sh, tools/ab_collect.sh).  Both "lighter" synchronisations measured SLOWER on
-// configs[4] (1408 us with the barriers, 1419 us with leader-only waits, 1455 us with the counter release): the
-// barriers keep the four warps of a tile on the same instructions, and the loop body (159 KB of SASS) lives or dies
-// by instruction-cache sharing.  Also slower: keeping two 16-column tcgen05.ld chunks in flight in the epilogues
+// Measured slower on configs[4] (DESIGN.md §4): keeping two 16-column tcgen05.ld chunks in flight in the epilogues
 // (software prefetch of the next chunk, 1,508 vs 1,420 us) -- more live registers and code for a latency the other
-// tiles already cover.  Also slower: separate locks for the operand buffer X and the TMEM slot with one X buffer
-// per tile (X built while other tiles hold the slots, buffer released after layer 1, per-tile mbarriers): 1,470 vs
-// 1,400 us single TF32, 2,625 vs 2,295 us split TF32 -- every tile then queues for a slot at the same moment, where
-// the single lock staggers the tiles by itself.  Also slower (+1.2 %): skipping the actor's zero-weight hidden units in
-// the layer-3 dot products behind uniform branches.  No gain: the layer-3 dot products as packed FFMA2 (fma.rn.f32x2 with
-// a broadcast scalar: half the FMA instructions, same time).
-#define PDX_COL_LEADER_WAIT 0        // 1 = only the issuing warp waits at the hand-off barriers, the others arrive
-#endif
-#ifndef PDX_COL_NANOSLEEP
-#define PDX_COL_NANOSLEEP 40         // back-off of the slot spin in ns (200: +1 % kernel time)
-#endif
-#ifndef PDX_COL_COUNTER_RELEASE
-#define PDX_COL_COUNTER_RELEASE 0    // 1 = the tile's last warp out of the layer-2 epilogue releases the slot (no barrier)
-#endif
+// tiles already cover.  Separate locks for the operand buffer X and the TMEM slot with one X buffer per tile (X built
+// while other tiles hold the slots, buffer released after layer 1, per-tile mbarriers): 1,470 vs 1,400 us single
+// TF32, 2,625 vs 2,295 us split TF32 -- every tile then queues for a slot at the same moment, where the single lock
+// staggers the tiles by itself.  Skipping the actor's zero-weight hidden units in the layer-3 dot products behind
+// uniform branches (+1.2 %).  No gain: the layer-3 dot products as packed FFMA2 (fma.rn.f32x2 with a broadcast
+// scalar: half the FMA instructions, same time).
 
 namespace pdx {
+
+constexpr unsigned kSlotSpinNs = 40;         // back-off of the slot spin in ns (200: +1 % kernel time)
 
 struct CollectArgs {
   int32_t obs_dim, k1, act_dim, n_steps;
@@ -136,6 +125,9 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
   const int tile_threads = 32 * tile_warps;
   const int bar_id = 1 + tile;                                // named barrier of the tile (0 = __syncthreads)
   const bool leader_warp = wq == 0;
+  // Every warp of a tile waits at its hand-off barriers, although only the issuing warp needs the other warps' data:
+  // the barriers keep the tile's warps on the same instructions, and the loop body (159 KB of SASS) lives or dies by
+  // instruction-cache sharing (leader-only waits and a counter release of the slot measured slower, DESIGN.md §4)
 
   extern __shared__ __align__(128) unsigned char smem[];
   const ColSmem sp = collect_smem<X3>(K1, D, B >> 5);
@@ -144,7 +136,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
   uint32_t* slot_busy = reinterpret_cast<uint32_t*>(smem + 72);    // [kSlots]
   uint32_t* slot_phase = reinterpret_cast<uint32_t*>(smem + 80);   // [kSlots] parity of the slot's two mbarriers
   uint32_t* tile_info = reinterpret_cast<uint32_t*>(smem + 96);    // [4] slot | parity << 8 of the tile's current policy step
-  uint32_t* tile_done = reinterpret_cast<uint32_t*>(smem + 112);   // [4] warps of the tile that are through with the slot
+  uint32_t* tile_done = reinterpret_cast<uint32_t*>(smem + 112);   // [4] read by nothing: see the slot release
   float* act_std = reinterpret_cast<float*>(smem + 128);           // exp(log_std)[4], log_std[4]
   float2* norm = reinterpret_cast<float2*>(smem + sp.norm);        // [K1] (mean, 1 / (std + eps))
   float* common = reinterpret_cast<float*>(smem + sp.common);      // w3a[64][4], w3c[64], b3[16]
@@ -241,7 +233,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
     }
     StepCtx<T> sc;
     sc.state = state; sc.n = n; sc.i = i; sc.valid = valid; sc.lane = lane; sc.tid = tid; sc.B = B;
-    sc.row0 = my_row; sc.row1 = my_row; sc.stg = nullptr; sc.RS = D; sc.next_ap = nullptr; sc.acc_sum = acc_sum; sc.acc_ext = acc_ext; sc.NT = 1;
+    sc.row0 = my_row; sc.row1 = my_row; sc.stg = nullptr; sc.RS = D; sc.acc_sum = acc_sum; sc.acc_ext = acc_ext; sc.NT = 1;
     sc.fast2 = false; sc.latency = Mo::BULLET && c.use_latency; sc.any_fin = false;
     sc.bulk = ((reinterpret_cast<uintptr_t>(a.b.obs) | (uintptr_t)((uint64_t)n * D * sizeof(T))) & 15u) == 0 &&
               (((uint64_t)max((int64_t)0, min((int64_t)32, n - (i - lane))) * D * sizeof(T)) & 15u) == 0;
@@ -255,7 +247,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
 #pragma unroll
           for (int q = 0; q < Cfg::kSlots; ++q)
             if (s < 0 && atomicCAS(&slot_busy[q], 0u, 1u) == 0u) s = q;
-          if (s < 0) { __nanosleep(PDX_COL_NANOSLEEP); if (it > (1u << 24)) __trap(); }
+          if (s < 0) { __nanosleep(kSlotSpinNs); if (it > (1u << 24)) __trap(); }
         }
         __threadfence_block();
         tile_info[tile] = (uint32_t)s | (slot_phase[s] << 8);
@@ -312,8 +304,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
         if (X3) *reinterpret_cast<float4*>(xl + kc * kLboA + row * 16) = make_float4(lo[0], lo[1], lo[2], lo[3]);
       }
       fence_async_smem();                                      // generic-proxy writes of X -> visible to the tensor core
-      // only the issuing warp waits for the tile's rows; the others go on to their Gaussian draws
-      if (leader_warp || !PDX_COL_LEADER_WAIT) named_bar_sync(bar_id, tile_threads); else named_bar_arrive(bar_id, tile_threads);
+      named_bar_sync(bar_id, tile_threads);
       // ---- layer 1: D1[128 x 128] = X . B1 (columns 0..63 actor, 64..127 critic)
       if (leader_warp) {
         constexpr uint32_t idesc = make_idesc(kN1);
@@ -364,7 +355,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
       }
       tmem_wait_st();
       tc_fence_before();
-      if (leader_warp || !PDX_COL_LEADER_WAIT) named_bar_sync(bar_id, tile_threads); else named_bar_arrive(bar_id, tile_threads);
+      named_bar_sync(bar_id, tile_threads);
       // ---- layer 2: D2[:, 0:64] = a2[:, 0:64] . B2a, D2[:, 64:128] = a2[:, 64:128] . B2c (A from TMEM)
       if (leader_warp) {
         tc_fence_after();
@@ -423,15 +414,10 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
         }
       }
       tc_fence_before();
-#if !PDX_COL_COUNTER_RELEASE
       named_bar_sync(bar_id, tile_threads);
-      if (leader_warp && lane == 0) {
-#else
-      __syncwarp();
-      if (lane == 0 && atomicAdd(&tile_done[tile], 1u) == (uint32_t)tile_warps - 1u) {
-#endif
-        // the tile's last warp to have read its D2 rows gives the slot back (no barrier: the others are on their way
-        // into env.step)
+      if (leader_warp && lane == 0) {                          // every warp of the tile has read its D2 rows: slot back
+        // tile_done has no reader.  Its two stores stay because without them ptxas allocates the loop's registers
+        // differently, and k_collect measured 0.8 % (single TF32) and 1.2 % (split TF32) slower on a B200 (1,000 W).
         tile_done[tile] = 0u;
         slot_phase[slot] = par ^ 1u;
         __threadfence_block();
@@ -523,7 +509,6 @@ static cudaError_t launch_collect(const KArgs<float>& ka, CollectArgs& p, int sm
   int warps = (int)((per_cta + 31) / 32);
   if (warps < 1) warps = 1;
   if (warps > max_warps) warps = max_warps;
-  if (const char* e = getenv("PDX_COLLECT_WARPS")) { const int wv = atoi(e); if (wv >= 1 && wv <= 16) warps = wv; }   // tuning hook
   p.warps_per_cta = warps;
   p.groups = (int32_t)((n + (int64_t)warps * 32 - 1) / ((int64_t)warps * 32));
   const ColSmem sp = collect_smem<X3>(p.k1, ka.c.obs_dim, warps);

@@ -68,16 +68,11 @@ static void fill_devcfg(const PdxConfig& p, DevCfg<T>& d) {
 struct LaunchShape { int block, tiles; size_t smem; };
 template <class T>
 static LaunchShape pick_shape(int D, int E, int wmode) {
-  int forced = 0;
-  if (const char* e = getenv("PDX_BLOCK")) {          // tuning hook: 32 / 64 / 128 / 256
-    const int b = atoi(e);
-    if (b >= 32 && b <= kMaxBlock && b % 32 == 0) forced = b;
-  }
   LaunchShape best{0, 0, 0};
   int best_warps = -1;
   const int blocks[3] = {128, 64, 32};
   for (int bi = 0; bi < 3; ++bi) {
-    const int block = forced ? forced : blocks[bi];
+    const int block = blocks[bi];
     for (int tiles = 2; tiles >= 1; --tiles) {
       const size_t smem = rollout_smem_bytes<T>(block, D, tiles, E, wmode);
       if (smem > (size_t)227 * 1024) continue;
@@ -86,7 +81,6 @@ static LaunchShape pick_shape(int D, int E, int wmode) {
       const int warps = (by_smem < by_regs ? by_smem : by_regs) * (block / 32);
       if (warps > best_warps) { best_warps = warps; best = LaunchShape{block, tiles, smem}; }
     }
-    if (forced) break;
   }
   return best;
 }
@@ -107,7 +101,9 @@ static cudaError_t launch_kind(int kind, const KArgs<T>& ka, cudaStream_t st) {
   typedef Model<T, TASK, PHYS, NOISE, RNG, PID> Mo;
   constexpr bool quad_ok = sizeof(T) == 4 && Mo::E % 4 == 0 && Mo::C % 4 == 0;
   int wmode = (ka.c.obs_dim & 15) == 0 ? (quad_ok ? 2 : 1) : 0;
-  if (const char* e = getenv("PDX_WMODE")) {          // tuning hook: force mode 1 or 2 where legal
+  // PDX_WMODE forces mode 1 or 2 where legal: the tests run mode 1 as the reference of mode 2, switching the
+  // variable between two environments of one process (so it is read per launch)
+  if (const char* e = getenv("PDX_WMODE")) {
     const int wv = atoi(e);
     if (wmode && (wv == 1 || (wv == 2 && quad_ok))) wmode = wv;
   }
@@ -135,10 +131,9 @@ static cudaError_t launch_kind(int kind, const KArgs<T>& ka, cudaStream_t st) {
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  static const int pdl = getenv("PDX_PDL") ? atoi(getenv("PDX_PDL")) : 3;     // tuning hook: bit 0 = this kernel
   // opt-in per call (PDX_BUF_STATE_STABLE): measured, early launch of this kernel AND of a one-CTA-per-SM
   // tensor-core policy kernel around it collapses throughput (profiles/r1_summary.md), so the caller decides
-  lc.attrs = attr; lc.numAttrs = ((pdl & 1) && (ka.b.flags & PDX_BUF_STATE_STABLE)) ? 1 : 0;
+  lc.attrs = attr; lc.numAttrs = (ka.b.flags & PDX_BUF_STATE_STABLE) ? 1 : 0;
   return cudaLaunchKernelEx(&lc, kern, kb);
 }
 

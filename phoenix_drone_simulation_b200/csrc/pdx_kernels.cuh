@@ -16,23 +16,6 @@
 #pragma once
 #include "pdx_model.cuh"
 
-#ifndef PDX_FAST2
-#define PDX_FAST2 1
-#endif
-#ifndef PDX_ACT_PREFETCH
-// next step's action: 1 = its line is prefetched into L2 at the head of the step, 2 = into L1 (+ the one after into
-// L2), 3 = into L1, 4 = loaded into registers just before the package vote.  Measured on one box (tools/ab_variants.sh):
-// 1, 3 and 4 the same (10.20 G env-steps/s), 2 -1 %, none -2 %: at 3.5 warps per scheduler a warp's own stall is
-// covered by the others or not at all
-#define PDX_ACT_PREFETCH 1
-#endif
-#ifndef PDX_PREFETCH
-#define PDX_PREFETCH 1
-#endif
-#ifndef PDX_FLUSH_INLINE
-#define PDX_FLUSH_INLINE __forceinline__
-#endif
-
 namespace pdx {
 
 constexpr int kMaxBlock = 512;     // threads per block are chosen at run time (<= kMaxBlock)
@@ -634,8 +617,6 @@ struct StepCtx {
   T* row0; T* row1;           // this thread's row in the two observation tiles (row1 == row0 with one tile)
   T* stg;                     // column-major staging buffer of the warp (WIDE == 1 only)
   int RS;                     // words between the rows of two neighbouring lanes in a tile
-  const float4* next_ap;      // k_rollout: where this thread's action of the NEXT step is (nullptr: none) ...
-  float4 a_next;              // ... loaded into here just before the package vote (see rollout_step)
   double* acc_sum; T* acc_ext;
   int NT;                     // observation tiles (1 or 2)
   bool fast2, bulk, latency, any_fin;
@@ -788,13 +769,8 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
             const char* pk = reinterpret_cast<const char*>(
                 package_ptr<Mo>(state, n, i, H, (((int)w[L.ep_index] >> 4) + 1) & (kPackSlots - 1)));
 #pragma unroll
-            for (int b = 0; b < (int)(L.pack_quads * 4 * sizeof(T)) + 127; b += 128) {
-#if PDX_PREFETCH == 1
-              asm volatile("prefetch.global.L1 [%0];" ::"l"(pk + b));
-#elif PDX_PREFETCH == 2
-              asm volatile("prefetch.global.L2 [%0];" ::"l"(pk + b));
-#endif
-            }
+            for (int b = 0; b < (int)(L.pack_quads * 4 * sizeof(T)) + 127; b += 128)
+              asm volatile("prefetch.global.L1 [%0];" ::"l"(pk + b));     // (into L1: this lane reads them itself)
           }
         }
       }
@@ -1008,11 +984,6 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
       const int ew = (int)w[L.ep_index], e0 = ew >> 4, pend0 = ew & 15;
       const int total = (int)__reduce_add_sync(full, (unsigned)__popc(pend0));     // pending packages of the warp
       const bool urgent = (pend0 >> ((e0 + 1) & (kPackSlots - 1))) & 1;
-#if PDX_ACT_PREFETCH == 4
-      // next step's action: requested here, so that its L2 latency runs under the vote barrier and the row copy
-      // instead of at the head of the next step (four registers, live across the tail of the step only)
-      if (sc.next_ap) sc.a_next = *sc.next_ap;
-#endif
       if (vote(urgent || total >= 40)) {
         if (valid) m.store(state, n, i, true);             // the state is parked in its own planes around the
         // generator: nothing is live across it (inlined on top of the live state it spilled on the hot path)
@@ -1107,7 +1078,7 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
   // H = 2 with two tiles (the common case): the newest entry of a row is also the oldest entry of the NEXT
   // row, so every entry is written twice -- into this step's tile and into the next step's -- instead of
   // being read back and shifted (17 LDS + their latency at the head of every step)
-  const bool fast2 = PDX_FAST2 && !wide && H == 2 && NT == 2;
+  const bool fast2 = !wide && H == 2 && NT == 2;
   if (valid) {
     m.load(state, n, i);
     // history slots -> entries 1..H-1 of the "previous row" (tile1 plays the old tile at t = 0);
@@ -1129,7 +1100,6 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
   }
   StepCtx<T> sc;
   sc.state = state; sc.n = n; sc.i = i; sc.valid = valid; sc.lane = lane; sc.tid = tid; sc.B = B;
-  sc.next_ap = nullptr; sc.a_next = make_float4(0.f, 0.f, 0.f, 0.f);
   sc.row0 = my_row0; sc.row1 = my_row1; sc.stg = stg; sc.RS = RS; sc.acc_sum = acc_sum; sc.acc_ext = acc_ext; sc.NT = NT;
   sc.fast2 = fast2; sc.latency = Mo::BULLET && c.use_latency; sc.any_fin = false;
   // observation rows leave as one bulk copy per warp and step when the destination meets the 16-byte
@@ -1139,25 +1109,13 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
 
   for (int t = 0; t < a.n_steps; ++t) {
     // this step's action; the line of step t+1's action is requested now (prefetch: no register is held
-    // across the step), so that an L2/HBM miss does not sit at the head of the next step's dependency chain
+    // across the step), so that an L2/HBM miss does not sit at the head of the next step's dependency chain.
+    // Into L2: L1 prefetches and a register preload measured no faster, no prefetch 2 % slower (DESIGN.md §4)
     float4 a4 = make_float4(0.f, 0.f, 0.f, 0.f);
     if (valid) {
       const float4* ap = reinterpret_cast<const float4*>(a.actions) + (int64_t)t * n + i;
-#if PDX_ACT_PREFETCH == 4
-      a4 = (t == 0 || RNG != PDX_RNG_PHILOX) ? *ap : sc.a_next;
-      sc.next_ap = t + 1 < a.n_steps ? ap + n : nullptr;
-      if (t + 2 < a.n_steps) asm volatile("prefetch.global.L2 [%0];" ::"l"(ap + 2 * n));
-#else
       a4 = *ap;
-#endif
-#if PDX_ACT_PREFETCH == 1
       if (t + 1 < a.n_steps) asm volatile("prefetch.global.L2 [%0];" ::"l"(ap + n));
-#elif PDX_ACT_PREFETCH == 2
-      if (t + 1 < a.n_steps) asm volatile("prefetch.global.L1 [%0];" ::"l"(ap + n));
-      if (t + 2 < a.n_steps) asm volatile("prefetch.global.L2 [%0];" ::"l"(ap + 2 * n));
-#elif PDX_ACT_PREFETCH == 3
-      if (t + 1 < a.n_steps) asm volatile("prefetch.global.L1 [%0];" ::"l"(ap + n));
-#endif
     }
     // Package regeneration is voted per BLOCK: all warps of a block run the (long) generator at the same
     // step, and the barrier keeps them within one step of each other -- the step is ~30 KB of straight-line

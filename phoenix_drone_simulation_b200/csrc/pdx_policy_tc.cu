@@ -36,7 +36,6 @@
 // three times the (cheap) MMA cost, which is what the parity tests pin against torch.
 #include <cuda_runtime.h>
 #include <cstdint>
-#include <cstdlib>
 #include <cstdio>
 #include "../../include/phoenix_b200.h"
 #include "pdx_error.h"
@@ -652,8 +651,7 @@ extern "C" int pdx_policy_step_tc(int64_t n, int32_t obs_dim, const float* obs, 
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
-  static const int pdl = getenv("PDX_PDL") ? atoi(getenv("PDX_PDL")) : 3;     // tuning hook: bit 1 = this kernel
-  lc.attrs = attr; lc.numAttrs = (pdl & 2) ? 1 : 0;
+  lc.attrs = attr; lc.numAttrs = 1;
   const cudaError_t le = x3 ? cudaLaunchKernelEx(&lc, k_policy_tc<true>, a) : cudaLaunchKernelEx(&lc, k_policy_tc<false>, a);
   if (le != cudaSuccess) { cudaGetLastError(); return pdx::set_error(PDX_ERR_CUDA, cudaGetErrorString(le)); }
   return tc_status("pdx_policy_step_tc");

@@ -16,7 +16,6 @@ Cross-GPU traffic: two small all-reduces per rollout for the episode statistics 
 `OnlineMeanStd.update` -- nothing on the env.step itself (SURVEY.md 8e).
 """
 import ctypes as C
-import os
 import math
 
 import torch
@@ -474,7 +473,6 @@ class RolloutCollector:
         self.fused_used = False                # did the last collect() run through pdx_collect?
         self._final_obs_T = None               # [T, N, D], only when truncations can occur inside a rollout
         self._obs_moments = None
-        self.moments_in_kernel = os.environ.get('PDX_COLLECT_MOMENTS', '1') != '0'   # tuning hook: 0 = separate pass (k_moments)
 
     def _fused(self, generator=None):
         return (self.ac.fused and generator is None and self.env.dtype == torch.float32
@@ -548,7 +546,7 @@ class RolloutCollector:
             self._scratch = torch.empty(int(L.pdx_collect_scratch_bytes(env.device.index)), dtype=torch.uint8, device=env.device)
         out.scratch, out.scratch_bytes = p(self._scratch), self._scratch.numel()
         self._obs_moments = None
-        if oms is not None and self.moments_in_kernel:   # the running-statistics sums of the rollout, accumulated in-kernel
+        if oms is not None:                        # the running-statistics sums of the rollout, accumulated in-kernel
             self._obs_moments = (torch.zeros(2 * env.obs_dim, dtype=torch.float64, device=env.device), oms.mean.clone())
             out.obs_moments = p(self._obs_moments[0])
         rc = L.pdx_collect(C.byref(env.pdx), C.byref(buf), C.byref(pol), C.byref(out), env.seed, env._counter + 1, stream)

@@ -20,5 +20,5 @@ for n in [int(x) for x in sys.argv[3].split(',')]:
         e1.record()
         torch.cuda.synchronize()
         ms = e0.elapsed_time(e1) / 3
-        print(json.dumps({'env': env_id, 'k': kernel, 'fused': col.fused_used, 'n': n, 'T': T, 'ms': round(ms, 3), 'Gsteps': round(T * n / ms / 1e6, 3), 'warps': os.environ.get('PDX_COLLECT_WARPS')}), flush=True)
+        print(json.dumps({'env': env_id, 'k': kernel, 'fused': col.fused_used, 'n': n, 'T': T, 'ms': round(ms, 3), 'Gsteps': round(T * n / ms / 1e6, 3)}), flush=True)
         del env, ac, col
