@@ -501,7 +501,10 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
 
 template <int TASK, int PHYS, bool X3>
 static cudaError_t launch_collect(const KArgs<float>& ka, CollectArgs& p, int sms, cudaStream_t st) {
-  const int max_warps = 14;
+  // at most 14 warps, and no more than the shared-memory plan admits: wide rows with the split-TF32 images leave
+  // room for fewer (D = 40: 10 warps, D = 60: 3) -- the shard then takes more passes
+  int max_warps = 14;
+  while (max_warps > 1 && collect_smem<X3>(p.k1, ka.c.obs_dim, max_warps).total > (size_t)227 * 1024) --max_warps;
   const int64_t n = ka.b.n_envs;
   // passes and warps per CTA: the fewest passes that fit, then the smallest CTA that covers the shard in them
   int64_t passes = (n + (int64_t)sms * max_warps * 32 - 1) / ((int64_t)sms * max_warps * 32);

@@ -610,7 +610,8 @@ class RolloutCollector:
             # truncates when an episode reaches max_episode_steps, i.e. not before step `limit`
             if (not self.reset_each_rollout) or t + 1 >= limit or env.cfg.reset_on_nonfinite:
                 self.boot[t] = ac.value(env.final_obs) * self.trunc[t].float()
-        return self._finish(ac.value(self.obs[T]))
+        self.last_val.copy_(ac.value(self.obs[T]))          # as pdx_collect does: last_val is the cut's bootstrap on both paths
+        return self._finish(self.last_val)
 
     def _finish(self, last_val):
         env, ac, T = self.env, self.ac, self.T

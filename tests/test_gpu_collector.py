@@ -11,6 +11,7 @@ import pytest
 import torch
 
 from oracle import collector_oracle as co
+import tf32_reference as tfr
 
 pytestmark = pytest.mark.gpu
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden_collector')
@@ -84,15 +85,40 @@ def test_online_mean_std_on_device_matches_reference(name):
     np.testing.assert_allclose(oms(_cuda(g['probe'])).cpu().numpy(), g['forward'], rtol=1e-4, atol=1e-5)
 
 
+# k_policy_tc with single-TF32 operands (it rounds X and the hidden activations to nearest itself) against the
+# float64 model of those operands (tests/tf32_reference.py), |got - model| / (1 + |model|) for the mean; the value
+# adds the tanh.approx bound of its layer-2 activations per row.  Measured on a B200 (1,000 W): mean at most 1.3e-4
+# (2.4e-7 on the check-sum networks), value at most 3.4e-4 inside the tanh bound.  Tolerances: about 4x.
+TF32_RNA_MU = 6e-4
+TF32_RNA_V = 2e-4
+
+
+def _net_layers(net):
+    return [(m.weight.detach().cpu().numpy(), m.bias.detach().cpu().numpy()) for m in net if isinstance(m, torch.nn.Linear)]
+
+
+def _check_single_tf32(ac, obs, mu, val, label):
+    oms = ac.obs_oms
+    mean, std = (oms.mean.cpu().numpy(), oms.std.cpu().numpy()) if oms is not None else (None, None)
+    mu_m, v_m, terms = tfr.forward(obs.cpu().numpy(), mean, std, oms.eps if oms is not None else 0.0,
+                                   _net_layers(ac.pi), _net_layers(ac.v), 'rna')
+    n_out = mu_m.shape[1]
+    e_mu = float((np.abs(mu[:, :n_out].double().cpu().numpy() - mu_m) / (1 + np.abs(mu_m))).max())
+    e_v = float((np.abs(val.double().cpu().numpy() - v_m) - tfr.tanh_bound(terms)).max())
+    print(f'single TF32 {label}: mean vs model {e_mu:.2e}, value vs model beyond the tanh bound {e_v:.2e}')
+    assert e_mu <= TF32_RNA_MU and e_v <= TF32_RNA_V, (label, e_mu, e_v)
+    return mu_m
+
+
 @pytest.mark.parametrize('kernel', ['cuda', 'tc', 'tc_tf32'])
 def test_fused_policy_step_matches_torch_modules(kernel):
     """pdx_policy_step / pdx_policy_step_tc (standardise + actor MLP + critic MLP + sample + log-prob in
     one kernel) against the torch modules that own the weights.  'cuda' = CUDA-core float32 kernel and
     'tc' = tcgen05 tensor-core kernel with split-TF32 operands: tolerance 2e-5 abs on mean / value;
-    'tc_tf32' = single TF32 rounding of the operands: 1e-2 abs (its documented precision)."""
+    'tc_tf32' = single TF32 rounding of the operands: against the model of those operands (_check_single_tf32)."""
     from phoenix_drone_simulation_b200.rollout import ActorCritic
     torch.manual_seed(1)
-    tol = dict(rtol=1e-4, atol=2e-5) if kernel != 'tc_tf32' else dict(rtol=1e-2, atol=1e-2)
+    tol = dict(rtol=1e-4, atol=2e-5)                    # (single TF32 goes through _check_single_tf32)
     # (160, ...) is outside the tensor-core shared-memory plan: ActorCritic falls back to the CUDA-core kernel
     for obs_dim, pi_h, v_h, n in ((34, (50, 50), (64, 64), 5000), (160, (64, 64), (64, 32), 777), (17, (8, 50), (3, 64), 256),
                                   (40, (64, 64), (64, 64), 128 * 300 + 1), (48, (50, 50), (64, 64), 127)):
@@ -106,8 +132,11 @@ def test_fused_policy_step_matches_torch_modules(kernel):
         ac.step_into(obs, act, val, logp, mu)
         assert ac.tc_precision == ({'cuda': 0, 'tc': 3, 'tc_tf32': 1}[kernel] if obs_dim <= 64 else 0)
         o = ac.obs_oms(obs)
-        torch.testing.assert_close(mu, ac.pi(o), **tol)
-        torch.testing.assert_close(val, ac.v(o).squeeze(-1), **tol)
+        if ac.tc_precision == 1:
+            _check_single_tf32(ac, obs, mu, val, f'D={obs_dim} pi {pi_h} v {v_h}')
+        else:
+            torch.testing.assert_close(mu, ac.pi(o), **tol)
+            torch.testing.assert_close(val, ac.v(o).squeeze(-1), **tol)
         std = torch.exp(ac.log_std)
         ref_logp = torch.distributions.Normal(mu, std).log_prob(act).sum(-1)
         torch.testing.assert_close(logp, ref_logp, rtol=1e-4, atol=1e-4)
@@ -389,13 +418,22 @@ def test_policy_kernels_reproduce_reference_check_sums(kernel, tol):
     equal the file's check_sum (utils/export.py:47-53, utils/utils.py:324-330).  All three policy kernels
     (CUDA-core float32, tcgen05 split-TF32, tcgen05 single TF32) on six reference-exported networks
     (D = 40, 50-50 relu).  Tolerance: float32 kernels 1e-5 abs + 1e-5 rel (the reference computed the sum
-    in float32); single TF32 5e-3 (its documented operand rounding)."""
-    from phoenix_drone_simulation_b200.policy_io import verify_check_sum
+    in float32); single TF32 5e-3 against the check_sum (its operand rounding) and TF32_RNA_MU against the model
+    of its operands."""
+    from phoenix_drone_simulation_b200.policy_io import load_policy_json, verify_check_sum
     files = sorted(f for f in os.listdir(KAT_DIR) if f.endswith('.json'))
     assert len(files) == 6
     for f in files:
         got, exp = verify_check_sum(os.path.join(KAT_DIR, f), device='cuda', policy_kernel=kernel, rtol=tol, atol=tol)
         print(f'{f} [{kernel}]: kernel {got:.6f} vs check_sum {exp:.6f}')
+        if kernel == 'tc_tf32':                   # the same network(ones) against the model of its TF32 operands
+            ac = load_policy_json(os.path.join(KAT_DIR, f), device='cuda', standardize=False, policy_kernel=kernel)
+            ones = torch.ones((128, ac.pi.net[0].in_features), device='cuda')
+            act = torch.empty((128, 4), device='cuda'); val = torch.empty(128, device='cuda')
+            logp = torch.empty(128, device='cuda'); mu = torch.empty((128, 4), device='cuda')
+            ac.step_into(ones, act, val, logp, mu)
+            mu_m = _check_single_tf32(ac, ones, mu, val, f)
+            assert abs(got - float(mu_m[0].sum())) <= TF32_RNA_MU * (1 + abs(got)), (f, got, float(mu_m[0].sum()))
 
 
 @pytest.mark.parametrize('env_id,kernel,N,T', [('DroneHoverBulletEnv-v0', 'tc', 5000, 24), ('DroneHoverBulletEnv-v0', 'tc_tf32', 5000, 24),
