@@ -34,6 +34,14 @@ struct KArgs {
   int n_tiles;      // 2: observation tiles double buffered; 1: one tile, shifted in place
 };
 
+// The ep_index word (pdx_layout.h): uint32_t (e << 4) | pend.  float64 keeps the integer's value (exact below
+// 2^53), float32 the bit pattern: a float value would stop holding 16 e + pend exactly at e = 2^20 and lose
+// pending bits.  e counts modulo 2^28 (kEpMask) everywhere: here, in the package keys and in the tape path.
+__device__ __forceinline__ uint32_t ep_word(const float& w) { return __float_as_uint(w); }
+__device__ __forceinline__ uint32_t ep_word(const double& w) { return (uint32_t)w; }
+__device__ __forceinline__ void set_ep_word(float& w, uint32_t v) { w = __uint_as_float(v); }
+__device__ __forceinline__ void set_ep_word(double& w, uint32_t v) { w = (double)v; }
+
 // `package`: the draws of in-kernel auto-reset number `counter` of this environment (a stream of its
 // own: an explicit pdx_reset at call counter c and auto-reset package c must not share draws)
 template <class T, int RNG>
@@ -338,10 +346,10 @@ __device__ __forceinline__ void gen_package(const KArgs<T>& a, int64_t j, uint32
 // other pending slot-0 packages in lane order, slot 1, ...  One pass; more only if more than 32 lanes
 // were waiting for their next package (impossible: one per lane).
 template <class T, int TASK, int PHYS, bool NOISE, int RNG, bool PID>
-__device__ __forceinline__ int flush_pending(const KArgs<T>& a, int64_t warp_base, int e_mine, int pend) {
+__device__ __forceinline__ int flush_pending(const KArgs<T>& a, int64_t warp_base, uint32_t e_mine, int pend) {
   const unsigned full = 0xffffffffu;
   const int lane = threadIdx.x & 31;
-  const int next = (e_mine + 1) & (kPackSlots - 1);
+  const int next = (int)((e_mine + 1) & (kPackSlots - 1));
   // group 0: the next-needed slot of each lane where that slot is pending; groups 1..kPackSlots: slot s - 1
   // of each lane where pending and not already in group 0
   unsigned b[kPackSlots + 1];
@@ -360,12 +368,13 @@ __device__ __forceinline__ int flush_pending(const KArgs<T>& a, int64_t warp_bas
 #pragma unroll
   for (int g = 0; g <= kPackSlots; ++g)
     if (has && lane >= start[g] && lane < start[g + 1]) { grp = g; src = (int)__fns(b[g], 0, lane - start[g] + 1); }
-  const int e_src = __shfl_sync(full, e_mine, src);
+  const uint32_t e_src = __shfl_sync(full, e_mine, src);
   if (has) {
-    const int slot = grp == 0 ? ((e_src + 1) & (kPackSlots - 1)) : grp - 1;
+    const uint32_t slot = grp == 0 ? ((e_src + 1) & (kPackSlots - 1)) : (uint32_t)(grp - 1);
     // slot s holds a package p > e with p = s (mod kPackSlots): the first one the owner will ask this slot for
-    const int p = e_src + 1 + ((slot - (e_src + 1)) & (kPackSlots - 1));
-    gen_package<T, TASK, PHYS, NOISE, RNG, PID>(a, warp_base + src, (uint32_t)p);
+    // (modulo 2^28 like e: a multiple of kPackSlots, so the slot of p is unchanged)
+    const uint32_t p = (e_src + 1 + ((slot - (e_src + 1)) & (kPackSlots - 1))) & kEpMask;
+    gen_package<T, TASK, PHYS, NOISE, RNG, PID>(a, warp_base + src, p);
   }
   // which of my pending packages were among the first 32 items
   if (((pend >> next) & 1) && __popc(b[0] & ((1u << lane) - 1u)) < 32) pend &= ~(1 << next);
@@ -390,9 +399,8 @@ __device__ __forceinline__ void take_package(Model<T, TASK, PHYS, NOISE, RNG, PI
   constexpr int C = Mo::C;
   const DevCfg<T>& c = m.c;
   T* w = m.w;
-  const int ew = (int)w[L.ep_index];                 // 16 e + pending bits
-  const int e = ew >> 4;
-  const int slot = (e + 1) & (kPackSlots - 1);
+  const uint32_t ew = ep_word(w[L.ep_index]);        // (e << 4) | pending bits
+  const int slot = (int)(((ew >> 4) + 1) & (kPackSlots - 1));
   const T* pk = package_ptr<Mo>(state, n, i, history, slot);
   T ou[4], b0[3] = {T(0), T(0), T(0)};
 #pragma unroll
@@ -428,7 +436,7 @@ __device__ __forceinline__ void take_package(Model<T, TASK, PHYS, NOISE, RNG, PI
       w[L.gyro_bias + k] += pi2 * b0[k];
     }
   }
-  w[L.ep_index] = (T)((ew + 16) | (1 << slot));
+  set_ep_word(w[L.ep_index], (ew + 16) | (1u << slot));   // (32-bit wrap: e + 1 modulo 2^28)
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -767,7 +775,7 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
         if constexpr (POOL) {
           if (fin && c.auto_reset) {
             const char* pk = reinterpret_cast<const char*>(
-                package_ptr<Mo>(state, n, i, H, (((int)w[L.ep_index] >> 4) + 1) & (kPackSlots - 1)));
+                package_ptr<Mo>(state, n, i, H, (int)(((ep_word(w[L.ep_index]) >> 4) + 1) & (kPackSlots - 1))));
 #pragma unroll
             for (int b = 0; b < (int)(L.pack_quads * 4 * sizeof(T)) + 127; b += 128)
               asm volatile("prefetch.global.L1 [%0];" ::"l"(pk + b));     // (into L1: this lane reads them itself)
@@ -932,12 +940,12 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
           take_package(m, state, n, i, H, stale, o1, o2);
         } else {
           // the draws of auto-reset number e + 1 of this environment (same keys as gen_package in dump mode)
-          const int e_next = ((int)w[L.ep_index] >> 4) + 1;
+          const uint32_t e_next = ((ep_word(w[L.ep_index]) >> 4) + 1) & kEpMask;
           const Rng<T, RNG> rr = make_rng<T, RNG>(a, (uint64_t)e_next, i,
                                                   a.b.tape_reset ? a.b.tape_reset + (int64_t)t * c.slots_reset * n : nullptr,
                                                   a.dump_reset ? a.dump_reset + (int64_t)t * c.slots_reset * n : nullptr, true);
           reset_env(m, rr, stale, o1, o2);
-          w[L.ep_index] = (T)(16 * e_next);
+          set_ep_word(w[L.ep_index], e_next << 4);
         }
         bool rows_done = false;
         if constexpr (sizeof(T) == 4) {
@@ -981,7 +989,8 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
       // when some environment would find its NEXT slot still pending (all kPackSlots of its packages
       // used up since the last regeneration: a burst of very short episodes) -- so the take at the end of
       // a step never has to wait for a package.
-      const int ew = (int)w[L.ep_index], e0 = ew >> 4, pend0 = ew & 15;
+      const uint32_t ew = ep_word(w[L.ep_index]), e0 = ew >> 4;
+      const int pend0 = (int)(ew & 15);
       const int total = (int)__reduce_add_sync(full, (unsigned)__popc(pend0));     // pending packages of the warp
       const bool urgent = (pend0 >> ((e0 + 1) & (kPackSlots - 1))) & 1;
       if (vote(urgent || total >= 40)) {
@@ -993,7 +1002,7 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
 #pragma unroll
           for (int k = 0; k < Mo::NW; ++k) w[k] = T(0);
         }
-        w[L.ep_index] = (T)((ew & ~15) | pend1);
+        set_ep_word(w[L.ep_index], (ew & ~15u) | (uint32_t)pend1);
       }
     }
 

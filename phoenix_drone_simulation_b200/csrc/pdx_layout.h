@@ -12,6 +12,7 @@
 namespace pdx {
 
 constexpr int kPackSlots = 4;      // reset packages kept per environment (power of two: slot = package number & 3)
+constexpr uint32_t kEpMask = (1u << 28) - 1;   // the auto-reset counter e of the ep_index word counts modulo 2^28
 
 struct Layout {
   int xyz, vel;
@@ -23,9 +24,12 @@ struct Layout {
   int pid;                 // PID control modes: rate integral 3, rate last error 3, attitude integral 3,
                            // attitude last error 3 (control.py:133-134,226-227)
   int ep_return, ep_length;
-  int ep_index;            // 16 e + pend: e = number of in-kernel auto-resets this
-                           // environment has consumed (keys the reset draws), pend bit s = package slot s was
-                           // consumed and is not regenerated yet (one word: the step kernel has no register to spare)
+  int ep_index;            // uint32_t (e << 4) | pend: e = number of in-kernel auto-resets this environment
+                           // has consumed, modulo 2^28 (keys the reset draws), pend bit s = package slot s was
+                           // consumed and is not regenerated yet (one word: the step kernel has no register to
+                           // spare).  float64 holds the integer's value, float32 its bit pattern (which may read
+                           // as a denormal or a NaN: the word is only moved, never used in arithmetic); see
+                           // ep_word / set_ep_word in pdx_kernels.cuh
   int ref_offset;          // circle only
   int gyro_bias, gyro_lpf; // noise only
   int n_words;             // words before the history ring

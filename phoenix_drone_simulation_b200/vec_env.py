@@ -321,6 +321,33 @@ class VecEnv:
         for k, w in enumerate(range(fw, fw + nw)):
             self.state[w // 4, :, w % 4] = value[:, k]
 
+    def _ep_word(self):
+        """The state word ep_index of every environment, a view: uint32 (e << 4) | pend, held as the
+        value in float64 and as the bit pattern in float32 (csrc/pdx_layout.h)."""
+        fw, _ = self._field('ep_index')
+        if self.dtype == torch.float32:
+            return self.state.view(torch.int32)[fw // 4, :, fw % 4]
+        return self.state[fw // 4, :, fw % 4]
+
+    def episode_counters(self):
+        """(episodes, pending): int64 [N] in-kernel auto-resets each environment has consumed, modulo 2^28
+        (they key the reset draws), and int32 [N] bit mask of reset-package slots waiting to be regenerated."""
+        w = self._ep_word().to(torch.int64) & 0xFFFFFFFF
+        return w >> 4, (w & 15).to(torch.int32)
+
+    def set_episode_counters(self, episodes, pending=0b1111):
+        """Sets the counters `episode_counters` reports (scalars or [N] tensors; episodes modulo 2^28).
+        The pooled packages were drawn for the old counter: with all four pending bits (the default) the
+        end of the next step regenerates them under the new keys.  An episode that ends in that first step
+        still takes the old package of its slot."""
+        e = torch.as_tensor(episodes, dtype=torch.int64, device=self.device) & ((1 << 28) - 1)
+        p = torch.as_tensor(pending, dtype=torch.int64, device=self.device)
+        assert bool(((p >= 0) & (p < 16)).all()), 'pending is a mask of the 4 package slots'
+        w = ((e << 4) | p).expand(self.num_envs)
+        if self.dtype == torch.float32:
+            w = torch.where(w >= 1 << 31, w - (1 << 32), w).to(torch.int32)   # the same 32 bits, as int32
+        self._ep_word().copy_(w.to(self._ep_word().dtype))
+
     def state_dict(self):
         return {'state': self.state.clone(), 'counter': self._counter, 'seed': self.seed,
                 'env_id': self.env_id, 'stats': self.stats.clone()}

@@ -497,7 +497,7 @@ def test_fused_collector_kernel_is_policy_kernel_plus_env_kernel(env_id, kernel,
     # regenerates packages per 128-environment tile, the step kernel per block)
     for name in ('xyz', 'vel', 'ou', 'last_action', 'ep_length', 'gyro_bias', 'gyro_lpf', 'dt', 'mass'):
         torch.testing.assert_close(env.get_state(name), twin.get_state(name), rtol=1e-5, atol=1e-5)
-    assert torch.equal(env.get_state('ep_index') // 16, twin.get_state('ep_index') // 16)       # auto-resets consumed
+    assert torch.equal(env.episode_counters()[0], twin.episode_counters()[0])                  # auto-resets consumed
     # ---- the running-statistics sums accumulated in-kernel == a pass over the observations the policy saw
     mom, shift = data['obs_moments']
     x = col.obs[:T].reshape(T * N, -1).double() - shift.double()

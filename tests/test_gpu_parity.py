@@ -469,7 +469,8 @@ def test_padded_row_mode_matches_rotated_walk(env_id, kw, N):
             out_u['final_obs'].zero_()
             env.step_many(acts[20:24], out_u)
             res[mode] = (o0, {k: v.clone() for k, v in out.items()}, singles, out_u['obs'].clone(),
-                         {nm: env.get_state(nm) for nm in ('xyz', 'vel', 'ou', 'last_action', 'ep_return', 'ep_length', 'hist', 'dt', 'mass', 'ep_index')},
+                         {**{nm: env.get_state(nm) for nm in ('xyz', 'vel', 'ou', 'last_action', 'ep_return', 'ep_length', 'hist', 'dt', 'mass')},
+                          'episodes': env.episode_counters()[0]},
                          env.episode_stats().clone())
     finally:
         os.environ.pop('PDX_WMODE', None)
@@ -494,7 +495,7 @@ def test_padded_row_mode_matches_rotated_walk(env_id, kw, N):
     # state and the order of the statistics' atomics may differ; everything an episode can observe may not)
     for name in ('xyz', 'vel', 'ou', 'last_action', 'ep_return', 'ep_length', 'hist', 'dt', 'mass'):
         same(a[4][name], b[4][name], name)
-    assert torch.equal(a[4]['ep_index'] // 16, b[4]['ep_index'] // 16)
+    assert torch.equal(a[4]['episodes'], b[4]['episodes'])
     torch.testing.assert_close(a[5], b[5], rtol=1e-5, atol=0)
     assert int(a[5][0]) > 0, 'no episode ended: the reset path of the padded rows was not exercised'
 
