@@ -202,7 +202,12 @@ class OracleEnv:
                  observation_history_size=2, enable_reset_distribution=True,
                  aggregate_phy_steps=None, latency=0.015, motor_time_constant=0.080,
                  motor_thrust_noise=0.05, use_ground_effect=False,
-                 lin_damping=0.04, ang_damping=0.04, control_mode='PWM', **penalties):
+                 lin_damping=0.04, ang_damping=0.04, control_mode='PWM',
+                 observation_frequency=100, target_pos=(0, 0, 1), use_latency=None,
+                 use_motor_dynamics=None, **penalties):
+        """`use_latency` / `use_motor_dynamics`: None keeps the agent's default (agents.py:165,196); a bool
+        stands for the reference's debug scripts assigning drone.use_latency / drone.use_motor_dynamics
+        after construction (Bullet agent only; latency still needs latency >= TIME_STEP)."""
         self.task, self.physics = ENV_IDS[env_id]
         self.src = source if source is not None else NumpyGlobalSource()
         bullet = self.physics == 'bullet'
@@ -214,7 +219,7 @@ class OracleEnv:
         if self.task == 'takeoff' and not bullet:
             self.agg = 1                                             # takeoff.py:224
         self.TIME_STEP = 1.0 / self.sim_freq                         # base.py:98
-        self.obs_rate = int(self.sim_freq // 100)                    # base.py:108
+        self.obs_rate = int(self.sim_freq // observation_frequency)  # base.py:108
         self.dr = domain_randomization
         self.noise_on = observation_noise > 0
         self.H = observation_history_size
@@ -235,7 +240,11 @@ class OracleEnv:
         self.GND_EFF_H_CLIP = 0.25 * PROP_RADIUS * np.sqrt(
             (15 * max_rpm ** 2 * KF * GND_EFF_COEFF) / self.MAX_THRUST)
         self.use_latency = bullet and latency >= self.TIME_STEP       # agents.py:165
+        if use_latency is not None and bullet:
+            self.use_latency = bool(use_latency) and latency >= self.TIME_STEP
         self.use_motor_dynamics = bullet
+        if use_motor_dynamics is not None and bullet:
+            self.use_motor_dynamics = bool(use_motor_dynamics)
         self.buf_size = int(max(1, int(latency // self.TIME_STEP)))  # agents.py:180
         self.MOTOR_T = motor_time_constant
         self.ou_sigma = 0.2 * motor_thrust_noise                     # agents.py:206
@@ -279,7 +288,7 @@ class OracleEnv:
             self.ref[:, 2] = np.arange(300) / 300
         self.num_ref = 300
         self.ref_offset = 0
-        self.target_pos = np.array([0, 0, 1.0], dtype=np.float32)
+        self.target_pos = np.array(target_pos, dtype=np.float32)     # hover.py:14 (Circle / TakeOff overwrite it)
 
         z0 = 0.0125 if self.task == 'takeoff' else 1.0
         self.init_xyz = np.array([0, 0, z0], dtype=np.float32)       # float32! hover.py:44
@@ -719,8 +728,9 @@ def _quat_mul(a, b):
                      aw * bw - ax * bx - ay * by - az * bz])
 
 
-def draws_per_phase(env_id, observation_history_size=2, aggregate_phy_steps=None, latency=0.015):
-    """(reset_slots, step_slots): tape widths, counted by dry-running one reset + one step."""
+def draws_per_phase(env_id, **kwargs):
+    """(reset_slots, step_slots): tape widths, counted by dry-running one reset + one step of an OracleEnv
+    built with `kwargs`."""
     class _Count(TapeSource):
         def __init__(self):
             self.n = 0
@@ -741,8 +751,7 @@ def draws_per_phase(env_id, observation_history_size=2, aggregate_phy_steps=None
             return np.zeros(n)
 
     c = _Count()
-    env = OracleEnv(env_id, c, observation_history_size=observation_history_size,
-                    aggregate_phy_steps=aggregate_phy_steps, latency=latency)
+    env = OracleEnv(env_id, c, **kwargs)
     env.reset()
     env.step(np.zeros(4, dtype=np.float32))
     return c.counts['reset'], c.counts['step']

@@ -25,6 +25,13 @@ class VecEnv:
       seed (Philox key), env_offset (global index of env 0 of this shard: results do not
       depend on how environments are sharded), rng ('philox' | 'tape'),
       keep_final_obs (also return the last observation of finished episodes).
+
+    With auto_reset=False (config.EnvConfig) a finished environment is not reset in the step: it steps on from its
+    terminal state, as the reference does until the caller resets it (`reset(mask)`).  Its episode length keeps
+    counting, so `truncated` stays set once the time limit is reached and `terminated` follows done() step by step.
+    Every step on which an environment's episode is over (terminated or truncated) counts as a finished episode in
+    episode_stats() and reports the running length / return in `episode_length` / `episode_return`: an episode that
+    stays ended is counted again on each step.  The reset-package counters (`episode_counters`) do not move.
     """
 
     def __init__(self, env_id, num_envs, device='cuda', dtype=torch.float32, seed=0,
