@@ -315,6 +315,46 @@ int64_t pdx_collect_scratch_bytes(int32_t device);
 int pdx_collect(const PdxConfig* cfg, const PdxBuffers* buf, const PdxPolicy* policy, const PdxRollout* rollout,
                 uint64_t seed, uint64_t counter, void* stream);
 
+/* ---- deterministic evaluation of many policies on shared episodes (utils/evaluation.py:52-107) ----
+ * EnvironmentEvaluator.eval for P policies x E episodes in ONE launch (csrc/pdx_evaluate.cu): every policy acts
+ * with its actor mean on the standardised observation (core.py:282-289) for at most max_episode_steps steps, without
+ * auto-reset; an episode accumulates reward, cost and length up to and including the step that reports terminated
+ * or truncated.  Episode e of every policy starts from the same state and sees the same draws (keyed by
+ * buf->env_offset + e, step t at `counter + t` as pdx_step_many): the results of a policy do not depend on the
+ * other policies of the call.  The actor arithmetic is pdx_policy_step's, bit for bit.
+ *   buf: n_envs == episodes; state [P][pdx_state_quads][E][4], P copies of the state after pdx_init + pdx_reset of
+ *        E environments; obs [E][obs_dim], the observation that pdx_reset returned.  The state is read, not written.
+ * Supported: float32 with Philox draws, every task / physics / control mode, obs_dim up to the shared-memory plan
+ * (history 16 included); PDX_ERR_INVALID otherwise, and for bad arguments before any device call. */
+typedef struct PdxPolicySet {
+  int32_t n_policies;           /* P >= 1 */
+  int32_t episodes;             /* E >= 1, P * E < 2^31 */
+  int32_t obs_dim;
+  int32_t hidden[2];            /* actor hidden sizes (<= 64), the same for every policy */
+  int32_t n_out;                /* actor outputs (<= 4); actions past n_out are 0 */
+  int64_t stride;               /* floats between two images in `packed` (>= the actor part, a multiple of 4) */
+  const float* packed;          /* [P][stride]: pdx_policy_pack images; only the actor part is read */
+  const float* mean;            /* [P][obs_dim] observation normaliser, or NULL (with std) for none */
+  const float* std;             /* [P][obs_dim] */
+  float eps;                    /* (o - mean) / (std + eps) */
+  int32_t reserved;
+} PdxPolicySet;
+typedef struct PdxEvaluation {
+  double* ret;                  /* out [P][E] episode return  */
+  double* cost;                 /* out [P][E] episode cost    */
+  int32_t* length;              /* out [P][E] episode length  */
+  /* optional validation records, all or none, [T][P][E] with T = max_episode_steps; steps after every episode of
+   * a block ended are not written */
+  float* rec_obs;               /* [T][P][E][obs_dim] observation the actor saw */
+  float* rec_act;               /* [T][P][E][4] action */
+  float* rec_reward;            /* [T][P][E] */
+  float* rec_cost;              /* [T][P][E] */
+  uint8_t* rec_terminated;      /* [T][P][E] */
+  uint8_t* rec_truncated;       /* [T][P][E] */
+} PdxEvaluation;
+int pdx_evaluate(const PdxConfig* cfg, const PdxBuffers* buf, const PdxPolicySet* set, const PdxEvaluation* out,
+                 uint64_t seed, uint64_t counter, void* stream);
+
 /* Cross-rank combination of the 8-word episode statistics (utils/mpi_tools.py:217-240 does four
  * MPI all-reduces per key): the caller all-gathers the per-rank vectors into gathered[world][8]
  * (one NCCL call) and this writes out[0..4) = sums, out[4], out[6] = minima, out[5], out[7] = maxima. */

@@ -28,6 +28,7 @@ UNITS = {
     'pdx_rollout.cu': [],
     'pdx_policy_tc.cu': [],
     'pdx_collect.cu': ['-use_fast_math'],
+    'pdx_evaluate.cu': ['-use_fast_math'],
 }
 
 

@@ -628,6 +628,8 @@ struct StepCtx {
   double* acc_sum; T* acc_ext;
   int NT;                     // observation tiles (1 or 2)
   bool fast2, bulk, latency, any_fin;
+  T ev_reward, ev_cost;       // EVAL: this step's reward, cost and flags, handed to the caller
+  bool ev_terminated, ev_truncated;
 };
 
 // ---------------------------------------------------------------------------------------------
@@ -639,7 +641,11 @@ struct StepCtx {
 // ---------------------------------------------------------------------------------------------
 // WIDE: row mode (see rollout_smem_bytes) -- a template parameter because as a run-time branch it made ptxas spill
 // the 17 words of the new entry on BOTH paths.
-template <class T, int TASK, int PHYS, bool NOISE, int RNG, bool PID, int WIDE, class Vote>
+// EVAL (k_evaluate, csrc/pdx_evaluate.cu): no global per-step stores (observation rows and their bulk copies, reward,
+// cost, flags, episode return / length, final_obs) and no episode statistics; reward, cost and flags go to sc.ev_*.
+// Without auto-reset (an evaluation) no reset package is ever taken, so the package regeneration and its vote are
+// compiled out as well: `vote` is not called.
+template <class T, int TASK, int PHYS, bool NOISE, int RNG, bool PID, int WIDE, bool EVAL = false, class Vote>
 __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, PHYS, NOISE, RNG, PID>& m, StepCtx<T>& sc,
                                              const int t, const float4 a4, Vote vote) {
   typedef Model<T, TASK, PHYS, NOISE, RNG, PID> Mo;
@@ -674,7 +680,7 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
     // ---- this step's tile slice was last read by the warp's bulk copy of step t - n_tiles (lane 0 issues
     // the copies of the warp, so it is the lane that can wait for them).  No block-wide barrier: warps
     // run through their steps independently.
-    if (!fast2) {
+    if (!EVAL && !fast2) {
       if (lane == 0 || quad) { if (NT == 2) bulk_wait_read<1>(); else bulk_wait_read<0>(); }   // (quad: a lane sends its own row)
       __syncwarp();
     }
@@ -899,15 +905,20 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
       w[L.ep_length] = (T)n_ep;
 #pragma unroll
       for (int k = 0; k < 4; ++k) w[L.last_action + k] = actT[k];
-      reinterpret_cast<T*>(a.b.reward)[tn_off + i] = r;
-      reinterpret_cast<T*>(a.b.cost)[tn_off + i] = cst;
-      a.b.terminated[tn_off + i] = dn ? 1 : 0;
-      a.b.truncated[tn_off + i] = trunc ? 1 : 0;
-      ep_ret_out = w[L.ep_return];
-      ep_len_out = n_ep;
-      if (a.b.episode_return) reinterpret_cast<T*>(a.b.episode_return)[tn_off + i] = fin ? ep_ret_out : T(0);
-      if (a.b.episode_length) a.b.episode_length[tn_off + i] = fin ? ep_len_out : 0;
+      if constexpr (EVAL) {
+        sc.ev_reward = r; sc.ev_cost = cst; sc.ev_terminated = dn; sc.ev_truncated = trunc;
+      } else {
+        reinterpret_cast<T*>(a.b.reward)[tn_off + i] = r;
+        reinterpret_cast<T*>(a.b.cost)[tn_off + i] = cst;
+        a.b.terminated[tn_off + i] = dn ? 1 : 0;
+        a.b.truncated[tn_off + i] = trunc ? 1 : 0;
+        ep_ret_out = w[L.ep_return];
+        ep_len_out = n_ep;
+        if (a.b.episode_return) reinterpret_cast<T*>(a.b.episode_return)[tn_off + i] = fin ? ep_ret_out : T(0);
+        if (a.b.episode_length) a.b.episode_length[tn_off + i] = fin ? ep_len_out : 0;
+      }
     }
+    if constexpr (EVAL) return;
 
     // ---- finished episodes: statistics, auto-reset
     if (fin) {

@@ -395,6 +395,10 @@ int launch_policy(const PolArgs& a, cudaStream_t st) {
   const size_t words = 2 * ((D + 3) & ~3) + (size_t)(D * HP + HP + HP * HP + HP + HP * 4 + 4) +
                        (size_t)(D * HV + HV + HV * HV + HV + HV * 4 + 4) + (size_t)kHidMax * kPolBlock;
   const size_t smem = words * sizeof(float);
+  if (a.n == 0) {                                     // pack only (pdx_evaluate stages the actor part of wider images)
+    k_pack_policy<HP, HV><<<8, 256, 0, st>>>(a, const_cast<float*>(a.packed));
+    return launch_status("pdx_policy_pack");
+  }
   if (smem > (size_t)227 * 1024) return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step: obs_dim too wide for the shared-memory plan");
   int dev = 0;
   cudaGetDevice(&dev);
@@ -403,10 +407,6 @@ int launch_policy(const PolArgs& a, cudaStream_t st) {
     if (cudaFuncSetAttribute(k_policy<HP, HV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
       return launch_status("pdx_policy_step (shared-memory opt-in)");
     set_by_dev[dev & 63] = smem;
-  }
-  if (a.n == 0) {                                     // pack only
-    k_pack_policy<HP, HV><<<8, 256, 0, st>>>(a, const_cast<float*>(a.packed));
-    return launch_status("pdx_policy_pack");
   }
   const unsigned grid = (unsigned)((a.n + kPolBlock - 1) / kPolBlock);
   k_policy<HP, HV><<<grid, kPolBlock, smem, st>>>(a);

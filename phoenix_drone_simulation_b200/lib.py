@@ -82,6 +82,18 @@ class PdxRollout(C.Structure):
                 ('scratch_bytes', C.c_int64), ('obs_moments', C.c_void_p)]
 
 
+class PdxPolicySet(C.Structure):
+    _fields_ = [('n_policies', C.c_int32), ('episodes', C.c_int32), ('obs_dim', C.c_int32), ('hidden', C.c_int32 * 2),
+                ('n_out', C.c_int32), ('stride', C.c_int64), ('packed', C.c_void_p), ('mean', C.c_void_p),
+                ('std', C.c_void_p), ('eps', C.c_float), ('reserved', C.c_int32)]
+
+
+class PdxEvaluation(C.Structure):
+    _fields_ = [('ret', C.c_void_p), ('cost', C.c_void_p), ('length', C.c_void_p), ('rec_obs', C.c_void_p),
+                ('rec_act', C.c_void_p), ('rec_reward', C.c_void_p), ('rec_cost', C.c_void_p),
+                ('rec_terminated', C.c_void_p), ('rec_truncated', C.c_void_p)]
+
+
 _lib = None
 
 
@@ -137,6 +149,8 @@ def load():
     lib.pdx_policy_tc_pack_words.argtypes = [C.c_int32, P(PdxMlp), P(PdxMlp), C.c_int32]
     lib.pdx_policy_tc_pack_words.restype = C.c_int64
     lib.pdx_policy_tc_pack.argtypes = [C.c_int32, P(PdxMlp), P(PdxMlp), C.c_int32, C.c_void_p, C.c_void_p]
+    lib.pdx_evaluate.argtypes = [P(PdxConfig), P(PdxBuffers), P(PdxPolicySet), P(PdxEvaluation), C.c_uint64, C.c_uint64,
+                                 C.c_void_p]
     if lib.pdx_abi_version() != ABI_VERSION:
         raise PhoenixB200Error(f'ABI mismatch: library {lib.pdx_abi_version()} != binding {ABI_VERSION}')
     if lib.pdx_config_size() != C.sizeof(PdxConfig) or lib.pdx_buffers_size() != C.sizeof(PdxBuffers):
@@ -157,4 +171,5 @@ EXPORTED_SYMBOLS = [
     'pdx_step_many', 'pdx_dump_draws',
     'pdx_gae', 'pdx_moments', 'pdx_stats_combine', 'pdx_policy_step', 'pdx_policy_pack', 'pdx_policy_pack_words',
     'pdx_policy_step_tc', 'pdx_policy_tc_pack', 'pdx_policy_tc_pack_words', 'pdx_collect', 'pdx_collect_scratch_bytes', 'pdx_oms_update',
+    'pdx_evaluate',
 ]
