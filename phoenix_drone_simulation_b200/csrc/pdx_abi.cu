@@ -3,7 +3,6 @@
 #include <cstring>
 #include <cmath>
 #include "pdx_dispatch.cuh"
-#include "pdx_error.h"
 
 namespace {
 
@@ -20,12 +19,6 @@ namespace {
 int fail(int code, const char* fmt, const char* detail = "") {
   std::snprintf(g_err, sizeof(g_err), fmt, detail);
   return code;
-}
-
-int cuda_fail(cudaError_t e) {
-  if (e == cudaErrorNoDevice || e == cudaErrorInsufficientDriver)
-    return fail(PDX_ERR_NO_DEVICE, "no CUDA device (%s); this library has no CPU path", cudaGetErrorString(e));
-  return fail(PDX_ERR_CUDA, "CUDA error: %s", cudaGetErrorString(e));
 }
 
 pdx::Layout layout_of(const PdxConfig* c) {
@@ -62,7 +55,7 @@ int check_buffers(const PdxConfig* c, const PdxBuffers* b, bool step) {
   return PDX_OK;
 }
 
-int launch(int kind, const PdxConfig* cfg, const PdxBuffers* buf, const float* actions,
+int launch(const char* what, int kind, const PdxConfig* cfg, const PdxBuffers* buf, const float* actions,
            const uint8_t* mask, uint64_t seed, uint64_t counter, double* ds, double* dr, double* di,
            void* stream, int n_steps = 1) {
   int rc = validate(cfg);
@@ -81,13 +74,9 @@ int launch(int kind, const PdxConfig* cfg, const PdxBuffers* buf, const float* a
   }
   if (kind == pdx::KIND_STEP && !actions) return fail(PDX_ERR_INVALID, "null actions");
   if (kind == pdx::KIND_STEP && (n_steps < 1 || n_steps > (1 << 20))) return fail(PDX_ERR_INVALID, "n_steps must be in [1, 2^20]");
-  int ndev = 0;
-  cudaError_t e = cudaGetDeviceCount(&ndev);
-  if (e != cudaSuccess) return cuda_fail(e);
-  if (ndev == 0) return fail(PDX_ERR_NO_DEVICE, "no CUDA device; this library has no CPU path");
-  if (buf->device < 0 || buf->device >= ndev) return fail(PDX_ERR_INVALID, "bad device ordinal");
-  e = cudaSetDevice(buf->device);       // this library carries its own (static) CUDA runtime
-  if (e != cudaSuccess) return cuda_fail(e);
+  rc = pdx::select_device(buf->device);
+  if (rc) return rc;
+  cudaError_t e;
   pdx::LaunchArgs la{&c, buf, actions, mask, seed, counter, ds, dr, di, n_steps, (cudaStream_t)stream};
   const bool pid = c.control_mode != PDX_CTRL_PWM, simple = c.physics == PDX_PHYSICS_SIMPLE;
   if (c.dtype == PDX_DTYPE_F32)
@@ -96,8 +85,7 @@ int launch(int kind, const PdxConfig* cfg, const PdxBuffers* buf, const float* a
   else
     e = simple ? (pid ? pdx::launch_f64_simple_pid(kind, la) : pdx::launch_f64_simple(kind, la))
                : (pid ? pdx::launch_f64_bullet_pid(kind, la) : pdx::launch_f64_bullet(kind, la));
-  if (e != cudaSuccess) return cuda_fail(e);
-  return PDX_OK;
+  return pdx::cuda_error(what, e);
 }
 
 }  // namespace
@@ -176,28 +164,27 @@ int64_t pdx_rollout_bytes(const PdxConfig* cfg, int32_t n_steps) {
 
 int pdx_device_count(void) {
   int n = 0;
-  const cudaError_t e = cudaGetDeviceCount(&n);
-  if (e != cudaSuccess) { cuda_fail(e); return 0; }
+  pdx::count_devices(&n);
   return n;
 }
 
 int pdx_init(const PdxConfig* cfg, const PdxBuffers* buf, uint64_t seed, uint64_t counter, void* stream) {
-  return launch(pdx::KIND_INIT, cfg, buf, nullptr, nullptr, seed, counter, nullptr, nullptr, nullptr, stream);
+  return launch("pdx_init", pdx::KIND_INIT, cfg, buf, nullptr, nullptr, seed, counter, nullptr, nullptr, nullptr, stream);
 }
 
 int pdx_reset(const PdxConfig* cfg, const PdxBuffers* buf, const uint8_t* mask, uint64_t seed,
               uint64_t counter, void* stream) {
-  return launch(pdx::KIND_RESET, cfg, buf, nullptr, mask, seed, counter, nullptr, nullptr, nullptr, stream);
+  return launch("pdx_reset", pdx::KIND_RESET, cfg, buf, nullptr, mask, seed, counter, nullptr, nullptr, nullptr, stream);
 }
 
 int pdx_step(const PdxConfig* cfg, const PdxBuffers* buf, const float* actions, uint64_t seed,
              uint64_t counter, void* stream) {
-  return launch(pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, nullptr, nullptr, nullptr, stream);
+  return launch("pdx_step", pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, nullptr, nullptr, nullptr, stream);
 }
 
 int pdx_step_many(const PdxConfig* cfg, const PdxBuffers* buf, const float* actions, int32_t n_steps,
                   uint64_t seed, uint64_t counter, void* stream) {
-  return launch(pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, nullptr, nullptr, nullptr, stream, n_steps);
+  return launch("pdx_step_many", pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, nullptr, nullptr, nullptr, stream, n_steps);
 }
 
 }  // extern "C"
@@ -207,10 +194,10 @@ extern "C" int pdx_dump_draws(const PdxConfig* cfg, const PdxBuffers* buf, const
                               uint64_t seed, uint64_t counter, double* step_tape, double* reset_tape,
                               double* init_tape, void* stream) {
   if (init_tape)
-    return launch(pdx::KIND_INIT, cfg, buf, nullptr, nullptr, seed, counter, nullptr, nullptr, init_tape, stream);
+    return launch("pdx_dump_draws", pdx::KIND_INIT, cfg, buf, nullptr, nullptr, seed, counter, nullptr, nullptr, init_tape, stream);
   if (!actions && reset_tape)
-    return launch(pdx::KIND_RESET, cfg, buf, nullptr, nullptr, seed, counter, nullptr, reset_tape, nullptr, stream);
+    return launch("pdx_dump_draws", pdx::KIND_RESET, cfg, buf, nullptr, nullptr, seed, counter, nullptr, reset_tape, nullptr, stream);
   if (actions && step_tape && reset_tape)
-    return launch(pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, step_tape, reset_tape, nullptr, stream);
+    return launch("pdx_dump_draws", pdx::KIND_STEP, cfg, buf, actions, nullptr, seed, counter, step_tape, reset_tape, nullptr, stream);
   return fail(PDX_ERR_INVALID, "pdx_dump_draws: inconsistent tape pointers");
 }

@@ -28,10 +28,8 @@
 //
 // Global traffic per env-step is the rollout itself: observation row, action, value, log-probability,
 // reward, cost and the two flags.
-#include <cstdio>
 #include "pdx_dispatch.cuh"
 #include "pdx_tc.cuh"
-#include "pdx_error.h"
 
 // Measured slower on configs[4] (DESIGN.md §4): keeping two 16-column tcgen05.ld chunks in flight in the epilogues
 // (software prefetch of the next chunk, 1,508 vs 1,420 us) -- more live registers and code for a latency the other
@@ -327,10 +325,7 @@ __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArg
       // the Gaussian draw does not depend on the networks: under layer 1
       float eps[4], lp = 0.0f;
       {
-        const uint4 rr = tc_philox(make_uint4((uint32_t)ig, (uint32_t)(p.pol_counter + (uint64_t)t), (uint32_t)(ig >> 32), 0x504F4Cu),
-                                   make_uint2((uint32_t)p.pol_seed, (uint32_t)(p.pol_seed >> 32)));
-        pdx_policy_box_muller(rr.x, rr.y, &eps[0], &eps[1]);
-        pdx_policy_box_muller(rr.z, rr.w, &eps[2], &eps[3]);
+        policy_normals(p.pol_seed, p.pol_counter + (uint64_t)t, ig, eps);
 #pragma unroll
         for (int k = 0; k < 4; ++k)
           if (k < p.act_dim) lp += -0.5f * eps[k] * eps[k] - act_std[4 + k] - 0.9189385332046727f;
@@ -504,7 +499,7 @@ static cudaError_t launch_collect(const KArgs<float>& ka, CollectArgs& p, int sm
   // at most 14 warps, and no more than the shared-memory plan admits: wide rows with the split-TF32 images leave
   // room for fewer (D = 40: 10 warps, D = 60: 3) -- the shard then takes more passes
   int max_warps = 14;
-  while (max_warps > 1 && collect_smem<X3>(p.k1, ka.c.obs_dim, max_warps).total > (size_t)227 * 1024) --max_warps;
+  while (max_warps > 1 && collect_smem<X3>(p.k1, ka.c.obs_dim, max_warps).total > kMaxSmemBytes) --max_warps;
   const int64_t n = ka.b.n_envs;
   // passes and warps per CTA: the fewest passes that fit, then the smallest CTA that covers the shard in them
   int64_t passes = (n + (int64_t)sms * max_warps * 32 - 1) / ((int64_t)sms * max_warps * 32);
@@ -515,14 +510,9 @@ static cudaError_t launch_collect(const KArgs<float>& ka, CollectArgs& p, int sm
   p.warps_per_cta = warps;
   p.groups = (int32_t)((n + (int64_t)warps * 32 - 1) / ((int64_t)warps * 32));
   const ColSmem sp = collect_smem<X3>(p.k1, ka.c.obs_dim, warps);
-  if (sp.total > (size_t)227 * 1024) return cudaErrorInvalidConfiguration;
-  static size_t smem_set[16] = {};
-  const int dev = ka.b.device & 15;
-  if (sp.total > smem_set[dev]) {
-    const cudaError_t e = cudaFuncSetAttribute(k_collect<TASK, PHYS, X3>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sp.total);
-    if (e != cudaSuccess) return e;
-    smem_set[dev] = sp.total;
-  }
+  if (sp.total > kMaxSmemBytes) return cudaErrorInvalidConfiguration;
+  const cudaError_t e = opt_in_smem(k_collect<TASK, PHYS, X3>, ka.b.device, sp.total);
+  if (e != cudaSuccess) return e;
   const unsigned grid = (unsigned)(p.groups < sms ? p.groups : sms);
   k_collect<TASK, PHYS, X3><<<grid, warps * 32, sp.total, st>>>(ka, p);
   return cudaGetLastError();
@@ -558,17 +548,10 @@ extern "C" int pdx_collect(const PdxConfig* cfg, const PdxBuffers* buf, const Pd
     return set_error(PDX_ERR_INVALID, "pdx_collect: scratch buffer of pdx_collect_scratch_bytes() bytes required");
   if (buf->n_envs <= 0 || buf->n_envs >= ((int64_t)1 << 31) || !buf->state || !buf->obs || !buf->reward || !buf->cost || !buf->terminated || !buf->truncated)
     return set_error(PDX_ERR_INVALID, "pdx_collect: state / obs / reward / cost / terminated / truncated buffers are required");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return set_error(PDX_ERR_NO_DEVICE, "no CUDA device; this library has no CPU path"); }
-  if (buf->device < 0 || buf->device >= ndev) return set_error(PDX_ERR_INVALID, "bad device ordinal");
-  if (cudaSetDevice(buf->device) != cudaSuccess) return set_error(PDX_ERR_CUDA, "cudaSetDevice failed");
-  KArgs<float> ka;
-  fill_devcfg<float>(c, ka.c);
-  ka.b = *buf;
+  const int rc = select_device(buf->device);
+  if (rc) return rc;
+  KArgs<float> ka = make_kargs<float>(c, *buf, seed, counter, out->n_steps);
   ka.b.episode_return = nullptr; ka.b.episode_length = nullptr;
-  ka.actions = nullptr; ka.mask = nullptr; ka.seed = seed; ka.counter = counter;
-  ka.dump_step = ka.dump_reset = ka.dump_init = nullptr;
-  ka.n_steps = out->n_steps; ka.n_tiles = 1;
   CollectArgs p;
   p.obs_dim = c.obs_dim; p.k1 = tc_k1(c.obs_dim); p.act_dim = pi->n_out; p.n_steps = out->n_steps;
   p.obs0 = out->obs0; p.mean = pol->mean; p.std = pol->std; p.eps = pol->eps; p.log_std = pol->log_std; p.packed = pol->packed;
@@ -586,10 +569,5 @@ extern "C" int pdx_collect(const PdxConfig* cfg, const PdxBuffers* buf, const Pd
   if (circle) e = bullet ? PDX_COL(PDX_TASK_CIRCLE, PDX_PHYSICS_BULLET) : PDX_COL(PDX_TASK_CIRCLE, PDX_PHYSICS_SIMPLE);
   else e = bullet ? PDX_COL(PDX_TASK_HOVER, PDX_PHYSICS_BULLET) : PDX_COL(PDX_TASK_HOVER, PDX_PHYSICS_SIMPLE);
 #undef PDX_COL
-  if (e != cudaSuccess) {
-    char msg[256];
-    std::snprintf(msg, sizeof(msg), "pdx_collect: CUDA error: %s", cudaGetErrorString(e));
-    return set_error(PDX_ERR_CUDA, msg);
-  }
-  return PDX_OK;
+  return cuda_error("pdx_collect", e);
 }

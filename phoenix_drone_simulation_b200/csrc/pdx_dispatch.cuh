@@ -4,6 +4,7 @@
 #pragma once
 #include <cmath>
 #include <cstdlib>
+#include "pdx_host.h"
 #include "pdx_kernels.cuh"
 
 namespace pdx {
@@ -75,7 +76,7 @@ static LaunchShape pick_shape(int D, int E, int wmode) {
     const int block = blocks[bi];
     for (int tiles = 2; tiles >= 1; --tiles) {
       const size_t smem = rollout_smem_bytes<T>(block, D, tiles, E, wmode);
-      if (smem > (size_t)227 * 1024) continue;
+      if (smem > kMaxSmemBytes) continue;
       const int by_smem = (int)(((size_t)228 * 1024) / (smem + 1024));
       const int by_regs = 65536 / (128 * block);
       const int warps = (by_smem < by_regs ? by_smem : by_regs) * (block / 32);
@@ -109,32 +110,16 @@ static cudaError_t launch_kind(int kind, const KArgs<T>& ka, cudaStream_t st) {
   }
   const LaunchShape shape = pick_shape<T>(ka.c.obs_dim, ka.c.core_dim + 4, wmode);
   if (shape.block == 0) return cudaErrorInvalidConfiguration;
-  const int block = shape.block;
-  const size_t smem = shape.smem;
   KArgs<T> kb = ka;
   kb.n_tiles = shape.tiles;
-  const int wide = wmode;
   auto kern = wmode == 1 ? k_rollout<T, TASK, PHYS, NOISE, RNG, PID, 1> : k_rollout<T, TASK, PHYS, NOISE, RNG, PID, 0>;
   if constexpr (quad_ok) { if (wmode == 2) kern = k_rollout<T, TASK, PHYS, NOISE, RNG, PID, 2>; }
-  static size_t smem_set[3][16] = {};               // per variant and device: opt-in dynamic shared memory
-  const int dev = ka.b.device & 15;
-  if (smem > smem_set[wide][dev]) {
-    const cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return e;
-    smem_set[wide][dev] = smem;
-  }
-  const unsigned grid = (unsigned)((n + block - 1) / block);
-  // programmatic stream serialisation: the grid may start while its predecessor drains; the kernel
-  // waits (griddepcontrol.wait) before it reads or writes anything the predecessor could touch
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3(grid); lc.blockDim = dim3(block); lc.dynamicSmemBytes = smem; lc.stream = st;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  // opt-in per call (PDX_BUF_STATE_STABLE): measured, early launch of this kernel AND of a one-CTA-per-SM
+  const cudaError_t e = opt_in_smem(kern, ka.b.device, shape.smem);
+  if (e != cudaSuccess) return e;
+  const unsigned grid = (unsigned)((n + shape.block - 1) / shape.block);
+  // early launch only on request (PDX_BUF_STATE_STABLE): measured, early launch of this kernel AND of a one-CTA-per-SM
   // tensor-core policy kernel around it collapses throughput (profiles/r1_summary.md), so the caller decides
-  lc.attrs = attr; lc.numAttrs = (ka.b.flags & PDX_BUF_STATE_STABLE) ? 1 : 0;
-  return cudaLaunchKernelEx(&lc, kern, kb);
+  return launch_early(kern, grid, shape.block, shape.smem, st, (ka.b.flags & PDX_BUF_STATE_STABLE) != 0, kb);
 }
 
 template <class T, int TASK, int PHYS, bool PID>
@@ -147,15 +132,24 @@ static cudaError_t launch_nr(int kind, bool noise, int rng, const KArgs<T>& ka, 
   return launch_kind<T, TASK, PHYS, false, PDX_RNG_TAPE, PID>(kind, ka, st);
 }
 
+// Kernel arguments of a finalised config and its buffers, with no actions, mask or dump tapes and one observation tile.
+template <class T>
+static KArgs<T> make_kargs(const PdxConfig& cfg, const PdxBuffers& buf, uint64_t seed, uint64_t counter, int n_steps) {
+  KArgs<T> ka;
+  fill_devcfg<T>(cfg, ka.c);
+  ka.b = buf;
+  ka.actions = nullptr; ka.mask = nullptr; ka.seed = seed; ka.counter = counter;
+  ka.dump_step = ka.dump_reset = ka.dump_init = nullptr;
+  ka.n_steps = n_steps; ka.n_tiles = 1;
+  return ka;
+}
+
 // One arithmetic type, physics flavour and control family per translation unit.
 template <class T, int PHYS, bool PID>
 static cudaError_t launch_tu(int kind, const LaunchArgs& la) {
-  KArgs<T> ka;
-  fill_devcfg<T>(*la.cfg, ka.c);
-  ka.b = *la.buf;
-  ka.actions = la.actions; ka.mask = la.mask; ka.seed = la.seed; ka.counter = la.counter;
+  KArgs<T> ka = make_kargs<T>(*la.cfg, *la.buf, la.seed, la.counter, la.n_steps);
+  ka.actions = la.actions; ka.mask = la.mask;
   ka.dump_step = la.dump_step; ka.dump_reset = la.dump_reset; ka.dump_init = la.dump_init;
-  ka.n_steps = la.n_steps;
   ka.n_tiles = 2;
   const bool noise = la.cfg->observation_noise != 0;
   // pdx_dump_draws runs the TAPE-mode kernels with dump pointers set.

@@ -21,9 +21,7 @@
 //
 // Global traffic: the actor image and normaliser once per block, the initial state and observation once per
 // episode, 20 bytes of results per episode (plus the optional validation records).
-#include <cstdio>
 #include "pdx_dispatch.cuh"
-#include "pdx_error.h"
 
 namespace pdx {
 
@@ -64,11 +62,10 @@ __device__ __forceinline__ float ev_relu(float a) {          // fmaxf(a, 0) with
   return d;
 }
 
-// shared-memory plan (bytes): norm float2 [D], actor image [pi_words], rows [B][D], hidden columns [HP][B]
-__host__ __device__ inline int64_t eval_pi_words(int D, int HP) { return (int64_t)D * HP + HP + HP * HP + HP + HP * 4 + 4; }
+// shared-memory plan (bytes): norm float2 [D], actor image [policy_net_words], rows [B][D], hidden columns [HP][B]
 __host__ __device__ inline size_t eval_smem_bytes(int B, int D, int HP) {
   const size_t norm = ((size_t)D * 8 + 15) & ~(size_t)15;
-  return norm + (size_t)eval_pi_words(D, HP) * 4 + (size_t)B * D * 4 + (size_t)HP * B * 4;
+  return norm + (size_t)policy_net_words((int64_t)D, HP) * 4 + (size_t)B * D * 4 + (size_t)HP * B * 4;
 }
 
 // out[j] = b[j] + sum_i w[i][j] x_i for the kEvChunk outputs starting at w / b (row stride HP), in input order
@@ -145,7 +142,7 @@ __global__ void __maxnreg__(168) k_evaluate(const __grid_constant__ KArgs<float>
   extern __shared__ __align__(16) unsigned char smem[];
   float2* norm = reinterpret_cast<float2*>(smem);
   float* img = reinterpret_cast<float*>(smem + (((size_t)D * 8 + 15) & ~(size_t)15));
-  const int64_t piw = eval_pi_words(D, HP);
+  const int64_t piw = policy_net_words((int64_t)D, HP);
   float* tile = img + piw;
   float* hid = tile + (size_t)B * D;
   // normaliser as k_policy stages it: (mean, 1 / (std + eps)), correctly rounded
@@ -221,8 +218,8 @@ static cudaError_t launch_evaluate(const KArgs<float>& ka, EvalArgs& p, int sms,
   int64_t best_warps = -1;
   for (int B = 32; B <= 256; B *= 2) {
     const size_t smem = eval_smem_bytes(B, p.D, p.HP);
-    if (smem > (size_t)227 * 1024) break;
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kMaxSmemBytes) break;
+    cudaError_t e = opt_in_smem(kern, ka.b.device, smem);
     if (e != cudaSuccess) return e;
     int per_sm = 0;
     e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, B, smem);
@@ -234,8 +231,6 @@ static cudaError_t launch_evaluate(const KArgs<float>& ka, EvalArgs& p, int sms,
   }
   if (best_b == 0) return cudaErrorInvalidConfiguration;
   const size_t smem = eval_smem_bytes(best_b, p.D, p.HP);
-  cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  if (e != cudaSuccess) return e;
   p.blocks_per_policy = (p.E + best_b - 1) / best_b;
   kern<<<(unsigned)((int64_t)p.P * p.blocks_per_policy), best_b, smem, st>>>(ka, p);
   return cudaGetLastError();
@@ -274,30 +269,23 @@ extern "C" int pdx_evaluate(const PdxConfig* cfg, const PdxBuffers* buf, const P
   if (set->obs_dim != c.obs_dim || set->hidden[0] < 1 || set->hidden[0] > 64 || set->hidden[1] < 1 || set->hidden[1] > 64 ||
       set->n_out < 1 || set->n_out > 4)
     return set_error(PDX_ERR_INVALID, "pdx_evaluate: actor must match obs_dim, with two hidden layers of <= 64 units and <= 4 outputs");
-  const int HP = (set->hidden[0] <= 52 && set->hidden[1] <= 52) ? 52 : 64;
-  if (!set->packed || set->stride < eval_pi_words(c.obs_dim, HP) || (set->stride & 3) || (!set->mean) != (!set->std))
+  const int HP = policy_actor_pad(set->hidden[0], set->hidden[1]);
+  if (!set->packed || set->stride < policy_net_words((int64_t)c.obs_dim, HP) || (set->stride & 3) || (!set->mean) != (!set->std))
     return set_error(PDX_ERR_INVALID, "pdx_evaluate: packed images of pdx_policy_pack (stride >= the actor's words, a multiple of 4) "
                                       "and mean / std both given or both NULL are required");
   const bool rec = out->rec_obs || out->rec_act || out->rec_reward || out->rec_cost || out->rec_terminated || out->rec_truncated;
   if (!out->ret || !out->cost || !out->length ||
       (rec && !(out->rec_obs && out->rec_act && out->rec_reward && out->rec_cost && out->rec_terminated && out->rec_truncated)))
     return set_error(PDX_ERR_INVALID, "pdx_evaluate: ret / cost / length are required, the record buffers all or none");
-  if (eval_smem_bytes(32, c.obs_dim, HP) > (size_t)227 * 1024)
+  if (eval_smem_bytes(32, c.obs_dim, HP) > kMaxSmemBytes)
     return set_error(PDX_ERR_INVALID, "pdx_evaluate: obs_dim too wide for the shared-memory plan");
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) { cudaGetLastError(); return set_error(PDX_ERR_NO_DEVICE, "no CUDA device; this library has no CPU path"); }
-  if (buf->device < 0 || buf->device >= ndev) return set_error(PDX_ERR_INVALID, "bad device ordinal");
-  if (cudaSetDevice(buf->device) != cudaSuccess) return set_error(PDX_ERR_CUDA, "cudaSetDevice failed");
+  const int rc = select_device(buf->device);
+  if (rc) return rc;
   c.auto_reset = 0;                                           // an evaluation episode is not reset
-  KArgs<float> ka;
-  fill_devcfg<float>(c, ka.c);
-  ka.b = *buf;
+  KArgs<float> ka = make_kargs<float>(c, *buf, seed, counter, c.max_episode_steps);
   ka.b.obs = ka.b.reward = ka.b.cost = ka.b.final_obs = ka.b.episode_return = nullptr;
   ka.b.terminated = ka.b.truncated = nullptr; ka.b.episode_length = nullptr; ka.b.episode_stats = nullptr;
   ka.b.tape_step = ka.b.tape_reset = ka.b.tape_init = nullptr;
-  ka.actions = nullptr; ka.mask = nullptr; ka.seed = seed; ka.counter = counter;
-  ka.dump_step = ka.dump_reset = ka.dump_init = nullptr;
-  ka.n_steps = c.max_episode_steps; ka.n_tiles = 1;
   EvalArgs p;
   p.P = (int32_t)P; p.E = (int32_t)E; p.D = c.obs_dim; p.h1 = set->hidden[0]; p.h2 = set->hidden[1]; p.HP = HP;
   p.n_steps = c.max_episode_steps; p.blocks_per_policy = 1;
@@ -314,10 +302,5 @@ extern "C" int pdx_evaluate(const PdxConfig* cfg, const PdxBuffers* buf, const P
   if (c.task == PDX_TASK_HOVER) e = launch_evaluate_task<PDX_TASK_HOVER>(c, ka, p, sms, st);
   else if (c.task == PDX_TASK_CIRCLE) e = launch_evaluate_task<PDX_TASK_CIRCLE>(c, ka, p, sms, st);
   else e = launch_evaluate_task<PDX_TASK_TAKEOFF>(c, ka, p, sms, st);
-  if (e != cudaSuccess) {
-    char msg[256];
-    std::snprintf(msg, sizeof(msg), "pdx_evaluate: CUDA error: %s", cudaGetErrorString(e));
-    return set_error(PDX_ERR_CUDA, msg);
-  }
-  return PDX_OK;
+  return cuda_error("pdx_evaluate", e);
 }

@@ -104,6 +104,14 @@ constexpr Layout make_layout(int task, int physics, bool noise, bool pid = false
   return L;
 }
 
+// Image of pdx_policy_pack: the actor's net, then the critic's, each W1t[D][H], b1[H], W2t[H][H], b2[H], W3t[H][4],
+// b3[4] with the hidden width zero padded to H.  k_policy stages the whole image, k_evaluate the actor's net.
+// Words of one net, in the type of D: k_policy computes its shared-memory offsets in int, the ABI in int64_t.
+template <class I>
+constexpr I policy_net_words(I D, int H) { return D * H + H + H * H + H + H * 4 + 4; }
+// H of the actor's net (the critic's is 64)
+constexpr int policy_actor_pad(int h1, int h2) { return (h1 <= 52 && h2 <= 52) ? 52 : 64; }
+
 // Tape slot counts (reference draw order; SURVEY 3.3 / A.5).
 struct TapeSlots {
   int init, reset, step;

@@ -6,6 +6,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
+#include "../../include/phoenix_b200.h"
 
 namespace pdx {
 
@@ -130,6 +131,16 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 ctr, uint2 key) {
     key.y += W1;
   }
   return ctr;
+}
+
+// The policy's action noise: four standard normals for (seed, counter, env), from one Philox call on the counter
+// (env_lo, counter, env_hi, "POL") and two float32 Box-Muller pairs.  k_policy, k_policy_tc and k_collect all draw
+// it here, so they sample identical actions for the same (seed, counter, env).
+__device__ __forceinline__ void policy_normals(uint64_t seed, uint64_t counter, uint64_t env, float eps[4]) {
+  const uint4 r = philox4x32_10(make_uint4((uint32_t)env, (uint32_t)counter, (uint32_t)(env >> 32), 0x504F4Cu),
+                                make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
+  M<float>::box_muller(r.x, r.y, &eps[0], &eps[1]);
+  M<float>::box_muller(r.z, r.w, &eps[2], &eps[3]);
 }
 
 // Draw-site ids (4th counter word).  One Philox call per site id yields 4 words; a draw block

@@ -34,12 +34,8 @@
 // x = hi + lo (hi = tf32(x), lo = x - hi) and accumulates A_lo*B_hi + A_hi*B_lo + A_hi*B_hi into the
 // same fp32 TMEM accumulator (the dropped lo*lo term is 2^-22 relative): float32-level results at
 // three times the (cheap) MMA cost, which is what the parity tests pin against torch.
-#include <cuda_runtime.h>
-#include <cstdint>
-#include <cstdio>
-#include "../../include/phoenix_b200.h"
-#include "pdx_error.h"
-
+#include "pdx_host.h"
+#include "pdx_math.cuh"
 #include "pdx_tc.cuh"
 
 namespace {
@@ -490,11 +486,7 @@ __global__ void __launch_bounds__(TcCfg<X3>::kThreads + 32, TcCfg<X3>::kMinBlock
       // same (seed, counter, env).
       float eps[4] = {0.f, 0.f, 0.f, 0.f}, lp = 0.0f;
       if (cg == 0) {
-        const uint64_t i = (uint64_t)(a.env_offset + env0 + row);
-        const uint4 rr = tc_philox(make_uint4((uint32_t)i, (uint32_t)a.counter, (uint32_t)(i >> 32), 0x504F4Cu),
-                                   make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-        pdx_policy_box_muller(rr.x, rr.y, &eps[0], &eps[1]);
-        pdx_policy_box_muller(rr.z, rr.w, &eps[2], &eps[3]);
+        pdx::policy_normals(a.seed, a.counter, (uint64_t)(a.env_offset + env0 + row), eps);
 #pragma unroll
         for (int k = 0; k < 4; ++k)
           if (k < a.act_dim) lp += -0.5f * eps[k] * eps[k] - act_std[4 + k] - 0.9189385332046727f;
@@ -551,35 +543,13 @@ size_t tc_smem_bytes(int k1, int obs_dim, bool x3) {
          nb * (k1 / 4) * kLboA + (size_t)kTile * obs_dim * 4;
 }
 
-int tc_select_device_of(const void* ptr) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    return pdx::set_error(PDX_ERR_NO_DEVICE, "no CUDA device; this library has no CPU path");
-  }
-  cudaPointerAttributes attr;
-  if (cudaPointerGetAttributes(&attr, ptr) != cudaSuccess || attr.type != cudaMemoryTypeDevice) {
-    cudaGetLastError();
-    return pdx::set_error(PDX_ERR_INVALID, "buffer is not device memory");
-  }
-  return cudaSetDevice(attr.device) == cudaSuccess ? PDX_OK : pdx::set_error(PDX_ERR_CUDA, "cudaSetDevice failed");
-}
-
-int tc_status(const char* what) {
-  const cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) return PDX_OK;
-  char msg[256];
-  snprintf(msg, sizeof(msg), "%s: CUDA error: %s", what, cudaGetErrorString(e));
-  return pdx::set_error(PDX_ERR_CUDA, msg);
-}
-
 bool tc_shapes_ok(int32_t obs_dim, const PdxMlp* pi, const PdxMlp* v, int32_t precision) {
   if (obs_dim <= 0 || !pi || !v || (precision != 1 && precision != 3)) return false;
   if (pi->hidden[0] < 1 || pi->hidden[0] > 64 || pi->hidden[1] < 1 || pi->hidden[1] > 64 || pi->n_out < 1 || pi->n_out > 4) return false;
   if (v->hidden[0] < 1 || v->hidden[0] > 64 || v->hidden[1] < 1 || v->hidden[1] > 64 || v->n_out != 1) return false;
   const int k1 = tc_k1(obs_dim);
   if (k1 > 64) return false;                              // sixteen lanes walk the K chunks of a row (stage_to_x)
-  return tc_smem_bytes(k1, obs_dim, precision == 3) <= (size_t)227 * 1024;
+  return tc_smem_bytes(k1, obs_dim, precision == 3) <= pdx::kMaxSmemBytes;
 }
 
 }  // namespace
@@ -600,7 +570,7 @@ extern "C" int64_t pdx_policy_tc_pack_words(int32_t obs_dim, const PdxMlp* pi, c
 extern "C" int pdx_policy_tc_pack(int32_t obs_dim, const PdxMlp* pi, const PdxMlp* v, int32_t precision, float* packed, void* stream) {
   if (!packed || !tc_shapes_ok(obs_dim, pi, v, precision))
     return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_tc_pack: null buffer or shapes outside the tensor-core plan");
-  const int rc = tc_select_device_of(packed);
+  const int rc = pdx::select_device_of(packed);
   if (rc) return rc;
   PackArgs p;
   p.obs_dim = obs_dim; p.k1 = tc_k1(obs_dim); p.x3 = precision == 3;
@@ -608,7 +578,7 @@ extern "C" int pdx_policy_tc_pack(int32_t obs_dim, const PdxMlp* pi, const PdxMl
   for (int k = 0; k < 3; ++k) { p.pi_w[k] = pi->weight[k]; p.pi_b[k] = pi->bias[k]; p.v_w[k] = v->weight[k]; p.v_b[k] = v->bias[k]; }
   p.out = packed;
   k_pack_tc<<<16, 256, 0, (cudaStream_t)stream>>>(p);
-  return tc_status("pdx_policy_tc_pack");
+  return pdx::cuda_error("pdx_policy_tc_pack", cudaGetLastError());
 }
 
 extern "C" int pdx_policy_step_tc(int64_t n, int32_t obs_dim, const float* obs, const float* mean, const float* std, float eps,
@@ -619,7 +589,8 @@ extern "C" int pdx_policy_step_tc(int64_t n, int32_t obs_dim, const float* obs, 
   precision &= ~PDX_POLICY_TC_OVERLAP;
   if (n <= 0 || !obs || !log_std || !packed || !actions || !values || !logp || !tc_shapes_ok(obs_dim, pi, v, precision))
     return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_tc: null buffer, n <= 0 or shapes outside the tensor-core plan");
-  const int rc = tc_select_device_of(obs);
+  int dev = 0;
+  int rc = pdx::select_device_of(obs, &dev);
   if (rc) return rc;
   const bool x3 = precision == 3;
   TcArgs a;
@@ -629,30 +600,16 @@ extern "C" int pdx_policy_step_tc(int64_t n, int32_t obs_dim, const float* obs, 
   a.seed = seed; a.counter = counter; a.env_offset = env_offset; a.act = actions; a.val = values; a.logp = logp; a.mu = mu_out;
   a.n_tiles = (n + kTile - 1) / kTile;
   const size_t smem = tc_smem_bytes(a.k1, obs_dim, x3);
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static size_t set_by_dev[2][64] = {};              // opt-in dynamic shared memory, per device and variant
-  size_t& set_ref = set_by_dev[x3][dev & 63];
-  if (smem > set_ref) {
-    const cudaError_t e = x3 ? cudaFuncSetAttribute(k_policy_tc<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem)
-                             : cudaFuncSetAttribute(k_policy_tc<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    if (e != cudaSuccess) return tc_status("pdx_policy_step_tc (shared-memory opt-in)");
-    set_ref = smem;
-  }
+  auto kern = x3 ? k_policy_tc<true> : k_policy_tc<false>;
+  rc = pdx::cuda_error("pdx_policy_step_tc (shared-memory opt-in)", pdx::opt_in_smem(kern, dev, smem));
+  if (rc) return rc;
   int sms = 148;
   cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
   // persistent CTAs: TMEM (512 columns per SM) admits one precision-3 CTA or two precision-1 CTAs per SM
-  const int64_t resident = (int64_t)sms * (x3 ? 1 : ((size_t)2 * smem <= (size_t)227 * 1024 ? 2 : 1));
+  const int64_t resident = (int64_t)sms * (x3 ? 1 : (2 * smem <= pdx::kMaxSmemBytes ? 2 : 1));
   const unsigned grid = (unsigned)(a.n_tiles < resident ? a.n_tiles : resident);
-  // programmatic stream serialisation: the grid may start while its predecessor drains (see the kernel)
-  cudaLaunchConfig_t lc = {};
-  lc.gridDim = dim3(grid); lc.blockDim = dim3((x3 ? TcCfg<true>::kThreads : TcCfg<false>::kThreads) + 32);
-  lc.dynamicSmemBytes = smem; lc.stream = (cudaStream_t)stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-  attr[0].val.programmaticStreamSerializationAllowed = 1;
-  lc.attrs = attr; lc.numAttrs = 1;
-  const cudaError_t le = x3 ? cudaLaunchKernelEx(&lc, k_policy_tc<true>, a) : cudaLaunchKernelEx(&lc, k_policy_tc<false>, a);
-  if (le != cudaSuccess) { cudaGetLastError(); return pdx::set_error(PDX_ERR_CUDA, cudaGetErrorString(le)); }
-  return tc_status("pdx_policy_step_tc");
+  // the grid may start while its predecessor drains (see the kernel)
+  const int block = (x3 ? TcCfg<true>::kThreads : TcCfg<false>::kThreads) + 32;
+  const cudaError_t e = pdx::launch_early(kern, grid, block, smem, (cudaStream_t)stream, true, a);
+  return pdx::cuda_error("pdx_policy_step_tc", e != cudaSuccess ? e : cudaGetLastError());
 }

@@ -5,10 +5,9 @@
 //               restarts the recursions at episode boundaries.
 //   pdx_moments restates the per-rank sums behind OnlineMeanStd.update
 //               (utils/online_mean_std.py:70-84): sum x and sum (x - shift)^2 per column.
-#include <cuda_runtime.h>
-#include <cstdio>
-#include "../../include/phoenix_b200.h"
-#include "pdx_error.h"
+#include "pdx_host.h"
+#include "pdx_layout.h"
+#include "pdx_math.cuh"
 
 namespace {
 
@@ -128,30 +127,6 @@ __global__ void k_oms_update(int dim, const double* __restrict__ s1, const doubl
   }
 }
 
-// The library carries its own static CUDA runtime: select the device the data lives on.
-int select_device_of(const void* ptr, int* dev_out = nullptr) {
-  int ndev = 0;
-  if (cudaGetDeviceCount(&ndev) != cudaSuccess || ndev == 0) {
-    cudaGetLastError();
-    return pdx::set_error(PDX_ERR_NO_DEVICE, "no CUDA device; this library has no CPU path");
-  }
-  cudaPointerAttributes attr;
-  if (cudaPointerGetAttributes(&attr, ptr) != cudaSuccess || attr.type != cudaMemoryTypeDevice) {
-    cudaGetLastError();
-    return pdx::set_error(PDX_ERR_INVALID, "buffer is not device memory");
-  }
-  if (dev_out) *dev_out = attr.device;
-  return cudaSetDevice(attr.device) == cudaSuccess ? PDX_OK : pdx::set_error(PDX_ERR_CUDA, "cudaSetDevice failed");
-}
-
-int launch_status(const char* what) {
-  const cudaError_t e = cudaGetLastError();
-  if (e == cudaSuccess) return PDX_OK;
-  char msg[256];
-  std::snprintf(msg, sizeof(msg), "%s: CUDA error: %s", what, cudaGetErrorString(e));
-  return pdx::set_error(PDX_ERR_CUDA, msg);
-}
-
 }  // namespace
 
 extern "C" int pdx_gae(int64_t T, int64_t n, const float* rew, const float* val, const uint8_t* done,
@@ -161,19 +136,19 @@ extern "C" int pdx_gae(int64_t T, int64_t n, const float* rew, const float* val,
   if (T <= 0 || n <= 0) return pdx::set_error(PDX_ERR_INVALID, "pdx_gae: T and n must be positive");
   if (!rew || !val || !done || !boot_val || !last_val || !adv || !target_v || !disc_ret)
     return pdx::set_error(PDX_ERR_INVALID, "pdx_gae: null buffer");
-  const int rc = select_device_of(rew);
+  const int rc = pdx::select_device_of(rew);
   if (rc) return rc;
   const unsigned grid = (unsigned)((n + 127) / 128);
   k_gae<<<grid, 128, 0, (cudaStream_t)stream>>>(T, n, rew, val, done, boot_val, last_val, gamma, lam,
                                                 ret_scale, use_reward_scaling, ret_std_dev, adv, target_v, disc_ret);
-  return launch_status("pdx_gae");
+  return pdx::cuda_error("pdx_gae", cudaGetLastError());
 }
 
 extern "C" int pdx_moments(int64_t rows, int32_t dim, const float* x, const double* shift, double* out,
                            void* stream) {
   if (rows <= 0 || dim <= 0 || dim > 1024) return pdx::set_error(PDX_ERR_INVALID, "pdx_moments: rows must be positive and dim in [1, 1024]");
   if (!x || !out) return pdx::set_error(PDX_ERR_INVALID, "pdx_moments: null buffer");
-  const int rc = select_device_of(x);
+  const int rc = pdx::select_device_of(x);
   if (rc) return rc;
   // blockDim = (dim, rows per block): thread (y, x) reads x[row * dim + x], so the linear thread id
   // walks the row-major matrix contiguously -- every lane of every warp is busy whatever dim is
@@ -184,7 +159,7 @@ extern "C" int pdx_moments(int64_t rows, int32_t dim, const float* x, const doub
   const unsigned grid = (unsigned)(tiles < 2368 ? tiles : 2368);      // 16 x 148 SMs
   const size_t smem = 2ull * bx * by * sizeof(double);
   k_moments<<<grid, block, smem, (cudaStream_t)stream>>>(rows, dim, x, shift, out);
-  return launch_status("pdx_moments");
+  return pdx::cuda_error("pdx_moments", cudaGetLastError());
 }
 
 extern "C" int pdx_oms_update(int32_t dim, const double* s1, const double* s2, double rows, int32_t world, const float* shift,
@@ -192,21 +167,21 @@ extern "C" int pdx_oms_update(int32_t dim, const double* s1, const double* s2, d
                               void* stream) {
   if (dim <= 0 || !s1 || !s2 || rows <= 0 || world < 1 || !batch_mean || !batch_var || !mean || !std || !count || phase < 0 || phase > 3)
     return pdx::set_error(PDX_ERR_INVALID, "pdx_oms_update: bad argument");
-  const int rc = select_device_of(mean);
+  const int rc = pdx::select_device_of(mean);
   if (rc) return rc;
   const unsigned grid = (unsigned)((dim + 127) / 128);
   k_oms_update<<<grid, 128, 0, (cudaStream_t)stream>>>(dim, s1, s2, rows, (double)world, shift, batch_mean, batch_var, mean, std, count, phase);
   if (phase >= 2)
     k_oms_update<<<1, 32, 0, (cudaStream_t)stream>>>(dim, s1, s2, rows, (double)world, shift, batch_mean, batch_var, mean, std, count, 4);
-  return launch_status("pdx_oms_update");
+  return pdx::cuda_error("pdx_oms_update", cudaGetLastError());
 }
 
 extern "C" int pdx_stats_combine(int32_t world, const double* gathered, double* out, void* stream) {
   if (world <= 0 || !gathered || !out) return pdx::set_error(PDX_ERR_INVALID, "pdx_stats_combine: bad argument");
-  const int rc = select_device_of(gathered);
+  const int rc = pdx::select_device_of(gathered);
   if (rc) return rc;
   k_stats_combine<<<1, 32, 0, (cudaStream_t)stream>>>(world, gathered, out);
-  return launch_status("pdx_stats_combine");
+  return pdx::cuda_error("pdx_stats_combine", cudaGetLastError());
 }
 
 // =============================================================================================
@@ -223,18 +198,6 @@ namespace {
 
 constexpr int kPolBlock = 256;
 constexpr int kHidMax = 64;
-
-__device__ __forceinline__ uint4 pol_philox(uint4 ctr, uint2 key) {
-  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(M0, ctr.x), lo0 = M0 * ctr.x;
-    const uint32_t hi1 = __umulhi(M1, ctr.z), lo1 = M1 * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += W0; key.y += W1;
-  }
-  return ctr;
-}
 
 // tanh(x) = 1 - 2 / (exp(2x) + 1): two MUFU operations, ~1e-6 absolute error (tanhf costs ~30
 // instructions and there are 128 activations per environment).
@@ -307,7 +270,7 @@ __device__ __forceinline__ void run_net(const float* __restrict__ sm_net, const 
 template <int HP, int HV>
 __global__ void k_pack_policy(const PolArgs a, float* __restrict__ out) {
   const int D = a.obs_dim;
-  const int pi_words = D * HP + HP + HP * HP + HP + HP * 4 + 4;
+  const int pi_words = pdx::policy_net_words(D, HP);
   auto pack = [&](float* net, int H, const float* const* w, const float* const* b, int h1, int h2, int n_out) {
     float* w1 = net; float* b1 = w1 + D * H; float* w2 = b1 + H; float* b2 = w2 + H * H; float* w3 = b2 + H; float* b3 = w3 + H * 4;
     const int tid = blockIdx.x * blockDim.x + threadIdx.x, nt = gridDim.x * blockDim.x;
@@ -328,9 +291,9 @@ __global__ void __launch_bounds__(kPolBlock) k_policy(const PolArgs a) {
   float* nmean = pol_sm;
   float* ninv = nmean + ((D + 3) & ~3);
   float* pi_net = ninv + ((D + 3) & ~3);
-  const int pi_words = D * HP + HP + HP * HP + HP + HP * 4 + 4;
+  const int pi_words = pdx::policy_net_words(D, HP);
   float* v_net = pi_net + pi_words;
-  const int v_words = D * HV + HV + HV * HV + HV + HV * 4 + 4;
+  const int v_words = pdx::policy_net_words(D, HV);
   float* hid = v_net + v_words;
   // ---- stage the normaliser and the packed (zero padded, transposed) weights: a flat copy of the
   // blob k_pack_policy prepared (layout == the shared-memory plan from pi_net on)
@@ -351,27 +314,8 @@ __global__ void __launch_bounds__(kPolBlock) k_policy(const PolArgs a) {
   run_net<HP>(pi_net, row, nmean, ninv, D, a.pi_h1, a.pi_h2, false, hid, tid, mu);
   run_net<HV>(v_net, row, nmean, ninv, D, a.v_h1, a.v_h2, true, hid, tid, vv);
   // ---- sample: a = mu + std * eps, log p = sum(-eps^2/2 - log_std - log(2 pi)/2)
-  const uint64_t ig = (uint64_t)(a.env_offset + i);
-  const uint4 r = pol_philox(make_uint4((uint32_t)ig, (uint32_t)a.counter, (uint32_t)(ig >> 32), 0x504F4Cu),
-                             make_uint2((uint32_t)a.seed, (uint32_t)(a.seed >> 32)));
-  // Box-Muller with single MUFU operations (lg2, sqrt, sin, cos) -- the construction of the float32 step
-  // kernel (pdx_math.cuh) and of k_policy_tc, so both policy kernels draw identical actions
   float eps[4];
-  {
-    const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
-#pragma unroll
-    for (int p = 0; p < 2; ++p) {
-      const float u1 = 2.0f - __uint_as_float(0x3f800000u | (rw[2 * p] >> 9));       // (0,1]
-      const float u2 = __uint_as_float(0x3f800000u | (rw[2 * p + 1] >> 9)) - 1.0f;   // [0,1)
-      float l2, rad, sn, cs;
-      asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l2) : "f"(u1));
-      asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(rad) : "f"(-1.3862943611198906f * l2));
-      const float ang = 6.283185307179586f * u2;
-      asm("sin.approx.ftz.f32 %0, %1;" : "=f"(sn) : "f"(ang));
-      asm("cos.approx.ftz.f32 %0, %1;" : "=f"(cs) : "f"(ang));
-      eps[2 * p] = rad * cs; eps[2 * p + 1] = rad * sn;
-    }
-  }
+  pdx::policy_normals(a.seed, a.counter, (uint64_t)(a.env_offset + i), eps);
   float lp = 0.0f;
   float4 act = make_float4(0.f, 0.f, 0.f, 0.f);
   float* av = reinterpret_cast<float*>(&act);
@@ -390,27 +334,21 @@ __global__ void __launch_bounds__(kPolBlock) k_policy(const PolArgs a) {
 }
 
 template <int HP, int HV>
-int launch_policy(const PolArgs& a, cudaStream_t st) {
+int launch_policy(const PolArgs& a, int dev, cudaStream_t st) {
   const int D = a.obs_dim;
-  const size_t words = 2 * ((D + 3) & ~3) + (size_t)(D * HP + HP + HP * HP + HP + HP * 4 + 4) +
-                       (size_t)(D * HV + HV + HV * HV + HV + HV * 4 + 4) + (size_t)kHidMax * kPolBlock;
+  const size_t words = 2 * ((D + 3) & ~3) + (size_t)pdx::policy_net_words(D, HP) + (size_t)pdx::policy_net_words(D, HV) +
+                       (size_t)kHidMax * kPolBlock;
   const size_t smem = words * sizeof(float);
   if (a.n == 0) {                                     // pack only (pdx_evaluate stages the actor part of wider images)
     k_pack_policy<HP, HV><<<8, 256, 0, st>>>(a, const_cast<float*>(a.packed));
-    return launch_status("pdx_policy_pack");
+    return pdx::cuda_error("pdx_policy_pack", cudaGetLastError());
   }
-  if (smem > (size_t)227 * 1024) return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step: obs_dim too wide for the shared-memory plan");
-  int dev = 0;
-  cudaGetDevice(&dev);
-  static size_t set_by_dev[64] = {};                  // opt-in dynamic shared memory is a per-device attribute
-  if (smem > set_by_dev[dev & 63]) {
-    if (cudaFuncSetAttribute(k_policy<HP, HV>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess)
-      return launch_status("pdx_policy_step (shared-memory opt-in)");
-    set_by_dev[dev & 63] = smem;
-  }
+  if (smem > pdx::kMaxSmemBytes) return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step: obs_dim too wide for the shared-memory plan");
+  const int rc = pdx::cuda_error("pdx_policy_step (shared-memory opt-in)", pdx::opt_in_smem(k_policy<HP, HV>, dev, smem));
+  if (rc) return rc;
   const unsigned grid = (unsigned)((a.n + kPolBlock - 1) / kPolBlock);
   k_policy<HP, HV><<<grid, kPolBlock, smem, st>>>(a);
-  return launch_status("pdx_policy_step");
+  return pdx::cuda_error("pdx_policy_step", cudaGetLastError());
 }
 
 }  // namespace
@@ -421,8 +359,7 @@ static int policy_dispatch(int64_t n, int32_t obs_dim, const float* obs, const f
 
 extern "C" int64_t pdx_policy_pack_words(int32_t obs_dim, const PdxMlp* pi, const PdxMlp* v) {
   if (obs_dim <= 0 || !pi || !v) return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_pack_words: bad argument");
-  const int64_t D = obs_dim, HP = (pi->hidden[0] <= 52 && pi->hidden[1] <= 52) ? 52 : 64, HV = 64;
-  return (D * HP + HP + HP * HP + HP + HP * 4 + 4) + (D * HV + HV + HV * HV + HV + HV * 4 + 4);
+  return pdx::policy_net_words((int64_t)obs_dim, pdx::policy_actor_pad(pi->hidden[0], pi->hidden[1])) + pdx::policy_net_words((int64_t)obs_dim, 64);
 }
 
 extern "C" int pdx_policy_pack(int32_t obs_dim, const PdxMlp* pi, const PdxMlp* v, float* packed, void* stream) {
@@ -446,7 +383,8 @@ static int policy_dispatch(int64_t n, int32_t obs_dim, const float* obs, const f
     return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step: actor must have two hidden layers of <= 64 units and <= 4 outputs");
   if (v->hidden[0] < 1 || v->hidden[0] > kHidMax || v->hidden[1] < 1 || v->hidden[1] > kHidMax || v->n_out != 1)
     return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step: critic must have two hidden layers of <= 64 units and one output");
-  const int rc = select_device_of(obs);
+  int dev = 0;
+  const int rc = pdx::select_device_of(obs, &dev);
   if (rc) return rc;
   PolArgs a;
   a.n = n; a.obs_dim = obs_dim; a.act_dim = pi->n_out;
@@ -455,6 +393,6 @@ static int policy_dispatch(int64_t n, int32_t obs_dim, const float* obs, const f
   for (int k = 0; k < 3; ++k) { a.pi_w[k] = pi->weight[k]; a.pi_b[k] = pi->bias[k]; a.v_w[k] = v->weight[k]; a.v_b[k] = v->bias[k]; }
   a.log_std = log_std; a.packed = packed; a.seed = seed; a.counter = counter; a.env_offset = env_offset;
   a.act = actions; a.val = values; a.logp = logp; a.mu = mu_out;
-  const bool pi_small = a.pi_h1 <= 52 && a.pi_h2 <= 52;
-  return pi_small ? launch_policy<52, 64>(a, (cudaStream_t)stream) : launch_policy<64, 64>(a, (cudaStream_t)stream);
+  const cudaStream_t st = (cudaStream_t)stream;
+  return pdx::policy_actor_pad(a.pi_h1, a.pi_h2) == 52 ? launch_policy<52, 64>(a, dev, st) : launch_policy<64, 64>(a, dev, st);
 }

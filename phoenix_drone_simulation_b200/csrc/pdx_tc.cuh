@@ -1,7 +1,6 @@
 // tcgen05 / TMEM / TMA building blocks shared by the tensor-core policy kernel (pdx_policy_tc.cu) and the fused
 // collector kernel (pdx_collect.cu): PTX wrappers, the canonical no-swizzle K-major operand layout, TF32
-// rounding, the MUFU Box-Muller and Philox used for the policy's action noise, and the layout of the packed
-// weight image (written by k_pack_tc in pdx_policy_tc.cu).
+// rounding and the layout of the packed weight image (written by k_pack_tc in pdx_policy_tc.cu).
 #pragma once
 #include <cuda_runtime.h>
 #include <cstdint>
@@ -132,34 +131,6 @@ __device__ __forceinline__ float tanh_mufu(float x) {
   asm("tanh.approx.f32 %0, %1;" : "=f"(y) : "f"(x));
   return y;
 }
-// Box-Muller on two 32-bit words with single MUFU operations (lg2, sqrt, sin, cos), the construction the
-// float32 step kernel uses (pdx_math.cuh); k_policy (pdx_rollout.cu) uses the same, so both policy kernels
-// draw identical actions for the same (seed, counter, env).
-__device__ __forceinline__ void pdx_policy_box_muller(uint32_t a, uint32_t b, float* z0, float* z1) {
-  const float u1 = 2.0f - __uint_as_float(0x3f800000u | (a >> 9));     // (0,1]
-  const float u2 = __uint_as_float(0x3f800000u | (b >> 9)) - 1.0f;     // [0,1)
-  float l2, r, s, c;
-  asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l2) : "f"(u1));
-  asm("sqrt.approx.ftz.f32 %0, %1;" : "=f"(r) : "f"(-1.3862943611198906f * l2));   // -2 ln u1
-  const float ang = 6.283185307179586f * u2;
-  asm("sin.approx.ftz.f32 %0, %1;" : "=f"(s) : "f"(ang));
-  asm("cos.approx.ftz.f32 %0, %1;" : "=f"(c) : "f"(ang));
-  *z0 = r * c;
-  *z1 = r * s;
-}
-
-__device__ __forceinline__ uint4 tc_philox(uint4 ctr, uint2 key) {
-  const uint32_t M0 = 0xD2511F53u, M1 = 0xCD9E8D57u, W0 = 0x9E3779B9u, W1 = 0xBB67AE85u;
-#pragma unroll
-  for (int r = 0; r < 10; ++r) {
-    const uint32_t hi0 = __umulhi(M0, ctr.x), lo0 = M0 * ctr.x;
-    const uint32_t hi1 = __umulhi(M1, ctr.z), lo1 = M1 * ctr.z;
-    ctr = make_uint4(hi1 ^ ctr.y ^ key.x, lo1, hi0 ^ ctr.w ^ key.y, lo0);
-    key.x += W0; key.y += W1;
-  }
-  return ctr;
-}
-
 
 // tanh(x) = 1 - 2 / (2^(2 log2(e) x) + 1): FMUL, MUFU.EX2, FADD, MUFU.RCP, FFMA; saturates correctly
 // (ex2 -> inf gives rcp -> 0) so no clamp is needed; ~1e-6 absolute error

@@ -139,6 +139,65 @@ def test_no_cpu_fallback(lib):
     assert lib.pdx_gae(4, 4, *([host.ctypes.data] * 5), 0.99, 0.95, 1.0, 0, None, *([host.ctypes.data] * 3), None) == -3
 
 
+COMPUTE_ENTRY_POINTS = ['pdx_init', 'pdx_reset', 'pdx_step', 'pdx_step_many', 'pdx_gae', 'pdx_moments', 'pdx_oms_update',
+                        'pdx_stats_combine', 'pdx_policy_pack', 'pdx_policy_step', 'pdx_policy_tc_pack', 'pdx_policy_step_tc',
+                        'pdx_collect', 'pdx_evaluate']
+
+
+def _mlp(h1, h2, n_out):
+    m = L.PdxMlp()
+    m.hidden[0], m.hidden[1], m.n_out = h1, h2, n_out
+    return m
+
+
+@pytest.mark.skipif(torch.cuda.is_available(), reason='checks the behaviour WITHOUT a GPU')
+@pytest.mark.parametrize('entry', COMPUTE_ENTRY_POINTS)
+def test_every_compute_entry_point_reports_no_device(lib, entry):
+    """With arguments that pass validation and no CUDA device, every compute entry point returns PDX_ERR_NO_DEVICE
+    and says there is no CPU path.  The pointers are never dereferenced: the device check comes first."""
+    F = 0x1000
+    c = pds.EnvConfig('DroneHoverSimpleEnv-v0').to_pdx()
+    D = c.obs_dim
+    b = L.PdxBuffers()
+    b.n_envs = 4
+    for f in ('state', 'obs', 'reward', 'cost', 'terminated', 'truncated'):
+        setattr(b, f, F)
+    pi, v = _mlp(50, 50, 4), _mlp(64, 64, 1)
+    pol = L.PdxPolicy()
+    pol.obs_dim, pol.precision, pol.pi, pol.v, pol.log_std, pol.packed = D, 1, C.pointer(pi), C.pointer(v), F, F
+    ro = L.PdxRollout()
+    ro.n_steps, ro.scratch_bytes = 8, 1 << 40
+    for f in ('obs0', 'act', 'val', 'logp', 'last_val', 'scratch'):
+        setattr(ro, f, F)
+    ps = L.PdxPolicySet()
+    ps.n_policies, ps.episodes, ps.obs_dim, ps.n_out, ps.stride, ps.packed = 2, 4, D, 4, 32 * 1024, F
+    ps.hidden[0], ps.hidden[1] = 50, 50
+    ev = L.PdxEvaluation()
+    ev.ret, ev.cost, ev.length = F, F, F
+    cfg, buf, pi_, v_ = C.byref(c), C.byref(b), C.byref(pi), C.byref(v)
+    calls = {
+        'pdx_init': lambda: lib.pdx_init(cfg, buf, 0, 1, None),
+        'pdx_reset': lambda: lib.pdx_reset(cfg, buf, None, 0, 1, None),
+        'pdx_step': lambda: lib.pdx_step(cfg, buf, F, 0, 1, None),
+        'pdx_step_many': lambda: lib.pdx_step_many(cfg, buf, F, 8, 0, 1, None),
+        'pdx_gae': lambda: lib.pdx_gae(8, 4, F, F, F, F, F, 0.99, 0.95, 1.0, 0, None, F, F, F, None),
+        'pdx_moments': lambda: lib.pdx_moments(4, D, F, None, F, None),
+        'pdx_oms_update': lambda: lib.pdx_oms_update(D, F, F, 4.0, 1, None, F, F, F, F, F, 3, None),
+        'pdx_stats_combine': lambda: lib.pdx_stats_combine(1, F, F, None),
+        'pdx_policy_pack': lambda: lib.pdx_policy_pack(D, pi_, v_, F, None),
+        'pdx_policy_step': lambda: lib.pdx_policy_step(4, D, F, None, None, 0.0, pi_, v_, F, F, 0, 1, 0, F, F, F, None, None),
+        'pdx_policy_tc_pack': lambda: lib.pdx_policy_tc_pack(D, pi_, v_, 1, F, None),
+        'pdx_policy_step_tc': lambda: lib.pdx_policy_step_tc(4, D, F, None, None, 0.0, pi_, v_, F, F, 1, 0, 1, 0, F, F, F, None,
+                                                             None),
+        'pdx_collect': lambda: lib.pdx_collect(cfg, buf, C.byref(pol), C.byref(ro), 0, 1, None),
+        'pdx_evaluate': lambda: lib.pdx_evaluate(cfg, buf, C.byref(ps), C.byref(ev), 0, 1, None),
+    }
+    assert sorted(calls) == sorted(COMPUTE_ENTRY_POINTS)
+    assert lib.pdx_step(cfg, C.byref(L.PdxBuffers()), None, 0, 0, None) == -1   # a message that is not the one expected
+    assert calls[entry]() == -3                                 # PDX_ERR_NO_DEVICE
+    assert b'no CPU path' in lib.pdx_last_error()
+
+
 def test_product_package_does_not_import_oracle():
     """The oracle is test infrastructure: nothing under the product package may reference it."""
     pkg = os.path.join(ROOT, 'phoenix_drone_simulation_b200')
