@@ -27,6 +27,8 @@ def main():
     p.add_argument('--num-envs', type=int, default=4096, help='per GPU')
     p.add_argument('--steps', type=int, default=64)
     p.add_argument('--seed', type=int, default=0)
+    p.add_argument('--update-kernel', default='torch', choices=['torch', 'cuda'],
+                   help="'cuda': losses and gradients of the update in the fused kernels pdx_ppo_pi_grad / pdx_ppo_v_grad")
     a = p.parse_args()
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
@@ -39,7 +41,8 @@ def main():
             os.environ['NCCL_DEBUG_FILE'] = '/dev/stderr'     # stdout carries the JSON lines
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
     from phoenix_drone_simulation_b200.ppo import PPO
-    alg = PPO(a.env, num_envs=a.num_envs, steps=a.steps, epochs=a.epochs, device=f'cuda:{local}', seed=a.seed, dist=dist)
+    alg = PPO(a.env, num_envs=a.num_envs, steps=a.steps, epochs=a.epochs, device=f'cuda:{local}', seed=a.seed, dist=dist,
+              update_kernel=a.update_kernel)
     for _ in range(a.epochs):
         row = alg.learn_one_epoch()
         if rank == 0:

@@ -355,6 +355,45 @@ typedef struct PdxEvaluation {
 int pdx_evaluate(const PdxConfig* cfg, const PdxBuffers* buf, const PdxPolicySet* set, const PdxEvaluation* out,
                  uint64_t seed, uint64_t counter, void* stream);
 
+/* ---- PPO update: losses and exact gradients of one network (algs/ppo/ppo.py:22-40, algs/iwpg/iwpg.py:398-485) ----
+ * csrc/pdx_ppo.cu, CUDA cores, float32 with float64 cross-CTA sums.  Weights come straight from the torch nn.Linear
+ * tensors through PdxMlp; gradients are written into caller tensors of the same shapes (p.grad), the loss as a float32
+ * device scalar.  Networks: two hidden layers of <= 64 units; obs_dim 1 .. 384.
+ *   pdx_ppo_pi_grad, actor (relu, 4 outputs, log_std fixed: it gets no gradient), per sample i of the batch:
+ *     mu = pi(obs), logp = sum_j (-((a - mu) / std)^2 / 2 - log_std - log(2 pi) / 2), r = exp(logp - logp_old),
+ *     loss = -mean(min(r A, clip(r, 1 - clip_ratio, 1 + clip_ratio) A)); d loss / d logp = -r A / n where
+ *     r A <= clip(r) A and 0 elsewhere (torch's minimum / clamp backward).  grad == NULL: forward only.  Optional
+ *     mu [n][4] receives pi(obs); with mu_ref [n][4] (and kl) kl = mean_i sum_j (mu_ref - mu)^2 / (2 std^2), the
+ *     Gaussian KL at equal std.
+ *   pdx_ppo_v_grad, critic (tanh, 1 output): loss = mean((v(obs) - target_v)^2).
+ * Row i of the batch is index[i] (index NULL: i) of obs / act / adv / logp_old / target_v; mu / mu_ref are indexed
+ * by i.  Indices must lie inside the caller's tensors (not checked).  scratch: device memory of
+ * pdx_ppo_scratch_bytes(device, obs_dim, net) bytes (net->n_out 4 = actor, 1 = critic); a smaller one, down to one
+ * CTA's partial sums, runs fewer CTAs.  Results are bit-identical from run to run for the same device, inputs and
+ * scratch size (fixed assignment of samples to CTAs, fixed summation order).  PDX_ERR_INVALID for unsupported shapes
+ * and bad arguments, before any device call. */
+typedef struct PdxMlpGrad {
+  float* weight[3];             /* [out][in], like PdxMlp.weight */
+  float* bias[3];
+} PdxMlpGrad;
+typedef struct PdxPpoBatch {
+  int64_t n;                    /* samples, >= 1 */
+  int32_t obs_dim;
+  int32_t reserved;
+  const float* obs;             /* [rows][obs_dim] standardised observations */
+  const int64_t* index;         /* optional [n]; NULL = rows 0 .. n-1 */
+  const float* act;             /* [rows][4]  actor  */
+  const float* adv;             /* [rows]     actor  */
+  const float* logp_old;        /* [rows]     actor  */
+  const float* target_v;        /* [rows]     critic */
+} PdxPpoBatch;
+int64_t pdx_ppo_scratch_bytes(int32_t device, int32_t obs_dim, const PdxMlp* net);
+int pdx_ppo_pi_grad(const PdxPpoBatch* batch, const PdxMlp* pi, const float* log_std, float clip_ratio,
+                    const PdxMlpGrad* grad, float* loss, float* mu, const float* mu_ref, float* kl,
+                    void* scratch, int64_t scratch_bytes, void* stream);
+int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const PdxMlpGrad* grad, float* loss,
+                   void* scratch, int64_t scratch_bytes, void* stream);
+
 /* Cross-rank combination of the 8-word episode statistics (utils/mpi_tools.py:217-240 does four
  * MPI all-reduces per key): the caller all-gathers the per-rank vectors into gathered[world][8]
  * (one NCCL call) and this writes out[0..4) = sums, out[4], out[6] = minima, out[5], out[7] = maxima. */

@@ -94,6 +94,16 @@ class PdxEvaluation(C.Structure):
                 ('rec_terminated', C.c_void_p), ('rec_truncated', C.c_void_p)]
 
 
+class PdxMlpGrad(C.Structure):
+    _fields_ = [('weight', C.c_void_p * 3), ('bias', C.c_void_p * 3)]
+
+
+class PdxPpoBatch(C.Structure):
+    _fields_ = [('n', C.c_int64), ('obs_dim', C.c_int32), ('reserved', C.c_int32), ('obs', C.c_void_p),
+                ('index', C.c_void_p), ('act', C.c_void_p), ('adv', C.c_void_p), ('logp_old', C.c_void_p),
+                ('target_v', C.c_void_p)]
+
+
 _lib = None
 
 
@@ -151,6 +161,12 @@ def load():
     lib.pdx_policy_tc_pack.argtypes = [C.c_int32, P(PdxMlp), P(PdxMlp), C.c_int32, C.c_void_p, C.c_void_p]
     lib.pdx_evaluate.argtypes = [P(PdxConfig), P(PdxBuffers), P(PdxPolicySet), P(PdxEvaluation), C.c_uint64, C.c_uint64,
                                  C.c_void_p]
+    lib.pdx_ppo_scratch_bytes.argtypes = [C.c_int32, C.c_int32, P(PdxMlp)]
+    lib.pdx_ppo_scratch_bytes.restype = C.c_int64
+    lib.pdx_ppo_pi_grad.argtypes = [P(PdxPpoBatch), P(PdxMlp), C.c_void_p, C.c_float, P(PdxMlpGrad), C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.pdx_ppo_v_grad.argtypes = [P(PdxPpoBatch), P(PdxMlp), P(PdxMlpGrad), C.c_void_p, C.c_void_p, C.c_int64,
+                                   C.c_void_p]
     if lib.pdx_abi_version() != ABI_VERSION:
         raise PhoenixB200Error(f'ABI mismatch: library {lib.pdx_abi_version()} != binding {ABI_VERSION}')
     if lib.pdx_config_size() != C.sizeof(PdxConfig) or lib.pdx_buffers_size() != C.sizeof(PdxBuffers):
@@ -171,5 +187,5 @@ EXPORTED_SYMBOLS = [
     'pdx_step_many', 'pdx_dump_draws',
     'pdx_gae', 'pdx_moments', 'pdx_stats_combine', 'pdx_policy_step', 'pdx_policy_pack', 'pdx_policy_pack_words',
     'pdx_policy_step_tc', 'pdx_policy_tc_pack', 'pdx_policy_tc_pack_words', 'pdx_collect', 'pdx_collect_scratch_bytes', 'pdx_oms_update',
-    'pdx_evaluate',
+    'pdx_evaluate', 'pdx_ppo_scratch_bytes', 'pdx_ppo_pi_grad', 'pdx_ppo_v_grad',
 ]
