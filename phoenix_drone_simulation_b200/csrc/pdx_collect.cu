@@ -94,18 +94,6 @@ __host__ __device__ inline ColSmem collect_smem(int k1, int D, int warps) {
 // live in a caller-provided global scratch buffer instead of shared memory (which the weight images need).
 __host__ __device__ inline size_t collect_scratch_per_cta(int threads) { return (size_t)threads * (4 * 8 + 4 * 4); }
 
-__device__ __forceinline__ bool tile_vote(int bar_id, int n_threads, bool pred) {
-  uint32_t out;
-  asm volatile(
-      "{\n\t.reg .pred p, q;\n\tsetp.ne.b32 p, %3, 0;\n\t"
-      "barrier.cta.red.or.pred q, %1, %2, p;\n\t"
-      "selp.u32 %0, 1, 0, q;\n\t}\n"
-      : "=r"(out)
-      : "r"(bar_id), "r"(n_threads), "r"((uint32_t)pred)
-      : "memory");
-  return out != 0;
-}
-
 template <int TASK, int PHYS, bool X3>
 __global__ void __launch_bounds__(512, 1) k_collect(const __grid_constant__ KArgs<float> a, const __grid_constant__ CollectArgs p) {
   typedef float T;

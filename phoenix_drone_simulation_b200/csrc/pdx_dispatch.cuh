@@ -60,30 +60,42 @@ static void fill_devcfg(const PdxConfig& p, DevCfg<T>& d) {
   d.ground_z = (T)p.ground_z;
 }
 
-// Launch shape of k_rollout: threads per block (<= 128 so that a 65,536-env shard still spreads
-// over all 148 SMs) and one or two observation tiles, chosen to maximise the warps resident per SM
-// under the shared-memory plan.  The kernel is compiled for 144 registers (no spills on the step path):
-// 64-thread blocks then fit 7 per SM = 14 warps, which is what a 65,536-env shard offers per SM
-// (13.8) -- warps of a block share nothing but the launch, so small blocks cost nothing;
-// ties go to double buffering, then to the larger block.
+// Launch shape of k_rollout for a shard of n environments on `sms` SMs: threads per block and one or two
+// observation tiles.  The kernel runs at 128 registers, so an SM holds 16 warps whatever the block size.
+//   * A shard that fits in one wave (every block resident at once; the block scheduler spreads them breadth
+//     first): blocks of 128 to 512 threads, the shape with the fewest warps on the busiest SM.  A launch
+//     lasts as long as its busiest SM, and the next launch waits for all of it.  65,536 environments in
+//     128-thread blocks are 512 blocks on 148 SMs, 68 SMs with 16 warps and 80 with 12; in 448-thread blocks
+//     they are one block of 14 warps per SM (measured on a B200: 393.6 -> 378.1 us per 64-step launch).
+//   * A larger shard: blocks of 128, 64 or 32 threads, the most warps resident per SM under the
+//     shared-memory plan.
+// Ties go to the larger block, then to double buffering.  A one-wave shard never takes blocks of fewer than 128
+// threads: their warps vote on package regeneration in groups of one to three and drift apart (measured at
+// 65,536 environments, where they balance as well as 448 threads: 64 threads 538 us, 32 threads 963 us per launch).
 struct LaunchShape { int block, tiles; size_t smem; };
 template <class T>
-static LaunchShape pick_shape(int D, int E, int wmode) {
-  LaunchShape best{0, 0, 0};
+static LaunchShape pick_shape(int D, int E, int wmode, int64_t n, int sms) {
+  LaunchShape best{0, 0, 0}, best_wave{0, 0, 0};
   int best_warps = -1;
-  const int blocks[3] = {128, 64, 32};
-  for (int bi = 0; bi < 3; ++bi) {
-    const int block = blocks[bi];
+  int64_t best_busiest = -1;
+  for (int block = 512; block >= 32; block -= 32) {
+    const bool classic = block == 128 || block == 64 || block == 32;
     for (int tiles = 2; tiles >= 1; --tiles) {
       const size_t smem = rollout_smem_bytes<T>(block, D, tiles, E, wmode);
       if (smem > kMaxSmemBytes) continue;
       const int by_smem = (int)(((size_t)228 * 1024) / (smem + 1024));
       const int by_regs = 65536 / (128 * block);
-      const int warps = (by_smem < by_regs ? by_smem : by_regs) * (block / 32);
-      if (warps > best_warps) { best_warps = warps; best = LaunchShape{block, tiles, smem}; }
+      const int per_sm = by_smem < by_regs ? by_smem : by_regs;
+      if (per_sm == 0) continue;
+      const int warps = per_sm * (block / 32);
+      if (classic && warps > best_warps) { best_warps = warps; best = LaunchShape{block, tiles, smem}; }
+      const int64_t grid = (n + block - 1) / block;
+      if (block < 128 || grid > (int64_t)per_sm * sms) continue;
+      const int64_t busiest = (grid + sms - 1) / sms * (block / 32);
+      if (best_busiest < 0 || busiest < best_busiest) { best_busiest = busiest; best_wave = LaunchShape{block, tiles, smem}; }
     }
   }
-  return best;
+  return best_busiest >= 0 ? best_wave : best;
 }
 
 template <class T, int TASK, int PHYS, bool NOISE, int RNG, bool PID>
@@ -108,7 +120,10 @@ static cudaError_t launch_kind(int kind, const KArgs<T>& ka, cudaStream_t st) {
     const int wv = atoi(e);
     if (wmode && (wv == 1 || (wv == 2 && quad_ok))) wmode = wv;
   }
-  const LaunchShape shape = pick_shape<T>(ka.c.obs_dim, ka.c.core_dim + 4, wmode);
+  int sms = 0;
+  const cudaError_t es = sm_count(ka.b.device, &sms);
+  if (es != cudaSuccess) return es;
+  const LaunchShape shape = pick_shape<T>(ka.c.obs_dim, ka.c.core_dim + 4, wmode, n, sms);
   if (shape.block == 0) return cudaErrorInvalidConfiguration;
   KArgs<T> kb = ka;
   kb.n_tiles = shape.tiles;

@@ -80,6 +80,18 @@ cudaError_t opt_in_smem(void (*kernel)(A...), int device, size_t bytes) {
   return opt_in_smem(reinterpret_cast<const void*>(kernel), device, bytes);
 }
 
+// Streaming multiprocessors of `device`, read once per device ordinal and kept for the whole library.
+inline cudaError_t sm_count(int device, int* sms) {
+  static std::mutex mu;
+  static std::map<int, int> known;
+  std::lock_guard<std::mutex> lock(mu);
+  auto it = known.find(device);
+  if (it != known.end()) { *sms = it->second; return cudaSuccess; }
+  const cudaError_t e = cudaDeviceGetAttribute(sms, cudaDevAttrMultiProcessorCount, device);
+  if (e == cudaSuccess) known[device] = *sms;
+  return e;
+}
+
 // Launches kernel(arg).  With `early`, programmatic stream serialisation: the grid may start while its predecessor
 // on the stream drains, so the kernel must wait (griddepcontrol.wait) before it touches anything the predecessor
 // could write.

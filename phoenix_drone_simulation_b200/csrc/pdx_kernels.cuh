@@ -563,6 +563,20 @@ __device__ __forceinline__ void block_reduce_episode_stats(double* gs, const dou
   }
 }
 
+// OR of `pred` over the `n_threads` threads (a multiple of 32) that meet at named barrier `bar_id` (1..15; 0 is
+// __syncthreads): the package vote of a 128-thread group in k_rollout and of a tile in k_collect
+__device__ __forceinline__ bool tile_vote(int bar_id, int n_threads, bool pred) {
+  uint32_t out;
+  asm volatile(
+      "{\n\t.reg .pred p, q;\n\tsetp.ne.b32 p, %3, 0;\n\t"
+      "barrier.cta.red.or.pred q, %1, %2, p;\n\t"
+      "selp.u32 %0, 1, 0, q;\n\t}\n"
+      : "=r"(out)
+      : "r"(bar_id), "r"(n_threads), "r"((uint32_t)pred)
+      : "memory");
+  return out != 0;
+}
+
 // ---- bulk asynchronous copy shared -> global (TMA engine), bulk-group completion ------------
 __device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
   const uint32_t s = (uint32_t)__cvta_generic_to_shared(ssrc);
@@ -992,7 +1006,8 @@ __device__ __forceinline__ void rollout_step(const KArgs<T>& a, Model<T, TASK, P
       }
     }
     if constexpr (POOL) {
-      // Package regeneration is decided per BLOCK, one barrier vote per step: all warps of a block run the
+      // Package regeneration is decided per vote group (`vote`: a 128-thread group of k_rollout's block, a tile
+      // of k_collect), one barrier vote per step: all warps of a group run the
       // (long) generator at the same step, and the barrier keeps them within one step of each other -- the
       // step loop is ~30 KB of straight-line code, and warps that drift apart each stream it through the
       // instruction caches on their own (measured: `no_instruction` became the top stall).  The vote
@@ -1097,8 +1112,9 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
   }
   // H = 2 with two tiles (the common case): the newest entry of a row is also the oldest entry of the NEXT
   // row, so every entry is written twice -- into this step's tile and into the next step's -- instead of
-  // being read back and shifted (17 LDS + their latency at the head of every step)
-  const bool fast2 = !wide && H == 2 && NT == 2;
+  // being read back and shifted (17 LDS + their latency at the head of every step).  Not in row mode 2: its
+  // history moves with 128-bit copies from the previous row, which the first step reads from tile1.
+  const bool fast2 = !wide && !quad && H == 2 && NT == 2;
   if (valid) {
     m.load(state, n, i);
     // history slots -> entries 1..H-1 of the "previous row" (tile1 plays the old tile at t = 0);
@@ -1126,6 +1142,7 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
   // rules of the bulk engine for every step (else: flat coalesced copy by the warp)
   sc.bulk = ((reinterpret_cast<uintptr_t>(a.b.obs) | (uintptr_t)((uint64_t)n * D * sizeof(T))) & 15u) == 0 &&
             (((uint64_t)max((int64_t)0, min((int64_t)32, n - (i - lane))) * D * sizeof(T)) & 15u) == 0;
+  const int vote_bar = 1 + (tid >> 7), vote_threads = min(128, B - (tid & ~127));
 
   for (int t = 0; t < a.n_steps; ++t) {
     // this step's action; the line of step t+1's action is requested now (prefetch: no register is held
@@ -1137,11 +1154,13 @@ __global__ void __maxnreg__(128) k_rollout(const __grid_constant__ KArgs<T> a) {
       a4 = *ap;
       if (t + 1 < a.n_steps) asm volatile("prefetch.global.L2 [%0];" ::"l"(ap + n));
     }
-    // Package regeneration is voted per BLOCK: all warps of a block run the (long) generator at the same
-    // step, and the barrier keeps them within one step of each other -- the step is ~30 KB of straight-line
-    // code, and warps that drift apart each stream it through the instruction caches on their own
-    // (measured: `no_instruction` became the top stall)
-    rollout_step<T, TASK, PHYS, NOISE, RNG, PID, WIDE>(a, m, sc, t, a4, [](bool p) { return __syncthreads_or(p) != 0; });
+    // Package regeneration is voted per 128-thread group of the block (named barrier 1 + group; the last group
+    // may be partial): all warps of a group run the (long) generator at the same step, and the barrier keeps
+    // them within one step of each other -- the step is ~30 KB of straight-line code, and warps that drift
+    // apart each stream it through the instruction caches on their own (measured: `no_instruction` became the
+    // top stall).  Barrier 0 belongs to the epilogue's statistics.
+    rollout_step<T, TASK, PHYS, NOISE, RNG, PID, WIDE>(a, m, sc, t, a4,
+                                                       [&](bool p) { return tile_vote(vote_bar, vote_threads, p); });
   }
 
   // ---- epilogue: state and history back to HBM, statistics, drain the bulk engine
