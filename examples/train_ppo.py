@@ -1,10 +1,11 @@
 #!/usr/bin/env python
-"""PPO training on the batched engine, one process per GPU.
+"""On-policy training (PPO, IWPG, NPG or TRPO) on the batched engine, one process per GPU.
 
     python examples/train_ppo.py --env DroneHoverSimpleEnv-v0 --epochs 30
+    python examples/train_ppo.py --alg trpo --update-kernel cuda
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 examples/train_ppo.py --epochs 30
 
-Counterpart of `python -m phoenix_drone_simulation.train --alg ppo --env <id> --cores N`
+Counterpart of `python -m phoenix_drone_simulation.train --alg {ppo,iwpg,npg,trpo} --env <id> --cores N`
 (train.py:97-149 of the reference): environments shard over the GPUs by global index, gradients,
 the observation normaliser and the episode statistics are all-reduced over NCCL, and -- like the
 reference's check_distributed_parameters (algs/iwpg/iwpg.py:228-237) -- the ranks verify at the end
@@ -22,13 +23,16 @@ import torch  # noqa: E402
 
 def main():
     p = argparse.ArgumentParser()
+    p.add_argument('--alg', default='ppo', choices=['ppo', 'iwpg', 'npg', 'trpo'],
+                   help="iwpg: PPO's loop with the unclipped surrogate; npg / trpo: conjugate-gradient policy steps")
     p.add_argument('--env', default='DroneHoverSimpleEnv-v0')
     p.add_argument('--epochs', type=int, default=30)
     p.add_argument('--num-envs', type=int, default=4096, help='per GPU')
     p.add_argument('--steps', type=int, default=64)
     p.add_argument('--seed', type=int, default=0)
     p.add_argument('--update-kernel', default='torch', choices=['torch', 'cuda'],
-                   help="'cuda': losses and gradients of the update in the fused kernels pdx_ppo_pi_grad / pdx_ppo_v_grad")
+                   help="'cuda': losses, gradients (and NPG / TRPO's Fisher-vector products) of the update in the fused "
+                        "kernels pdx_ppo_pi_grad / pdx_ppo_v_grad / pdx_ppo_pi_fvp")
     a = p.parse_args()
     world = int(os.environ.get('WORLD_SIZE', '1'))
     rank = int(os.environ.get('RANK', '0'))
@@ -40,9 +44,12 @@ def main():
         if os.environ.get('NCCL_DEBUG') and not os.environ.get('NCCL_DEBUG_FILE'):
             os.environ['NCCL_DEBUG_FILE'] = '/dev/stderr'     # stdout carries the JSON lines
         dist.init_process_group('nccl', device_id=torch.device('cuda', local))
+    from phoenix_drone_simulation_b200.npg import NPG
     from phoenix_drone_simulation_b200.ppo import PPO
-    alg = PPO(a.env, num_envs=a.num_envs, steps=a.steps, epochs=a.epochs, device=f'cuda:{local}', seed=a.seed, dist=dist,
-              update_kernel=a.update_kernel)
+    from phoenix_drone_simulation_b200.trpo import TRPO
+    cls, kw = {'ppo': (PPO, {}), 'iwpg': (PPO, {'clip_ratio': None}), 'npg': (NPG, {}), 'trpo': (TRPO, {})}[a.alg]
+    alg = cls(a.env, num_envs=a.num_envs, steps=a.steps, epochs=a.epochs, device=f'cuda:{local}', seed=a.seed, dist=dist,
+              update_kernel=a.update_kernel, **kw)
     for _ in range(a.epochs):
         row = alg.learn_one_epoch()
         if rank == 0:

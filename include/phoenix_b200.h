@@ -365,6 +365,8 @@ int pdx_evaluate(const PdxConfig* cfg, const PdxBuffers* buf, const PdxPolicySet
  *     r A <= clip(r) A and 0 elsewhere (torch's minimum / clamp backward).  grad == NULL: forward only.  Optional
  *     mu [n][4] receives pi(obs); with mu_ref [n][4] (and kl) kl = mean_i sum_j (mu_ref - mu)^2 / (2 std^2), the
  *     Gaussian KL at equal std.
+ *     clip_ratio = +INFINITY: no clip, loss = -mean(r A) (IWPG / NPG / TRPO's surrogate), d loss / d logp = -r A / n
+ *     everywhere; a non-finite ratio makes the loss non-finite, as in torch.
  *   pdx_ppo_v_grad, critic (tanh, 1 output): loss = mean((v(obs) - target_v)^2).
  * Row i of the batch is index[i] (index NULL: i) of obs / act / adv / logp_old / target_v; mu / mu_ref are indexed
  * by i.  Indices must lie inside the caller's tensors (not checked).  scratch: device memory of
@@ -393,6 +395,19 @@ int pdx_ppo_pi_grad(const PdxPpoBatch* batch, const PdxMlp* pi, const float* log
                     void* scratch, int64_t scratch_bytes, void* stream);
 int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const PdxMlpGrad* grad, float* loss,
                    void* scratch, int64_t scratch_bytes, void* stream);
+/* Fisher-vector product of the actor (algs/npg/npg.py Fvp) for conjugate-gradient policy updates:
+ *     out = scale * (1/n) sum_i J_i^T diag(std^-2) J_i dir + damping * dir,   J_i = d pi(obs_i) / d theta  [4 x params]
+ * = scale x the Hessian of pdx_ppo_pi_grad's kl (mean over samples, sum over the 4 action dimensions) at the current
+ * weights applied to dir, plus damping.  theta = the six nn.Linear tensors of `pi` (log_std is frozen and has no
+ * entry); `dir` and `out` are shaped like them ([out][in] weights and biases, dir->hidden == pi->hidden, n_out 4), and
+ * `out` must not overlap `dir`.  The batch uses n, obs_dim, obs and index only (every 4th row: pass an index).
+ * scratch: pdx_ppo_scratch_bytes(device, obs_dim, pi) bytes.  Float32 per sample, float64 sums rounded once;
+ * bit-identical from run to run like the gradients.  PDX_ERR_INVALID before any device call for the shapes
+ * pdx_ppo_pi_grad rejects, a dir of another shape, missing pointers, non-finite scale, negative or non-finite damping
+ * and a scratch smaller than one CTA's partials. */
+int pdx_ppo_pi_fvp(const PdxPpoBatch* batch, const PdxMlp* pi, const float* log_std, const PdxMlp* dir,
+                   float scale, float damping, const PdxMlpGrad* out, void* scratch, int64_t scratch_bytes,
+                   void* stream);
 
 /* Cross-rank combination of the 8-word episode statistics (utils/mpi_tools.py:217-240 does four
  * MPI all-reduces per key): the caller all-gathers the per-rank vectors into gathered[world][8]

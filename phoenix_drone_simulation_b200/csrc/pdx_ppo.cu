@@ -1,5 +1,7 @@
 // pdx_ppo_pi_grad / pdx_ppo_v_grad: the losses of PPO's update (algs/ppo/ppo.py:22-40, algs/iwpg/iwpg.py:446-485)
 // and their exact gradients with respect to every nn.Linear weight and bias of one network, on the CUDA cores in float32.
+// pdx_ppo_pi_fvp: NPG / TRPO's Fisher-vector product (algs/npg/npg.py Fvp) on the same plan, with a tangent pass
+// along the direction between the forward and the backward pass (k_ppo_fvp).
 //
 // Design
 //   * persistent grid, fixed assignment of sample tiles to CTAs (tile t -> CTA t mod G); one thread per sample of a
@@ -20,6 +22,8 @@
 // Arithmetic per sample (D inputs, h1 / h2 hidden units, O outputs): forward D h1 + h1 h2 + O h2 FMAs, backward data
 // O h2 + h1 h2, weight gradients D h1 + h1 h2 + O h2 (biases aside).  This unit is built without -use_fast_math:
 // expf and tanhf are the accurate ones.
+#include <cmath>
+
 #include "pdx_host.h"
 #include "pdx_layout.h"
 
@@ -39,10 +43,13 @@ __host__ __device__ constexpr int act_stride(int H) { return tile_stride(H + 1);
 __host__ __device__ inline int ppo_entries(int D, int h1, int h2, int O) { return h1 * (D + 1) + h2 * (h1 + 1) + O * (h2 + 1) + 2; }
 
 // shared-memory plan (floats): W1t[round4(D+1)][H], W2t[H+4][H], W2[H][H], W3t[H][4], b3[4];
-// tiles X[S][tile_stride(D+1)], A1, A2, D1, D2 [S][act_stride(H)], D3[S][4]; the final reduction's S doubles
-inline size_t ppo_smem_bytes(int S, int D, int H) {
-  const size_t w = (size_t)round4(D + 1) * H + (size_t)(H + 4) * H + (size_t)H * H + 4 * H + 4;
-  const size_t t = (size_t)S * tile_stride(D + 1) + 4 * (size_t)S * act_stride(H) + 4 * (size_t)S + 2 * (size_t)S;
+// tiles X[S][tile_stride(D+1)], A1, A2, D1, D2 [S][act_stride(H)], D3[S][4]; the final reduction's S doubles.
+// The Fisher-vector product (fvp) adds dW3t[H][4], db3[4], gives W2 H + 4 rows (it holds dW2t during the tangent
+// pass, W1t holds dW1t) and needs no loss reduction.
+inline size_t ppo_smem_bytes(int S, int D, int H, bool fvp = false) {
+  const size_t w = (size_t)round4(D + 1) * H + (size_t)(H + 4) * H + (size_t)(fvp ? H + 4 : H) * H + (fvp ? 8 : 4) * H +
+                   (fvp ? 8 : 4);
+  const size_t t = (size_t)S * tile_stride(D + 1) + 4 * (size_t)S * act_stride(H) + 4 * (size_t)S + (fvp ? 0 : 2 * (size_t)S);
   return (w + t) * sizeof(float);
 }
 
@@ -56,13 +63,15 @@ struct PpoArgs {
   float lo, hi;                               // 1 - clip_ratio, 1 + clip_ratio
   float* mu; const float* mu_ref;
   double* part;                               // [G][E2]
+  const float* dw[3]; const float* db[3];     // fvp: the direction, shaped like the network
 };
 
-// acc[j] = sum_{i < nin4} W[i][j] in[i] for the H outputs (W row stride H), inputs in order
+// what one k_ppo-plan launch computes
+enum PpoKind { kCritic, kClipped, kUnclipped, kFvp };
+
+// acc[j] += sum_{i < nin4} W[i][j] in[i] for the H outputs (W row stride H), inputs in order
 template <int H>
-__device__ __forceinline__ void dense(const float* __restrict__ W, int nin4, const float* __restrict__ in, float (&acc)[H]) {
-#pragma unroll
-  for (int j = 0; j < H; ++j) acc[j] = 0.0f;
+__device__ __forceinline__ void dense_add(const float* __restrict__ W, int nin4, const float* __restrict__ in, float (&acc)[H]) {
   for (int i = 0; i < nin4; i += 4) {
     const float4 x4 = *reinterpret_cast<const float4*>(in + i);
     const float xs[4] = {x4.x, x4.y, x4.z, x4.w};
@@ -81,14 +90,40 @@ __device__ __forceinline__ void dense(const float* __restrict__ W, int nin4, con
   }
 }
 
+template <int H>
+__device__ __forceinline__ void dense(const float* __restrict__ W, int nin4, const float* __restrict__ in, float (&acc)[H]) {
+#pragma unroll
+  for (int j = 0; j < H; ++j) acc[j] = 0.0f;
+  dense_add<H>(W, nin4, in, acc);
+}
+
+// dst[i][j] = [W | b]^T of an [nout][nin] layer with the bias as input row nin, zero padded to `rows` x H
+template <int H>
+__device__ __forceinline__ void stage_t(float* dst, int rows, const float* W, const float* b, int nin, int nout) {
+  for (int k = threadIdx.x; k < rows * H; k += blockDim.x) {
+    const int i = k / H, j = k % H;
+    dst[k] = j < nout ? (i < nin ? W[j * nin + i] : i == nin ? b[j] : 0.0f) : 0.0f;
+  }
+}
+
+// dst[j][i] = W[j][i] of an [nout][nin] layer, zero padded to H x H
+template <int H>
+__device__ __forceinline__ void stage_w(float* dst, const float* W, int nin, int nout) {
+  for (int k = threadIdx.x; k < H * H; k += blockDim.x) {
+    const int j = k / H, i = k % H;
+    dst[k] = (j < nout && i < nin) ? W[j * nin + i] : 0.0f;
+  }
+}
+
 template <bool ACTOR>
 __device__ __forceinline__ float act_fn(float z) { return ACTOR ? (z > 0.0f ? z : 0.0f) : tanhf(z); }
 // derivative from the activation's output: relu' = 1 only for z > 0 (torch threshold_backward), tanh' = 1 - a^2
 template <bool ACTOR>
 __device__ __forceinline__ float act_grad(float a) { return ACTOR ? (a > 0.0f ? 1.0f : 0.0f) : 1.0f - a * a; }
 
-template <bool ACTOR, bool GRAD, int H>
-__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
+template <int KIND, bool GRAD, int H>
+__device__ __forceinline__ void ppo_body(const PpoArgs& a) {
+  constexpr bool ACTOR = KIND != kCritic, FVP = KIND == kFvp;
   constexpr int AS = act_stride(H);
   const int S = blockDim.x, tid = threadIdx.x;
   const int D = a.D, h1 = a.h1, h2 = a.h2, O = a.O;
@@ -96,10 +131,12 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
   extern __shared__ __align__(16) float ppo_sm[];
   float* w1t = ppo_sm;                        // [D1][H]
   float* w2t = w1t + D1 * H;                  // [H + 4][H]
-  float* w2b = w2t + (H + 4) * H;             // [H][H]
-  float* w3t = w2b + H * H;                   // [H][4]
+  float* w2b = w2t + (H + 4) * H;             // [H][H] (fvp: [H + 4][H])
+  float* w3t = w2b + (FVP ? H + 4 : H) * H;   // [H][4]
   float* b3 = w3t + 4 * H;                    // [4]
-  float* X = b3 + 4;                          // [S][XS]
+  float* dw3t = b3 + 4;                       // fvp: [H][4]
+  float* db3 = dw3t + 4 * H;                  // fvp: [4]
+  float* X = FVP ? db3 + 4 : b3 + 4;          // [S][XS]
   float* A1 = X + S * XS;
   float* A2 = A1 + S * AS;
   float* D1t = A2 + S * AS;
@@ -124,6 +161,13 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
     w3t[k] = (j < h2 && o < O) ? a.w[2][o * h2 + j] : 0.0f;
   }
   if (tid < 4) b3[tid] = tid < O ? a.b[2][tid] : 0.0f;
+  if (FVP) {
+    for (int k = tid; k < 4 * H; k += S) {
+      const int j = k / 4, o = k % 4;
+      dw3t[k] = j < h2 ? a.dw[2][o * h2 + j] : 0.0f;
+    }
+    if (tid < 4) db3[tid] = a.db[2][tid];
+  }
   float ls[4] = {0.f, 0.f, 0.f, 0.f}, sd[4] = {1.f, 1.f, 1.f, 1.f};
   if (ACTOR) {
 #pragma unroll
@@ -139,6 +183,7 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
   for (int64_t tile = blockIdx.x; tile < a.ntiles; tile += gridDim.x) {
     const int64_t base = tile * S;
     __syncthreads();                          // the previous tile's readers are done with X (and the weights staged)
+    if (FVP && tile != blockIdx.x) stage_t<H>(w1t, D1, a.w[0], a.b[0], D, h1);    // dW1t during the tangent pass
     for (int k = tid; k < S * XS; k += S) {
       const int s = k / XS, c = k - s * XS;
       const int64_t i = base + s;
@@ -184,7 +229,46 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
     a2r[h2] = 1.0f;
     // ---- loss term and d loss / d output (without the 1 / n of the mean, applied in float64 by k_ppo_reduce)
     float d3[4] = {0.f, 0.f, 0.f, 0.f};
-    if (valid) {
+    if (FVP) {
+      // ---- tangent pass along the direction: u = J dir, J = d mu / d theta of this sample; d3 = u / std^2
+      __syncthreads();                        // every thread is done with W1t and W2
+      stage_t<H>(w1t, D1, a.dw[0], a.db[0], D, h1);
+      stage_t<H>(w2b, H + 4, a.dw[1], a.db[1], h1, h2);
+      __syncthreads();
+      dense<H>(w1t, D1, xr, acc);            // dz1 = dW1 [x, 1]
+#pragma unroll
+      for (int j4 = 0; j4 < AS / 4; ++j4) {  // da1 = dz1 relu'(z1) into the D1 row (the backward pass overwrites it);
+        float v[4];                           // entry h1 is 0, the bias input of [da1, 0]
+        const float4 av = *reinterpret_cast<const float4*>(a1r + 4 * j4);
+        const float as[4] = {av.x, av.y, av.z, av.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) v[q] = 4 * j4 + q < H ? acc[4 * j4 + q] * act_grad<true>(as[q]) : 0.0f;
+        *reinterpret_cast<float4*>(d1r + 4 * j4) = make_float4(v[0], v[1], v[2], v[3]);
+      }
+      dense<H>(w2b, round4(h1 + 1), a1r, acc);        // dz2 = dW2 [a1, 1] + W2 [da1, 0]
+      dense_add<H>(w2t, round4(h1 + 1), d1r, acc);
+      float u[4] = {db3[0], db3[1], db3[2], db3[3]};  // u = dW3 [a2, 1] + W3 (dz2 relu'(z2))
+#pragma unroll
+      for (int j4 = 0; j4 < H / 4; ++j4) {
+        const float4 av = *reinterpret_cast<const float4*>(a2r + 4 * j4);
+        const float as[4] = {av.x, av.y, av.z, av.w};
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const int j = 4 * j4 + q;
+          const float da2 = acc[j] * act_grad<true>(as[q]);
+          const float4 dv = reinterpret_cast<const float4*>(dw3t)[j], wv = reinterpret_cast<const float4*>(w3t)[j];
+          u[0] = fmaf(wv.x, da2, fmaf(dv.x, as[q], u[0])); u[1] = fmaf(wv.y, da2, fmaf(dv.y, as[q], u[1]));
+          u[2] = fmaf(wv.z, da2, fmaf(dv.z, as[q], u[2])); u[3] = fmaf(wv.w, da2, fmaf(dv.w, as[q], u[3]));
+        }
+      }
+      if (valid) {
+#pragma unroll
+        for (int k = 0; k < 4; ++k) d3[k] = u[k] / (sd[k] * sd[k]);
+      }
+      __syncthreads();                        // every thread is done with dW2t: W2 back for the backward pass
+      stage_w<H>(w2b, a.w[1], h1, h2);
+      __syncthreads();
+    } else if (valid) {
       if (ACTOR) {
         float z[4], lp = 0.0f;
 #pragma unroll
@@ -194,11 +278,18 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
         }
         const float A = a.adv[row];
         const float r = expf(lp - a.logp_old[row]);
-        const float s1 = r * A, s2 = fminf(fmaxf(r, a.lo), a.hi) * A;
-        lsum -= (double)fminf(s1, s2);
-        // torch: minimum passes the gradient to r A where r A <= clip(r) A (a tie inside the clip range is a tie of
-        // r A with itself); clamp passes nothing outside [lo, hi].  d logp / d mu = (a - mu) / std^2
-        const float g = s1 <= s2 ? -s1 : 0.0f;
+        const float s1 = r * A;
+        float g;
+        if (KIND == kUnclipped) {             // -(r A).mean(): a non-finite ratio reaches the loss, as in torch
+          lsum -= (double)s1;
+          g = -s1;
+        } else {
+          const float s2 = fminf(fmaxf(r, a.lo), a.hi) * A;
+          lsum -= (double)fminf(s1, s2);
+          // torch: minimum passes the gradient to r A where r A <= clip(r) A (a tie inside the clip range is a tie of
+          // r A with itself); clamp passes nothing outside [lo, hi].  d logp / d mu = (a - mu) / std^2
+          g = s1 <= s2 ? -s1 : 0.0f;
+        }
 #pragma unroll
         for (int k = 0; k < 4; ++k) d3[k] = g * z[k] / sd[k];
         if (a.mu) {
@@ -279,6 +370,7 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
       }
     }
   }
+  if (FVP) return;                            // no loss: the reduction's entries E2 - 2, E2 - 1 are not written
   // ---- loss and KL sums of this CTA, in thread order
   __syncthreads();
   red[tid] = lsum;
@@ -297,6 +389,17 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) {
     part[a.E2 - 1] = s;
   }
 }
+
+template <bool ACTOR, bool GRAD, int H>
+__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo(const PpoArgs a) { ppo_body<ACTOR ? kClipped : kCritic, GRAD, H>(a); }
+
+template <bool GRAD, int H>
+__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_unclipped(const PpoArgs a) { ppo_body<kUnclipped, GRAD, H>(a); }
+
+// J^T diag(std^-2) J dir summed over the samples (J = d mu / d theta): the tangent pass gives u = J dir, the backward
+// pass and the weight-gradient patches of the actor's gradient turn d3 = u / std^2 into J^T d3
+template <int H>
+__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_fvp(const PpoArgs a) { ppo_body<kFvp, true, H>(a); }
 
 struct ReduceArgs {
   int32_t G, D, h1, h2, O, E2;
@@ -323,6 +426,30 @@ __global__ void k_ppo_reduce(const ReduceArgs a) {
   else (l == 0 ? a.gb[0] : l == 1 ? a.gb[1] : a.gb[2])[r] = v;
 }
 
+struct FvpReduceArgs {
+  int32_t G, D, h1, h2, E2;
+  double scale_n, damping;                    // scale / n
+  const double* part;
+  const float* dw[3]; const float* db[3];     // the direction
+  float* gw[3]; float* gb[3];
+};
+
+// k_ppo_reduce for the Fisher-vector product: out = scale / n * (sum of the CTA partials in CTA order) + damping * dir,
+// in float64, rounded once
+__global__ void k_ppo_fvp_reduce(const FvpReduceArgs a) {
+  const int e = blockIdx.x * blockDim.x + threadIdx.x;
+  if (e >= a.E2 - 2) return;
+  double s = 0.0;
+  for (int g = 0; g < a.G; ++g) s += a.part[(int64_t)g * a.E2 + e];
+  int l = 0, in = a.D, k = e;
+  if (k >= a.h1 * (a.D + 1)) { k -= a.h1 * (a.D + 1); l = 1; in = a.h1;
+    if (k >= a.h2 * (a.h1 + 1)) { k -= a.h2 * (a.h1 + 1); l = 2; in = a.h2; } }
+  const int r = k / (in + 1), c = k % (in + 1);
+  const float* d = c < in ? a.dw[l] + r * in + c : a.db[l] + r;
+  float* o = c < in ? a.gw[l] + r * in + c : a.gb[l] + r;
+  *o = (float)(s * a.scale_n + a.damping * (double)*d);
+}
+
 bool mlp_ok(const PdxMlp* m, int n_out) {
   if (!m || m->hidden[0] < 1 || m->hidden[0] > 64 || m->hidden[1] < 1 || m->hidden[1] > 64 || m->n_out != n_out) return false;
   for (int k = 0; k < 3; ++k)
@@ -337,32 +464,38 @@ bool grad_ok(const PdxMlpGrad* g) {
 }
 
 // tile size: the largest of 128, 64, 32 whose shared-memory plan fits
-int ppo_tile(int D, int H) {
+int ppo_tile(int D, int H, bool fvp) {
   for (int S = kPpoMaxBlock; S >= 32; S /= 2)
-    if (ppo_smem_bytes(S, D, H) <= kMaxSmemBytes) return S;
+    if (ppo_smem_bytes(S, D, H, fvp) <= kMaxSmemBytes) return S;
   return 0;
 }
 
-template <bool ACTOR, bool GRAD, int H>
-cudaError_t launch_ppo(const PpoArgs& a, int S, int G, int dev, cudaStream_t st) {
-  const size_t smem = ppo_smem_bytes(S, a.D, H);
-  const cudaError_t e = opt_in_smem(k_ppo<ACTOR, GRAD, H>, dev, smem);
+template <typename K>
+cudaError_t launch_ppo(K kernel, const PpoArgs& a, int S, size_t smem, int G, int dev, cudaStream_t st) {
+  const cudaError_t e = opt_in_smem(kernel, dev, smem);
   if (e != cudaSuccess) return e;
-  k_ppo<ACTOR, GRAD, H><<<G, S, smem, st>>>(a);
+  kernel<<<G, S, smem, st>>>(a);
   return cudaGetLastError();
 }
 
-template <bool ACTOR, bool GRAD>
-cudaError_t launch_ppo_h(const PpoArgs& a, int H, int S, int G, int dev, cudaStream_t st) {
-  return H == 52 ? launch_ppo<ACTOR, GRAD, 52>(a, S, G, dev, st) : launch_ppo<ACTOR, GRAD, 64>(a, S, G, dev, st);
+template <int H>
+cudaError_t launch_kind(int kind, bool grad, const PpoArgs& a, int S, size_t smem, int G, int dev, cudaStream_t st) {
+  switch (kind) {
+    case kCritic: return launch_ppo(k_ppo<false, true, H>, a, S, smem, G, dev, st);
+    case kClipped: return launch_ppo(grad ? k_ppo<true, true, H> : k_ppo<true, false, H>, a, S, smem, G, dev, st);
+    case kUnclipped: return launch_ppo(grad ? k_ppo_unclipped<true, H> : k_ppo_unclipped<false, H>, a, S, smem, G, dev, st);
+    default: return launch_ppo(k_ppo_fvp<H>, a, S, smem, G, dev, st);
+  }
 }
 
-int ppo_run(const char* what, bool actor, const PdxPpoBatch* b, const PdxMlp* net, const float* log_std, float clip_ratio,
-            const PdxMlpGrad* grad, float* loss, float* mu, const float* mu_ref, float* kl, void* scratch,
-            int64_t scratch_bytes, void* stream) {
+// one launch of the k_ppo plan and its reduction.  kFvp: `grad` receives the product, dir / scale / damping are used
+int ppo_run(const char* what, int kind, const PdxPpoBatch* b, const PdxMlp* net, const float* log_std, float clip_ratio,
+            const PdxMlpGrad* grad, float* loss, float* mu, const float* mu_ref, float* kl, const PdxMlp* dir,
+            float scale, float damping, void* scratch, int64_t scratch_bytes, void* stream) {
+  const bool actor = kind != kCritic, fvp = kind == kFvp;
   const int D = b->obs_dim, h1 = net->hidden[0], h2 = net->hidden[1], O = actor ? 4 : 1;
   const int H = (h1 <= 52 && h2 <= 52) ? 52 : 64;
-  const int S = ppo_tile(D, H);
+  const int S = ppo_tile(D, H, fvp);
   if (S == 0) return set_error(PDX_ERR_INVALID, "pdx_ppo: obs_dim too wide for the shared-memory plan");
   const int E2 = ppo_entries(D, h1, h2, O);
   const int64_t per_cta = (int64_t)E2 * sizeof(double);
@@ -383,13 +516,22 @@ int ppo_run(const char* what, bool actor, const PdxPpoBatch* b, const PdxMlp* ne
   a.lo = (float)(1.0 - (double)clip_ratio); a.hi = (float)(1.0 + (double)clip_ratio);
   a.mu = mu; a.mu_ref = mu_ref;
   a.part = static_cast<double*>(scratch);
+  for (int k = 0; k < 3; ++k) { a.dw[k] = fvp ? dir->weight[k] : nullptr; a.db[k] = fvp ? dir->bias[k] : nullptr; }
   int64_t G = a.ntiles < sms ? a.ntiles : sms;
   if (G > scratch_bytes / per_cta) G = scratch_bytes / per_cta;
   const cudaStream_t st = (cudaStream_t)stream;
-  cudaError_t e;
-  if (actor) e = grad ? launch_ppo_h<true, true>(a, H, S, (int)G, dev, st) : launch_ppo_h<true, false>(a, H, S, (int)G, dev, st);
-  else e = launch_ppo_h<false, true>(a, H, S, (int)G, dev, st);
+  const size_t smem = ppo_smem_bytes(S, D, H, fvp);
+  const cudaError_t e = H == 52 ? launch_kind<52>(kind, grad != nullptr, a, S, smem, (int)G, dev, st)
+                                : launch_kind<64>(kind, grad != nullptr, a, S, smem, (int)G, dev, st);
   if (e != cudaSuccess) return cuda_error(what, e);
+  if (fvp) {
+    FvpReduceArgs r;
+    r.G = (int)G; r.D = D; r.h1 = h1; r.h2 = h2; r.E2 = E2; r.part = a.part;
+    r.scale_n = (double)scale / (double)b->n; r.damping = damping;
+    for (int k = 0; k < 3; ++k) { r.dw[k] = dir->weight[k]; r.db[k] = dir->bias[k]; r.gw[k] = grad->weight[k]; r.gb[k] = grad->bias[k]; }
+    k_ppo_fvp_reduce<<<(E2 + 255) / 256, 256, 0, st>>>(r);
+    return cuda_error(what, cudaGetLastError());
+  }
   ReduceArgs r;
   r.G = (int)G; r.D = D; r.h1 = h1; r.h2 = h2; r.O = O; r.E2 = E2; r.inv_n = 1.0 / (double)b->n; r.part = a.part;
   for (int k = 0; k < 3; ++k) { r.gw[k] = grad ? grad->weight[k] : nullptr; r.gb[k] = grad ? grad->bias[k] : nullptr; }
@@ -428,11 +570,42 @@ extern "C" int pdx_ppo_pi_grad(const PdxPpoBatch* batch, const PdxMlp* pi, const
     return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad: batch needs n >= 1, 1 <= obs_dim <= 384, obs, act, adv and logp_old");
   if (!mlp_ok(pi, 4) || !log_std)
     return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad: actor must have two hidden layers of <= 64 units, 4 outputs and log_std");
-  if (!(clip_ratio >= 0.0f && clip_ratio < 1e30f))
-    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad: clip_ratio must be finite and >= 0");
+  const bool unclipped = clip_ratio == INFINITY;
+  if (!(clip_ratio >= 0.0f && (clip_ratio < 1e30f || unclipped)))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad: clip_ratio must be >= 0 (finite, or +inf for no clip)");
   if (!loss || (grad && !grad_ok(grad)) || (!mu_ref) != (!kl))
     return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad: loss is required, a gradient with all six tensors, mu_ref and kl both or neither");
-  return ppo_run("pdx_ppo_pi_grad", true, batch, pi, log_std, clip_ratio, grad, loss, mu, mu_ref, kl, scratch, scratch_bytes, stream);
+  return ppo_run("pdx_ppo_pi_grad", unclipped ? kUnclipped : kClipped, batch, pi, log_std, clip_ratio, grad, loss, mu, mu_ref,
+                 kl, nullptr, 0.0f, 0.0f, scratch, scratch_bytes, stream);
+}
+
+extern "C" int pdx_ppo_pi_fvp(const PdxPpoBatch* batch, const PdxMlp* pi, const float* log_std, const PdxMlp* dir,
+                              float scale, float damping, const PdxMlpGrad* out, void* scratch, int64_t scratch_bytes,
+                              void* stream) {
+  using namespace pdx;
+  if (!batch_ok(batch))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: batch needs n >= 1, 1 <= obs_dim <= 384 and obs");
+  if (!mlp_ok(pi, 4) || !log_std)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: actor must have two hidden layers of <= 64 units, 4 outputs and log_std");
+  if (!mlp_ok(dir, 4) || dir->hidden[0] != pi->hidden[0] || dir->hidden[1] != pi->hidden[1])
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: dir must have the actor's shape and all six tensors");
+  if (!out || !grad_ok(out))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: out needs all six tensors");
+  // out must not overlap dir: k_ppo_fvp_reduce reads dir while it writes out
+  const int64_t D = batch->obs_dim, h1 = pi->hidden[0], h2 = pi->hidden[1];
+  const int64_t rows[3] = {h1, h2, 4}, cols[3] = {D, h1, h2};
+  for (int i = 0; i < 6; ++i)
+    for (int j = 0; j < 6; ++j) {
+      const uintptr_t o = (uintptr_t)(i < 3 ? (const void*)out->weight[i] : (const void*)out->bias[i - 3]);
+      const uintptr_t d = (uintptr_t)(j < 3 ? (const void*)dir->weight[j] : (const void*)dir->bias[j - 3]);
+      const uintptr_t no = 4 * (uintptr_t)(i < 3 ? rows[i] * cols[i] : rows[i - 3]);
+      const uintptr_t nd = 4 * (uintptr_t)(j < 3 ? rows[j] * cols[j] : rows[j - 3]);
+      if (o < d + nd && d < o + no) return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: out must not alias dir");
+    }
+  if (!std::isfinite(scale) || !(damping >= 0.0f) || !std::isfinite(damping))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp: scale must be finite, damping finite and >= 0");
+  return ppo_run("pdx_ppo_pi_fvp", kFvp, batch, pi, log_std, 0.0f, out, nullptr, nullptr, nullptr, nullptr, dir, scale,
+                 damping, scratch, scratch_bytes, stream);
 }
 
 extern "C" int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const PdxMlpGrad* grad, float* loss,
@@ -444,5 +617,6 @@ extern "C" int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const P
     return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad: critic must have two hidden layers of <= 64 units and one output");
   if (!loss || !grad || !grad_ok(grad))
     return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad: loss and a gradient with all six tensors are required");
-  return ppo_run("pdx_ppo_v_grad", false, batch, v, nullptr, 0.0f, grad, loss, nullptr, nullptr, nullptr, scratch, scratch_bytes, stream);
+  return ppo_run("pdx_ppo_v_grad", kCritic, batch, v, nullptr, 0.0f, grad, loss, nullptr, nullptr, nullptr, nullptr, 0.0f, 0.0f,
+                 scratch, scratch_bytes, stream);
 }

@@ -167,6 +167,8 @@ def load():
                                     C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
     lib.pdx_ppo_v_grad.argtypes = [P(PdxPpoBatch), P(PdxMlp), P(PdxMlpGrad), C.c_void_p, C.c_void_p, C.c_int64,
                                    C.c_void_p]
+    lib.pdx_ppo_pi_fvp.argtypes = [P(PdxPpoBatch), P(PdxMlp), C.c_void_p, P(PdxMlp), C.c_float, C.c_float,
+                                   P(PdxMlpGrad), C.c_void_p, C.c_int64, C.c_void_p]
     if lib.pdx_abi_version() != ABI_VERSION:
         raise PhoenixB200Error(f'ABI mismatch: library {lib.pdx_abi_version()} != binding {ABI_VERSION}')
     if lib.pdx_config_size() != C.sizeof(PdxConfig) or lib.pdx_buffers_size() != C.sizeof(PdxBuffers):
@@ -187,5 +189,5 @@ EXPORTED_SYMBOLS = [
     'pdx_step_many', 'pdx_dump_draws',
     'pdx_gae', 'pdx_moments', 'pdx_stats_combine', 'pdx_policy_step', 'pdx_policy_pack', 'pdx_policy_pack_words',
     'pdx_policy_step_tc', 'pdx_policy_tc_pack', 'pdx_policy_tc_pack_words', 'pdx_collect', 'pdx_collect_scratch_bytes', 'pdx_oms_update',
-    'pdx_evaluate', 'pdx_ppo_scratch_bytes', 'pdx_ppo_pi_grad', 'pdx_ppo_v_grad',
+    'pdx_evaluate', 'pdx_ppo_scratch_bytes', 'pdx_ppo_pi_grad', 'pdx_ppo_v_grad', 'pdx_ppo_pi_fvp',
 ]

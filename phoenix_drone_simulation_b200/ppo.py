@@ -6,7 +6,8 @@ Mirrors the reference's on-policy loop (paths relative to phoenix_drone_simulati
   algs/iwpg/iwpg.py:398-485  update(): value net `train_v_iterations` x `num_mini_batches`
                              mini-batch steps, policy net `train_pi_iterations` full-batch steps,
                              gradients averaged across ranks (mpi_avg_grads, mpi_tools.py:30-36)
-  algs/ppo/ppo.py:22-40      clipped surrogate loss
+  algs/ppo/ppo.py:22-40      clipped surrogate loss (clip_ratio=None: IWPG's unclipped -(r A).mean(),
+                             algs/iwpg/iwpg.py compute_loss_pi)
   algs/ppo/defaults.py:6-19  networks pi 50-50 relu, v 64-64 tanh, gamma 0.99
 The env.step hot path, GAE, running statistics and the fused policy step are CUDA kernels of this
 repo.  The update's losses and gradients run as torch autograd (update_kernel='torch', the default and
@@ -87,7 +88,7 @@ def _vec(t, rows, what):
 
 def pi_loss_and_grad(ac, obs, act, adv, logp_old, clip_ratio, index=None, grad=True, mu=None, mu_ref=None):
     """PPO's clipped surrogate loss of the actor (algs/ppo/ppo.py:22-40, without the entropy term) in ONE fused CUDA
-    kernel (pdx_ppo_pi_grad).  obs [rows, D] standardised, act [rows, 4], adv / logp_old [rows], float32 CUDA;
+    kernel (pdx_ppo_pi_grad); clip_ratio None (or inf): the unclipped -(r A).mean() of IWPG / NPG / TRPO.  obs [rows, D] standardised, act [rows, 4], adv / logp_old [rows], float32 CUDA;
     optional int64 `index` [n] selects the rows.  grad=True writes d loss / d weight and bias into p.grad of ac.pi's
     nn.Linear layers (log_std is frozen and gets none).  mu [n, 4]: receives pi(obs).  mu_ref [n, 4]: the Gaussian
     KL mean_i sum_j (mu_ref - mu)^2 / (2 std^2) is computed too.  Returns (loss, kl): 0-d float32 device tensors
@@ -101,10 +102,81 @@ def pi_loss_and_grad(ac, obs, act, adv, logp_old, clip_ratio, index=None, grad=T
     p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
     for t in (mu, mu_ref):
         assert t is None or (t.is_cuda and t.dtype == torch.float32 and t.is_contiguous() and t.shape == (b.n, 4))
-    _lib.check(L.pdx_ppo_pi_grad(C.byref(b), C.byref(mlp), p(ac.log_std.data), float(clip_ratio),
+    clip = math.inf if clip_ratio is None else float(clip_ratio)
+    _lib.check(L.pdx_ppo_pi_grad(C.byref(b), C.byref(mlp), p(ac.log_std.data), clip,
                                  C.byref(g) if g is not None else None, p(loss), p(mu), p(mu_ref), p(kl),
                                  p(scratch), scratch.numel(), st))
     return loss, kl
+
+
+def pi_net_params(ac):
+    """The actor's nn.Linear tensors in the order of the reference's get_flat_params_from(ac.pi.net): W1, b1, W2, b2,
+    W3, b3.  log_std (in ac.pi.parameters(), frozen) is not among them."""
+    return [p_ for m in ac.pi if isinstance(m, torch.nn.Linear) for p_ in (m.weight, m.bias)]
+
+
+def flat_views(flat, params):
+    """Views into the flat vector `flat`, one per tensor of `params`, in order and with their shapes."""
+    out, k = [], 0
+    for p_ in params:
+        out.append(flat[k:k + p_.numel()].view_as(p_))
+        k += p_.numel()
+    assert k == flat.numel(), (k, flat.numel())
+    return out
+
+
+def pi_flat_params(ac):
+    return torch.cat([p_.detach().reshape(-1) for p_ in pi_net_params(ac)])
+
+
+def set_pi_flat_params(ac, flat):
+    with torch.no_grad():
+        for p_, v in zip(pi_net_params(ac), flat_views(flat, pi_net_params(ac))):
+            p_.copy_(v)
+
+
+def pi_fvp_torch(ac, obs, direction, damping, scale, index=None):
+    """The reference's Fvp (algs/npg/npg.py) restated literally: the double backward of the mean per-dimension Normal
+    KL of the detached current policy to itself, applied to `direction`, plus damping * direction.  scale 1/4 is that
+    KL (its mean runs over the 4 action dimensions too); another scale multiplies it by 4 * scale."""
+    params = pi_net_params(ac)
+    o = obs if index is None else obs[index]
+    mu = ac.pi(o)
+    std = torch.exp(ac.log_std).to(mu.dtype)
+    q_dist = torch.distributions.Normal(mu, std)
+    with torch.no_grad():
+        p_dist = torch.distributions.Normal(mu.detach(), std)
+    kl = torch.distributions.kl.kl_divergence(p_dist, q_dist).mean() * (scale * mu.shape[-1])
+    grads = torch.autograd.grad(kl, params, create_graph=True)
+    flat_grad_kl = torch.cat([g.view(-1) for g in grads])
+    kl_p = (flat_grad_kl * direction).sum()
+    grads = torch.autograd.grad(kl_p, params, retain_graph=False)
+    return torch.cat([g.contiguous().view(-1) for g in grads]) + direction * damping
+
+
+def pi_fvp(ac, obs, direction, damping, scale, index=None, out=None):
+    """Fisher-vector product of the actor in ONE fused CUDA kernel (pdx_ppo_pi_fvp):
+        scale * (1/n) sum_i J_i^T diag(std^-2) J_i direction + damping * direction,  J_i = d pi(obs_i) / d theta
+    = scale x the Hessian of pi_loss_and_grad's kl (sum over the 4 action dimensions) applied to `direction`, plus
+    damping; scale = 1/4 is the reference's Fvp (pi_fvp_torch).  direction / out: flat float32 CUDA vectors in the
+    order of pi_net_params; the kernel reads and writes them through views, without copies.  Optional int64 `index`
+    selects the rows (NPG: every 4th).  Returns `out` (allocated when None); nothing is read back to the host."""
+    L, b, mlp, scratch, st = _prepare(ac, ac.pi, 4, obs, index)
+    params = pi_net_params(ac)
+    assert direction.is_cuda and direction.dtype == torch.float32 and direction.is_contiguous() and direction.dim() == 1
+    out = torch.empty_like(direction) if out is None else out
+    assert out.dtype == torch.float32 and out.is_contiguous() and out.shape == direction.shape
+    d = _lib.PdxMlp()
+    d.hidden[0], d.hidden[1], d.n_out = mlp.hidden[0], mlp.hidden[1], 4
+    g = _lib.PdxMlpGrad()
+    dv, ov = flat_views(direction, params), flat_views(out, params)
+    for k in range(3):
+        d.weight[k], d.bias[k] = dv[2 * k].data_ptr(), dv[2 * k + 1].data_ptr()
+        g.weight[k], g.bias[k] = ov[2 * k].data_ptr(), ov[2 * k + 1].data_ptr()
+    _lib.check(L.pdx_ppo_pi_fvp(C.byref(b), C.byref(mlp), C.c_void_p(ac.log_std.data.data_ptr()), C.byref(d),
+                                float(scale), float(damping), C.byref(g), C.c_void_p(scratch.data_ptr()),
+                                scratch.numel(), st))
+    return out
 
 
 def v_loss_and_grad(ac, obs, target_v, index=None):
@@ -148,6 +220,7 @@ class PPO:
         # carries obs[T] and bootstraps the cut with V(obs[T]), iwpg.py:376-378).
         self.collector = RolloutCollector(self.env, self.ac, steps, gamma=gamma, lam=lam, dist=dist,
                                           reset_each_rollout=steps >= self.env.max_episode_steps)
+        # clip_ratio None: the unclipped surrogate -(r A).mean() (the reference's IWPG)
         self.clip_ratio, self.entropy_coef, self.target_kl = clip_ratio, entropy_coef, target_kl
         self.train_pi_iterations, self.train_v_iterations = train_pi_iterations, train_v_iterations
         self.num_mini_batches, self.use_kl_early_stopping = num_mini_batches, use_kl_early_stopping
@@ -179,8 +252,11 @@ class PPO:
     def _loss_pi(self, obs, act, adv, logp_old):            # ppo.py:22-40
         mu, std, logp = self._log_prob(obs, act)
         ratio = torch.exp(logp - logp_old)
-        clip_adv = adv * torch.clamp(ratio, 1 - self.clip_ratio, 1 + self.clip_ratio)
-        loss = -torch.min(ratio * adv, clip_adv).mean()
+        if self.clip_ratio is None:                         # iwpg.py compute_loss_pi
+            loss = -(ratio * adv).mean()
+        else:
+            clip_adv = adv * torch.clamp(ratio, 1 - self.clip_ratio, 1 + self.clip_ratio)
+            loss = -torch.min(ratio * adv, clip_adv).mean()
         if self.entropy_coef:
             # ppo.py:32: `loss_pi -= entropy_coef * dist.entropy().mean()` -- the mean over the batch AND the
             # action dimensions of the per-dimension Gaussian entropy
