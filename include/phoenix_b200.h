@@ -37,7 +37,7 @@
 extern "C" {
 #endif
 
-#define PDX_ABI_VERSION 7
+#define PDX_ABI_VERSION 8
 
 typedef enum PdxStatus {
   PDX_OK = 0,
@@ -408,6 +408,53 @@ int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const PdxMlpGrad* 
 int pdx_ppo_pi_fvp(const PdxPpoBatch* batch, const PdxMlp* pi, const float* log_std, const PdxMlp* dir,
                    float scale, float damping, const PdxMlpGrad* out, void* scratch, int64_t scratch_bytes,
                    void* stream);
+
+/* ---- populations: P members (independent agents) of one env configuration on one GPU ----
+ * Member m owns environments [m N, (m + 1) N) of one P N-environment shard and has its own networks, normalisers and
+ * optimiser state.  Every member entry point runs the body of its single-network sibling on member m's slice with
+ * blockIdx.y = m, so member m's results equal the sibling's on that slice BIT FOR BIT (the moments: to float64
+ * rounding, the sibling's atomic sums have no fixed order either).  Layouts: parameters [P][out][in] / [P][out],
+ * policy images [P][stride], normalisers [P][D], log_std [P][4]; everything per sample is member-major [P][n][.],
+ * rollouts are [T][P N][.].  PDX_ERR_INVALID for bad arguments before any device call.
+ *
+ * pdx_policy_step_members: pdx_policy_step for P members of n environments each.  obs / actions / values / logp /
+ *   mu_out [P][n][.]; mean / std [P][obs_dim] (both NULL: no standardisation); log_std [P][pi->n_out]; packed: P
+ *   pdx_policy_pack images `stride` floats apart (a multiple of 4, >= pdx_policy_pack_words); pi / v give the shapes,
+ *   the same for every member.  Member m's noise is keyed by the global environment index env_offset + m n + i. */
+int pdx_policy_step_members(int32_t members, int64_t n, int32_t obs_dim, const float* obs, const float* mean,
+                            const float* std, float eps, const PdxMlp* pi, const PdxMlp* v, const float* log_std,
+                            const float* packed, int64_t stride, uint64_t seed, uint64_t counter, int64_t env_offset,
+                            float* actions, float* values, float* logp, float* mu_out, void* stream);
+/* pdx_gae for a [T][P n] population rollout: column c belongs to member c / n, whose rewards are scaled by
+ * ret_std_dev[c / n] + ret_scale when ret_std_dev ([P], device) is not NULL. */
+int pdx_gae_members(int32_t members, int64_t T, int64_t n, const float* rew, const float* val, const uint8_t* done,
+                    const float* boot_val, const float* last_val, float gamma, float lam, float ret_scale,
+                    int use_reward_scaling, const float* ret_std_dev, float* adv, float* target_v, float* disc_ret,
+                    void* stream);
+/* pdx_moments of every member's T n rows of x [T][P n][dim]: out[m][0..dim) += sum x, out[m][dim..2dim) +=
+ * sum (x - shift[m])^2; shift [P][dim] or NULL, out [P][2 dim]. */
+int pdx_moments_members(int32_t members, int64_t T, int64_t n, int32_t dim, const float* x, const double* shift,
+                        double* out, void* stream);
+/* pdx_ppo_pi_grad / pdx_ppo_v_grad for P members in one launch.  batch->n: samples per member; the batch tensors are
+ * [P][rows][.] (rows >= n without an index), the optional index [P][n] holds member-local row numbers; the networks
+ * `pi` / `v` and the gradients point at stacked [P][out][in] / [P][out] tensors; log_std [P][4]; mu / mu_ref [P][n][4];
+ * loss and kl [P].  active: optional [P] bytes, a member whose byte is 0 gets no tiles and none of its outputs is
+ * written.  scratch: P x pdx_ppo_scratch_bytes(); each member runs the CTAs a single launch with scratch_bytes / P
+ * bytes would, so its results equal that launch's bit for bit. */
+int pdx_ppo_pi_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                            const PdxMlp* pi, const float* log_std, float clip_ratio, const PdxMlpGrad* grad,
+                            float* loss, float* mu, const float* mu_ref, float* kl, void* scratch,
+                            int64_t scratch_bytes, void* stream);
+int pdx_ppo_v_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                           const PdxMlp* v, const PdxMlpGrad* grad, float* loss, void* scratch, int64_t scratch_bytes,
+                           void* stream);
+/* torch.optim.Adam (its foreach arithmetic: lerp_, mul_ / addcmul_, sqrt / bias correction, addcdiv_) on one parameter
+ * tensor stacked over P members ([P][numel] param / grad / exp_avg / exp_avg_sq, float32): member m uses its own step
+ * count steps[m] (float64, already incremented for this step) and is left untouched where active[m] == 0 (active
+ * optional [P] bytes). */
+int pdx_adam_members(int32_t members, int64_t numel, float* param, const float* grad, float* exp_avg, float* exp_avg_sq,
+                     const double* steps, const uint8_t* active, float lr, float beta1, float beta2, float eps,
+                     void* stream);
 
 /* Cross-rank combination of the 8-word episode statistics (utils/mpi_tools.py:217-240 does four
  * MPI all-reduces per key): the caller all-gathers the per-rank vectors into gathered[world][8]

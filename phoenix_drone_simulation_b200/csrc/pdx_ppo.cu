@@ -2,6 +2,8 @@
 // and their exact gradients with respect to every nn.Linear weight and bias of one network, on the CUDA cores in float32.
 // pdx_ppo_pi_fvp: NPG / TRPO's Fisher-vector product (algs/npg/npg.py Fvp) on the same plan, with a tangent pass
 // along the direction between the forward and the backward pass (k_ppo_fvp).
+// pdx_ppo_{pi,v}_grad_members: the same for P members of a population in one launch (k_ppo_members, blockIdx.y =
+// member), bit-identical to the single-network launch on each member's slice; pdx_adam_members: their Adam step.
 //
 // Design
 //   * persistent grid, fixed assignment of sample tiles to CTAs (tile t -> CTA t mod G); one thread per sample of a
@@ -401,6 +403,35 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_unclipped(const PpoArgs a)
 template <int H>
 __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_fvp(const PpoArgs a) { ppo_body<kFvp, true, H>(a); }
 
+template <class T>
+__device__ __forceinline__ T* member_ptr(T* p, int64_t off) { return p ? p + off : p; }
+
+// A population's members in one launch: grid (G, P), blockIdx.y = member.  Member m's CTA slot x runs ppo_body on
+// member m's slices exactly as CTA x of a single-network launch with the same G would: same tiles, same partial
+// layout, so the results equal pdx_ppo_*_grad on that member's rows bit for bit.  An inactive member does nothing.
+// `rows`: rows per member of the batch tensors (obs [P][rows][D], act [P][rows][4], adv [P][rows], ...); index
+// and mu / mu_ref are [P][n] / [P][n][4]; parameters [P][out][in] / [P][out]; log_std [P][4]; partials [P][G][E2].
+template <int KIND, bool GRAD, int H>
+__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_members(const PpoArgs a, int64_t rows, const uint8_t* active) {
+  const int m = blockIdx.y;
+  if (active && !active[m]) return;
+  PpoArgs b = a;
+  b.obs = a.obs + m * rows * a.D;
+  b.index = member_ptr(a.index, m * a.n);
+  b.act = member_ptr(a.act, m * rows * 4);
+  b.adv = member_ptr(a.adv, m * rows);
+  b.logp_old = member_ptr(a.logp_old, m * rows);
+  b.target_v = member_ptr(a.target_v, m * rows);
+  const int in[3] = {a.D, a.h1, a.h2}, out[3] = {a.h1, a.h2, a.O};
+#pragma unroll
+  for (int k = 0; k < 3; ++k) { b.w[k] = a.w[k] + (int64_t)m * out[k] * in[k]; b.b[k] = a.b[k] + (int64_t)m * out[k]; }
+  b.log_std = member_ptr(a.log_std, 4 * m);
+  b.mu = member_ptr(a.mu, m * a.n * 4);
+  b.mu_ref = member_ptr(a.mu_ref, m * a.n * 4);
+  b.part = a.part + (int64_t)m * gridDim.x * a.E2;
+  ppo_body<KIND, GRAD, H>(b);
+}
+
 struct ReduceArgs {
   int32_t G, D, h1, h2, O, E2;
   double inv_n;
@@ -409,8 +440,29 @@ struct ReduceArgs {
   float* loss; float* kl;
 };
 
+__device__ __forceinline__ void ppo_reduce_body(const ReduceArgs& a);
+
 // entry e of every CTA's partial summed in CTA order, / n, into the gradient tensors ([out][in] + bias) / loss / kl
-__global__ void k_ppo_reduce(const ReduceArgs a) {
+__global__ void k_ppo_reduce(const ReduceArgs a) { ppo_reduce_body(a); }
+
+// k_ppo_reduce per member (blockIdx.y): partials [P][G][E2] into the stacked gradients, loss[P] and kl[P]
+__global__ void k_ppo_reduce_members(const ReduceArgs a, const uint8_t* active) {
+  const int m = blockIdx.y;
+  if (active && !active[m]) return;
+  ReduceArgs b = a;
+  b.part = a.part + (int64_t)m * a.G * a.E2;
+  const int in[3] = {a.D, a.h1, a.h2}, out[3] = {a.h1, a.h2, a.O};
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    b.gw[k] = member_ptr(a.gw[k], (int64_t)m * out[k] * in[k]);
+    b.gb[k] = member_ptr(a.gb[k], (int64_t)m * out[k]);
+  }
+  b.loss = a.loss + m;
+  b.kl = member_ptr(a.kl, m);
+  ppo_reduce_body(b);
+}
+
+__device__ __forceinline__ void ppo_reduce_body(const ReduceArgs& a) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= a.E2 || (!a.gw[0] && e < a.E2 - 2)) return;
   double s = 0.0;
@@ -544,6 +596,71 @@ bool batch_ok(const PdxPpoBatch* b) {
   return b && b->n >= 1 && b->obs_dim >= 1 && b->obs_dim <= kPpoMaxObs && b->obs;
 }
 
+template <int H>
+cudaError_t launch_kind_members(int kind, bool grad, const PpoArgs& a, int64_t rows, const uint8_t* active, int S,
+                                size_t smem, int G, int P, int dev, cudaStream_t st) {
+  auto go = [&](auto kernel) {
+    const cudaError_t e = opt_in_smem(kernel, dev, smem);
+    if (e != cudaSuccess) return e;
+    kernel<<<dim3(G, P), S, smem, st>>>(a, rows, active);
+    return cudaGetLastError();
+  };
+  switch (kind) {
+    case kCritic: return go(k_ppo_members<kCritic, true, H>);
+    case kClipped: return grad ? go(k_ppo_members<kClipped, true, H>) : go(k_ppo_members<kClipped, false, H>);
+    default: return grad ? go(k_ppo_members<kUnclipped, true, H>) : go(k_ppo_members<kUnclipped, false, H>);
+  }
+}
+
+// ppo_run for P members (k_ppo_members + k_ppo_reduce_members): each member gets the G of a single launch with
+// scratch_bytes / P bytes of scratch
+int ppo_run_members(const char* what, int kind, int P, const PdxPpoBatch* b, int64_t rows, const uint8_t* active,
+                    const PdxMlp* net, const float* log_std, float clip_ratio, const PdxMlpGrad* grad, float* loss,
+                    float* mu, const float* mu_ref, float* kl, void* scratch, int64_t scratch_bytes, void* stream) {
+  const bool actor = kind != kCritic;
+  const int D = b->obs_dim, h1 = net->hidden[0], h2 = net->hidden[1], O = actor ? 4 : 1;
+  const int H = (h1 <= 52 && h2 <= 52) ? 52 : 64;
+  const int S = ppo_tile(D, H, false);
+  if (S == 0) return set_error(PDX_ERR_INVALID, "pdx_ppo_*_members: obs_dim too wide for the shared-memory plan");
+  const int E2 = ppo_entries(D, h1, h2, O);
+  const int64_t per_cta = (int64_t)E2 * sizeof(double);
+  if (!scratch || scratch_bytes / P < per_cta)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_*_members: scratch of members x pdx_ppo_scratch_bytes() bytes required");
+  int dev = 0;
+  int rc = select_device_of(b->obs, &dev);
+  if (rc) return rc;
+  int sms = 148;
+  rc = cuda_error(what, cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  if (rc) return rc;
+  PpoArgs a;
+  a.n = b->n; a.ntiles = (b->n + S - 1) / S;
+  a.D = D; a.h1 = h1; a.h2 = h2; a.O = O; a.E2 = E2;
+  a.obs = b->obs; a.index = b->index; a.act = b->act; a.adv = b->adv; a.logp_old = b->logp_old; a.target_v = b->target_v;
+  for (int k = 0; k < 3; ++k) { a.w[k] = net->weight[k]; a.b[k] = net->bias[k]; a.dw[k] = nullptr; a.db[k] = nullptr; }
+  a.log_std = log_std;
+  a.lo = (float)(1.0 - (double)clip_ratio); a.hi = (float)(1.0 + (double)clip_ratio);
+  a.mu = mu; a.mu_ref = mu_ref;
+  a.part = static_cast<double*>(scratch);
+  int64_t G = a.ntiles < sms ? a.ntiles : sms;
+  if (G > scratch_bytes / P / per_cta) G = scratch_bytes / P / per_cta;
+  const cudaStream_t st = (cudaStream_t)stream;
+  const size_t smem = ppo_smem_bytes(S, D, H, false);
+  const cudaError_t e = H == 52 ? launch_kind_members<52>(kind, grad != nullptr, a, rows, active, S, smem, (int)G, P, dev, st)
+                                : launch_kind_members<64>(kind, grad != nullptr, a, rows, active, S, smem, (int)G, P, dev, st);
+  if (e != cudaSuccess) return cuda_error(what, e);
+  ReduceArgs r;
+  r.G = (int)G; r.D = D; r.h1 = h1; r.h2 = h2; r.O = O; r.E2 = E2; r.inv_n = 1.0 / (double)b->n; r.part = a.part;
+  for (int k = 0; k < 3; ++k) { r.gw[k] = grad ? grad->weight[k] : nullptr; r.gb[k] = grad ? grad->bias[k] : nullptr; }
+  r.loss = loss; r.kl = kl;
+  k_ppo_reduce_members<<<dim3((E2 + 255) / 256, P), 256, 0, st>>>(r, active);
+  return cuda_error(what, cudaGetLastError());
+}
+
+// the member arguments shared by both entry points: P in [1, 65535], rows >= n without an index, rows >= 1 with one
+bool members_ok(int32_t P, const PdxPpoBatch* b, int64_t rows) {
+  return P >= 1 && P <= 65535 && rows >= 1 && (b->index || rows >= b->n);
+}
+
 }  // namespace
 }  // namespace pdx
 
@@ -619,4 +736,76 @@ extern "C" int pdx_ppo_v_grad(const PdxPpoBatch* batch, const PdxMlp* v, const P
     return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad: loss and a gradient with all six tensors are required");
   return ppo_run("pdx_ppo_v_grad", kCritic, batch, v, nullptr, 0.0f, grad, loss, nullptr, nullptr, nullptr, nullptr, 0.0f, 0.0f,
                  scratch, scratch_bytes, stream);
+}
+
+extern "C" int pdx_ppo_pi_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                                       const PdxMlp* pi, const float* log_std, float clip_ratio, const PdxMlpGrad* grad,
+                                       float* loss, float* mu, const float* mu_ref, float* kl, void* scratch,
+                                       int64_t scratch_bytes, void* stream) {
+  using namespace pdx;
+  if (!batch_ok(batch) || !batch->act || !batch->adv || !batch->logp_old)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: batch needs n >= 1, 1 <= obs_dim <= 384, obs, act, adv and logp_old");
+  if (!members_ok(members, batch, rows))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: members must be in [1, 65535] and rows >= n (>= 1 with an index)");
+  if (!mlp_ok(pi, 4) || !log_std)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: actor must have two hidden layers of <= 64 units, 4 outputs and log_std");
+  const bool unclipped = clip_ratio == INFINITY;
+  if (!(clip_ratio >= 0.0f && (clip_ratio < 1e30f || unclipped)))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: clip_ratio must be >= 0 (finite, or +inf for no clip)");
+  if (!loss || (grad && !grad_ok(grad)) || (!mu_ref) != (!kl))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: loss is required, a gradient with all six tensors, mu_ref and kl both or neither");
+  return ppo_run_members("pdx_ppo_pi_grad_members", unclipped ? kUnclipped : kClipped, members, batch, rows, active, pi,
+                         log_std, clip_ratio, grad, loss, mu, mu_ref, kl, scratch, scratch_bytes, stream);
+}
+
+extern "C" int pdx_ppo_v_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                                      const PdxMlp* v, const PdxMlpGrad* grad, float* loss, void* scratch,
+                                      int64_t scratch_bytes, void* stream) {
+  using namespace pdx;
+  if (!batch_ok(batch) || !batch->target_v)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad_members: batch needs n >= 1, 1 <= obs_dim <= 384, obs and target_v");
+  if (!members_ok(members, batch, rows))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad_members: members must be in [1, 65535] and rows >= n (>= 1 with an index)");
+  if (!mlp_ok(v, 1))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad_members: critic must have two hidden layers of <= 64 units and one output");
+  if (!loss || !grad || !grad_ok(grad))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad_members: loss and a gradient with all six tensors are required");
+  return ppo_run_members("pdx_ppo_v_grad_members", kCritic, members, batch, rows, active, v, nullptr, 0.0f, grad, loss,
+                         nullptr, nullptr, nullptr, scratch, scratch_bytes, stream);
+}
+
+// Adam (torch.optim.Adam's foreach arithmetic) on one parameter tensor stacked over P members, numel entries per
+// member; member m steps with its own count steps[m] (already incremented) unless active[m] == 0
+__global__ void k_adam_members(int64_t numel, int64_t total, float* __restrict__ w, const float* __restrict__ g,
+                               float* __restrict__ m1, float* __restrict__ m2, const double* __restrict__ steps,
+                               const uint8_t* __restrict__ active, double lr, float b1, float b2, float eps) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= total) return;
+  const int64_t m = i / numel;
+  if (active && !active[m]) return;
+  const double t = steps[m];
+  const float step_size = (float)(-(lr / (1.0 - pow((double)b1, t))));
+  const float bc2_sqrt = (float)sqrt(1.0 - pow((double)b2, t));
+  const float gi = g[i];
+  const float a = m1[i] + (1.0f - b1) * (gi - m1[i]);                    // lerp_(g, 1 - beta1), weight < 0.5
+  const float v = m2[i] * b2 + (1.0f - b2) * gi * gi;                     // mul_(beta2).addcmul_(g, g, 1 - beta2)
+  m1[i] = a;
+  m2[i] = v;
+  w[i] = w[i] + step_size * (a / (sqrtf(v) / bc2_sqrt + eps));           // addcdiv_(a, sqrt(v) / bc2 + eps, -lr / bc1)
+}
+
+extern "C" int pdx_adam_members(int32_t members, int64_t numel, float* param, const float* grad, float* exp_avg,
+                                float* exp_avg_sq, const double* steps, const uint8_t* active, float lr, float beta1,
+                                float beta2, float eps, void* stream) {
+  using namespace pdx;
+  if (members < 1 || numel < 1 || numel > INT64_MAX / members || !param || !grad || !exp_avg || !exp_avg_sq || !steps)
+    return set_error(PDX_ERR_INVALID, "pdx_adam_members: members and numel must be positive, buffers non-null");
+  if (!(lr >= 0.0f) || !(beta1 >= 0.0f && beta1 < 1.0f) || !(beta2 >= 0.0f && beta2 < 1.0f) || !(eps >= 0.0f))
+    return set_error(PDX_ERR_INVALID, "pdx_adam_members: lr >= 0, betas in [0, 1), eps >= 0");
+  const int rc = select_device_of(param);
+  if (rc) return rc;
+  const int64_t total = members * numel;
+  k_adam_members<<<(unsigned)((total + 255) / 256), 256, 0, (cudaStream_t)stream>>>(
+      numel, total, param, grad, exp_avg, exp_avg_sq, steps, active, (double)lr, beta1, beta2, eps);
+  return cuda_error("pdx_adam_members", cudaGetLastError());
 }

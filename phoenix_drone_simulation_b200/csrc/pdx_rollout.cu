@@ -5,22 +5,20 @@
 //               restarts the recursions at episode boundaries.
 //   pdx_moments restates the per-rank sums behind OnlineMeanStd.update
 //               (utils/online_mean_std.py:70-84): sum x and sum (x - shift)^2 per column.
+//   *_members   the same (and the fused policy step) for the P members of a population, blockIdx.y = member.
 #include "pdx_host.h"
 #include "pdx_layout.h"
 #include "pdx_math.cuh"
 
 namespace {
 
-__global__ void __launch_bounds__(128) k_gae(int64_t T, int64_t n, const float* __restrict__ rew,
-                                             const float* __restrict__ val, const uint8_t* __restrict__ done,
-                                             const float* __restrict__ boot_val, const float* __restrict__ last_val,
-                                             float gamma, float lam, float ret_scale, int use_scaling,
-                                             const float* __restrict__ ret_std_dev,
-                                             float* __restrict__ adv, float* __restrict__ target_v,
-                                             float* __restrict__ disc_ret) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  if (ret_std_dev) ret_scale += ret_std_dev[0];     // running std of the returns, read on the device (no host sync)
+// column i of a [T][n] rollout
+__device__ __forceinline__ void gae_column(int64_t i, int64_t T, int64_t n, const float* __restrict__ rew,
+                                           const float* __restrict__ val, const uint8_t* __restrict__ done,
+                                           const float* __restrict__ boot_val, const float* __restrict__ last_val,
+                                           float gamma, float lam, float ret_scale, int use_scaling,
+                                           float* __restrict__ adv, float* __restrict__ target_v,
+                                           float* __restrict__ disc_ret) {
   float next_val = last_val[i];       // epoch cut: bootstrap with V(o_T)        (iwpg.py:376-378)
   float next_ret = next_val;          // rews = [..., last_val]                   (core.py:514)
   float next_adv = 0.0f;
@@ -55,16 +53,45 @@ __global__ void __launch_bounds__(128) k_gae(int64_t T, int64_t n, const float* 
   }
 }
 
-// blockDim = (cols padded to 32, rows per block); each block strides over row tiles.
-__global__ void k_moments(int64_t rows, int dim, const float* __restrict__ x,
-                          const double* __restrict__ shift, double* __restrict__ out) {
+__global__ void __launch_bounds__(128) k_gae(int64_t T, int64_t n, const float* __restrict__ rew,
+                                             const float* __restrict__ val, const uint8_t* __restrict__ done,
+                                             const float* __restrict__ boot_val, const float* __restrict__ last_val,
+                                             float gamma, float lam, float ret_scale, int use_scaling,
+                                             const float* __restrict__ ret_std_dev,
+                                             float* __restrict__ adv, float* __restrict__ target_v,
+                                             float* __restrict__ disc_ret) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (ret_std_dev) ret_scale += ret_std_dev[0];     // running std of the returns, read on the device (no host sync)
+  gae_column(i, T, n, rew, val, done, boot_val, last_val, gamma, lam, ret_scale, use_scaling, adv, target_v, disc_ret);
+}
+
+// k_gae over the [T][P * N] rollout of a population: column i belongs to member i / N and scales its rewards by that
+// member's running return std ret_std_dev[i / N]
+__global__ void __launch_bounds__(128) k_gae_members(int64_t T, int64_t n, int64_t N, const float* __restrict__ rew,
+                                                     const float* __restrict__ val, const uint8_t* __restrict__ done,
+                                                     const float* __restrict__ boot_val, const float* __restrict__ last_val,
+                                                     float gamma, float lam, float ret_scale, int use_scaling,
+                                                     const float* __restrict__ ret_std_dev,
+                                                     float* __restrict__ adv, float* __restrict__ target_v,
+                                                     float* __restrict__ disc_ret) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  if (ret_std_dev) ret_scale += ret_std_dev[i / N];
+  gae_column(i, T, n, rew, val, done, boot_val, last_val, gamma, lam, ret_scale, use_scaling, adv, target_v, disc_ret);
+}
+
+// blockDim = (cols padded to 32, rows per block); each block strides over row tiles; row r is at x + row(r)
+template <class Row>
+__device__ __forceinline__ void moments_body(int64_t rows, int dim, Row row, const double* __restrict__ shift,
+                                             double* __restrict__ out) {
   extern __shared__ double sm[];                     // [2][blockDim.y][blockDim.x]
   const int d = threadIdx.x;
   double s1 = 0.0, s2 = 0.0;
   if (d < dim) {
     const double sh = shift ? shift[d] : 0.0;
     for (int64_t r = (int64_t)blockIdx.x * blockDim.y + threadIdx.y; r < rows; r += (int64_t)gridDim.x * blockDim.y) {
-      const double v = (double)x[r * dim + d];
+      const double v = (double)row(r)[d];
       s1 += v;
       s2 += (v - sh) * (v - sh);
     }
@@ -81,6 +108,19 @@ __global__ void k_moments(int64_t rows, int dim, const float* __restrict__ x,
     atomicAdd(&out[d], s1);
     atomicAdd(&out[dim + d], s2);
   }
+}
+
+__global__ void k_moments(int64_t rows, int dim, const float* __restrict__ x,
+                          const double* __restrict__ shift, double* __restrict__ out) {
+  moments_body(rows, dim, [=](int64_t r) { return x + r * dim; }, shift, out);
+}
+
+// member blockIdx.y of a [T][P * N][dim] population rollout: its T * N rows, shift [P][dim], out [P][2 dim]
+__global__ void k_moments_members(int64_t T, int64_t N, int dim, const float* __restrict__ x,
+                                  const double* __restrict__ shift, double* __restrict__ out) {
+  const int64_t m = blockIdx.y, PN = (int64_t)gridDim.y * N;
+  moments_body(T * N, dim, [=](int64_t r) { return x + ((r / N) * PN + m * N + r % N) * dim; },
+               shift ? shift + m * dim : shift, out + 2 * m * dim);
 }
 
 // Combines the episode-statistics vectors of all ranks after one all-gather:
@@ -160,6 +200,41 @@ extern "C" int pdx_moments(int64_t rows, int32_t dim, const float* x, const doub
   const size_t smem = 2ull * bx * by * sizeof(double);
   k_moments<<<grid, block, smem, (cudaStream_t)stream>>>(rows, dim, x, shift, out);
   return pdx::cuda_error("pdx_moments", cudaGetLastError());
+}
+
+extern "C" int pdx_gae_members(int32_t members, int64_t T, int64_t n, const float* rew, const float* val,
+                               const uint8_t* done, const float* boot_val, const float* last_val, float gamma, float lam,
+                               float ret_scale, int use_reward_scaling, const float* ret_std_dev, float* adv,
+                               float* target_v, float* disc_ret, void* stream) {
+  if (members < 1 || T <= 0 || n <= 0 || n > INT64_MAX / members)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_gae_members: members, T and n must be positive");
+  if (!rew || !val || !done || !boot_val || !last_val || !adv || !target_v || !disc_ret)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_gae_members: null buffer");
+  const int rc = pdx::select_device_of(rew);
+  if (rc) return rc;
+  const int64_t cols = members * n;
+  const unsigned grid = (unsigned)((cols + 127) / 128);
+  k_gae_members<<<grid, 128, 0, (cudaStream_t)stream>>>(T, cols, n, rew, val, done, boot_val, last_val, gamma, lam,
+                                                        ret_scale, use_reward_scaling, ret_std_dev, adv, target_v, disc_ret);
+  return pdx::cuda_error("pdx_gae_members", cudaGetLastError());
+}
+
+extern "C" int pdx_moments_members(int32_t members, int64_t T, int64_t n, int32_t dim, const float* x,
+                                   const double* shift, double* out, void* stream) {
+  if (members < 1 || members > 65535 || T <= 0 || n <= 0 || dim <= 0 || dim > 1024)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_moments_members: members in [1, 65535], T and n positive, dim in [1, 1024]");
+  if (!x || !out) return pdx::set_error(PDX_ERR_INVALID, "pdx_moments_members: null buffer");
+  const int rc = pdx::select_device_of(x);
+  if (rc) return rc;
+  // pdx_moments' block shape; the row tiles of the whole launch stay within 16 x 148 SMs' worth of blocks
+  const int bx = dim;
+  const int by = bx >= 256 ? 1 : 256 / bx;
+  const int64_t tiles = (T * n + by - 1) / by;
+  const int64_t cap = (2368 + members - 1) / members;
+  const dim3 grid((unsigned)(tiles < cap ? tiles : cap), (unsigned)members);
+  const size_t smem = 2ull * bx * by * sizeof(double);
+  k_moments_members<<<grid, dim3(bx, by), smem, (cudaStream_t)stream>>>(T, n, dim, x, shift, out);
+  return pdx::cuda_error("pdx_moments_members", cudaGetLastError());
 }
 
 extern "C" int pdx_oms_update(int32_t dim, const double* s1, const double* s2, double rows, int32_t world, const float* shift,
@@ -286,51 +361,38 @@ __global__ void k_pack_policy(const PolArgs a, float* __restrict__ out) {
 
 template <int HP, int HV>
 __global__ void __launch_bounds__(kPolBlock) k_policy(const PolArgs a) {
-  extern __shared__ __align__(16) float pol_sm[];
-  const int D = a.obs_dim, tid = threadIdx.x;
-  float* nmean = pol_sm;
-  float* ninv = nmean + ((D + 3) & ~3);
-  float* pi_net = ninv + ((D + 3) & ~3);
-  const int pi_words = pdx::policy_net_words(D, HP);
-  float* v_net = pi_net + pi_words;
-  const int v_words = pdx::policy_net_words(D, HV);
-  float* hid = v_net + v_words;
-  // ---- stage the normaliser and the packed (zero padded, transposed) weights: a flat copy of the
-  // blob k_pack_policy prepared (layout == the shared-memory plan from pi_net on)
-  for (int i = tid; i < D; i += kPolBlock) {
-    nmean[i] = a.std ? a.mean[i] : 0.0f;
-    ninv[i] = a.std ? 1.0f / (a.std[i] + a.eps) : 1.0f;
-  }
-  {
-    const float4* src = reinterpret_cast<const float4*>(a.packed);
-    float4* dst = reinterpret_cast<float4*>(pi_net);
-    for (int k = tid; k < (pi_words + v_words) / 4; k += kPolBlock) dst[k] = src[k];
-  }
-  __syncthreads();
-  const int64_t i = (int64_t)blockIdx.x * kPolBlock + tid;
-  if (i >= a.n) return;
-  const float* row = a.obs + i * D;
-  float mu[4], vv[4];
-  run_net<HP>(pi_net, row, nmean, ninv, D, a.pi_h1, a.pi_h2, false, hid, tid, mu);
-  run_net<HV>(v_net, row, nmean, ninv, D, a.v_h1, a.v_h2, true, hid, tid, vv);
-  // ---- sample: a = mu + std * eps, log p = sum(-eps^2/2 - log_std - log(2 pi)/2)
-  float eps[4];
-  pdx::policy_normals(a.seed, a.counter, (uint64_t)(a.env_offset + i), eps);
-  float lp = 0.0f;
-  float4 act = make_float4(0.f, 0.f, 0.f, 0.f);
-  float* av = reinterpret_cast<float*>(&act);
-#pragma unroll
-  for (int k = 0; k < 4; ++k) {
-    if (k < a.act_dim) {
-      const float ls = a.log_std[k];
-      av[k] = mu[k] + expf(ls) * eps[k];
-      lp += -0.5f * eps[k] * eps[k] - ls - 0.9189385332046727f;
-    }
-  }
-  reinterpret_cast<float4*>(a.act)[i] = act;
-  a.val[i] = vv[0];
-  a.logp[i] = lp;
-  if (a.mu) reinterpret_cast<float4*>(a.mu)[i] = make_float4(mu[0], mu[1], mu[2], mu[3]);
+#include "pdx_policy_body.cuh"
+}
+
+// A population's policy step: member m = blockIdx.y runs k_policy's body on its own slices -- obs / act / val / logp /
+// mu [P][n][.], normaliser [P][D], log_std [P][act_dim], image [P][stride] -- and draws its noise at the global
+// environment index env_offset + m n + i, so its outputs equal pdx_policy_step on its rows bit for bit
+template <int HP, int HV>
+__global__ void __launch_bounds__(kPolBlock) k_policy_members(const PolArgs args, int64_t stride) {
+  const int64_t m = blockIdx.y, n = args.n;
+  PolArgs a = args;
+  a.obs = args.obs + m * n * args.obs_dim;
+  if (args.std) { a.mean = args.mean + m * args.obs_dim; a.std = args.std + m * args.obs_dim; }
+  a.log_std = args.log_std + m * args.act_dim;
+  a.packed = args.packed + m * stride;
+  a.env_offset = args.env_offset + m * n;
+  a.act = args.act + m * n * 4; a.val = args.val + m * n; a.logp = args.logp + m * n;
+  if (args.mu) a.mu = args.mu + m * n * 4;
+#include "pdx_policy_body.cuh"
+}
+
+template <int HP, int HV>
+int launch_policy_members(const PolArgs& a, int members, int64_t stride, int dev, cudaStream_t st) {
+  const int D = a.obs_dim;
+  const size_t words = 2 * ((D + 3) & ~3) + (size_t)pdx::policy_net_words(D, HP) + (size_t)pdx::policy_net_words(D, HV) +
+                       (size_t)kHidMax * kPolBlock;
+  const size_t smem = words * sizeof(float);
+  if (smem > pdx::kMaxSmemBytes) return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: obs_dim too wide for the shared-memory plan");
+  const int rc = pdx::cuda_error("pdx_policy_step_members (shared-memory opt-in)", pdx::opt_in_smem(k_policy_members<HP, HV>, dev, smem));
+  if (rc) return rc;
+  const dim3 grid((unsigned)((a.n + kPolBlock - 1) / kPolBlock), (unsigned)members);
+  k_policy_members<HP, HV><<<grid, kPolBlock, smem, st>>>(a, stride);
+  return pdx::cuda_error("pdx_policy_step_members", cudaGetLastError());
 }
 
 template <int HP, int HV>
@@ -395,4 +457,38 @@ static int policy_dispatch(int64_t n, int32_t obs_dim, const float* obs, const f
   a.act = actions; a.val = values; a.logp = logp; a.mu = mu_out;
   const cudaStream_t st = (cudaStream_t)stream;
   return pdx::policy_actor_pad(a.pi_h1, a.pi_h2) == 52 ? launch_policy<52, 64>(a, dev, st) : launch_policy<64, 64>(a, dev, st);
+}
+
+extern "C" int pdx_policy_step_members(int32_t members, int64_t n, int32_t obs_dim, const float* obs, const float* mean,
+                                       const float* std, float eps, const PdxMlp* pi, const PdxMlp* v,
+                                       const float* log_std, const float* packed, int64_t stride, uint64_t seed,
+                                       uint64_t counter, int64_t env_offset, float* actions, float* values, float* logp,
+                                       float* mu_out, void* stream) {
+  if (members < 1 || members > 65535 || n <= 0 || obs_dim <= 0 || obs_dim > 384)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: members in [1, 65535], n >= 1 and obs_dim in [1, 384]");
+  if (!obs || !pi || !v || !log_std || !packed || !actions || !values || !logp || (!mean) != (!std))
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: null buffer (mean and std: both or neither)");
+  if (pi->hidden[0] < 1 || pi->hidden[0] > kHidMax || pi->hidden[1] < 1 || pi->hidden[1] > kHidMax || pi->n_out < 1 || pi->n_out > 4)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: actor must have two hidden layers of <= 64 units and <= 4 outputs");
+  if (v->hidden[0] < 1 || v->hidden[0] > kHidMax || v->hidden[1] < 1 || v->hidden[1] > kHidMax || v->n_out != 1)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: critic must have two hidden layers of <= 64 units and one output");
+  const int HP = pdx::policy_actor_pad(pi->hidden[0], pi->hidden[1]);
+  if (stride < pdx::policy_net_words((int64_t)obs_dim, HP) + pdx::policy_net_words((int64_t)obs_dim, 64) || stride % 4)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: stride must be a multiple of 4 and >= pdx_policy_pack_words()");
+  const size_t words = 2 * ((obs_dim + 3) & ~3) + (size_t)pdx::policy_net_words(obs_dim, HP) +
+                       (size_t)pdx::policy_net_words(obs_dim, 64) + (size_t)kHidMax * kPolBlock;
+  if (words * sizeof(float) > pdx::kMaxSmemBytes)
+    return pdx::set_error(PDX_ERR_INVALID, "pdx_policy_step_members: obs_dim too wide for the shared-memory plan");
+  int dev = 0;
+  const int rc = pdx::select_device_of(obs, &dev);
+  if (rc) return rc;
+  PolArgs a;
+  a.n = n; a.obs_dim = obs_dim; a.act_dim = pi->n_out;
+  a.pi_h1 = pi->hidden[0]; a.pi_h2 = pi->hidden[1]; a.v_h1 = v->hidden[0]; a.v_h2 = v->hidden[1];
+  a.obs = obs; a.mean = mean; a.std = std; a.eps = eps;
+  for (int k = 0; k < 3; ++k) { a.pi_w[k] = pi->weight[k]; a.pi_b[k] = pi->bias[k]; a.v_w[k] = v->weight[k]; a.v_b[k] = v->bias[k]; }
+  a.log_std = log_std; a.packed = packed; a.seed = seed; a.counter = counter; a.env_offset = env_offset;
+  a.act = actions; a.val = values; a.logp = logp; a.mu = mu_out;
+  const cudaStream_t st = (cudaStream_t)stream;
+  return HP == 52 ? launch_policy_members<52, 64>(a, members, stride, dev, st) : launch_policy_members<64, 64>(a, members, stride, dev, st);
 }

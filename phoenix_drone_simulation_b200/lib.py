@@ -10,7 +10,7 @@ import os
 HERE = os.path.dirname(os.path.abspath(__file__))
 # PDX_LIB: another build of the same library (kernel A/B experiments); default: the in-tree build
 LIB_PATH = os.environ.get('PDX_LIB') or os.path.join(HERE, 'libphoenix_b200.so')
-ABI_VERSION = 7
+ABI_VERSION = 8
 PDX_BUF_STATE_STABLE = 1          # PdxBuffers.flags
 PDX_POLICY_TC_OVERLAP = 0x100     # or-ed into pdx_policy_step_tc's precision
 
@@ -169,6 +169,22 @@ def load():
                                    C.c_void_p]
     lib.pdx_ppo_pi_fvp.argtypes = [P(PdxPpoBatch), P(PdxMlp), C.c_void_p, P(PdxMlp), C.c_float, C.c_float,
                                    P(PdxMlpGrad), C.c_void_p, C.c_int64, C.c_void_p]
+    lib.pdx_policy_step_members.argtypes = [C.c_int32, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float,
+                                            P(PdxMlp), P(PdxMlp), C.c_void_p, C.c_void_p, C.c_int64, C.c_uint64,
+                                            C.c_uint64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p]
+    lib.pdx_gae_members.argtypes = [C.c_int32, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_int, C.c_void_p, C.c_void_p,
+                                    C.c_void_p, C.c_void_p, C.c_void_p]
+    lib.pdx_moments_members.argtypes = [C.c_int32, C.c_int64, C.c_int64, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_void_p]
+    lib.pdx_ppo_pi_grad_members.argtypes = [C.c_int32, P(PdxPpoBatch), C.c_int64, C.c_void_p, P(PdxMlp), C.c_void_p,
+                                            C.c_float, P(PdxMlpGrad), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_int64, C.c_void_p]
+    lib.pdx_ppo_v_grad_members.argtypes = [C.c_int32, P(PdxPpoBatch), C.c_int64, C.c_void_p, P(PdxMlp), P(PdxMlpGrad),
+                                           C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.pdx_adam_members.argtypes = [C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
     if lib.pdx_abi_version() != ABI_VERSION:
         raise PhoenixB200Error(f'ABI mismatch: library {lib.pdx_abi_version()} != binding {ABI_VERSION}')
     if lib.pdx_config_size() != C.sizeof(PdxConfig) or lib.pdx_buffers_size() != C.sizeof(PdxBuffers):
@@ -190,4 +206,6 @@ EXPORTED_SYMBOLS = [
     'pdx_gae', 'pdx_moments', 'pdx_stats_combine', 'pdx_policy_step', 'pdx_policy_pack', 'pdx_policy_pack_words',
     'pdx_policy_step_tc', 'pdx_policy_tc_pack', 'pdx_policy_tc_pack_words', 'pdx_collect', 'pdx_collect_scratch_bytes', 'pdx_oms_update',
     'pdx_evaluate', 'pdx_ppo_scratch_bytes', 'pdx_ppo_pi_grad', 'pdx_ppo_v_grad', 'pdx_ppo_pi_fvp',
+    'pdx_policy_step_members', 'pdx_gae_members', 'pdx_moments_members', 'pdx_ppo_pi_grad_members',
+    'pdx_ppo_v_grad_members', 'pdx_adam_members',
 ]
