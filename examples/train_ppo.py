@@ -4,6 +4,7 @@
     python examples/train_ppo.py --env DroneHoverSimpleEnv-v0 --epochs 30
     python examples/train_ppo.py --alg trpo --update-kernel cuda
     python examples/train_ppo.py --population 8 --num-envs 512 --update-kernel cuda    # seeds 0..7 in one process
+    python examples/train_ppo.py --population 4 --alg trpo --update-kernel cuda
     python -m torch.distributed.run --nnodes=1 --nproc-per-node 8 --master-addr 127.0.0.1 examples/train_ppo.py --epochs 30
 
 Counterpart of `python -m phoenix_drone_simulation.train --alg {ppo,iwpg,npg,trpo} --env <id> --cores N`
@@ -35,23 +36,26 @@ def main():
                    help="'cuda': losses, gradients (and NPG / TRPO's Fisher-vector products) of the update in the fused "
                         "kernels pdx_ppo_pi_grad / pdx_ppo_v_grad / pdx_ppo_pi_fvp")
     p.add_argument('--population', type=int, default=0,
-                   help='train this many PPO agents (seeds seed .. seed + P - 1, --num-envs environments each) in one '
-                        'process on one GPU (population.PopulationPPO); prints one row per member and epoch')
+                   help='train this many agents of --alg (seeds seed .. seed + P - 1, --num-envs environments each) in one '
+                        'process on one GPU (population.PopulationPPO / PopulationNPG / PopulationTRPO); prints one row '
+                        'per member and epoch')
     a = p.parse_args()
     if a.population:
-        if a.alg != 'ppo':
-            p.error('--population trains PPO agents')
         if int(os.environ.get('WORLD_SIZE', '1')) > 1:
             p.error('--population trains on one GPU: start it once per GPU, not under torch.distributed.run')
-        from phoenix_drone_simulation_b200.population import PopulationPPO
-        pop = PopulationPPO(a.env, members=a.population, num_envs_per_member=a.num_envs, steps=a.steps,
-                            epochs=a.epochs, seed=a.seed, update_kernel=a.update_kernel)
+        from phoenix_drone_simulation_b200.population import PopulationNPG, PopulationPPO, PopulationTRPO
+        cls, kw = {'ppo': (PopulationPPO, {}), 'iwpg': (PopulationPPO, {'clip_ratio': None}), 'npg': (PopulationNPG, {}),
+                   'trpo': (PopulationTRPO, {})}[a.alg]
+        pop = cls(a.env, members=a.population, num_envs_per_member=a.num_envs, steps=a.steps, epochs=a.epochs,
+                  seed=a.seed, update_kernel=a.update_kernel, **kw)
+        keys = ('EpRet', 'EpLen', 'episodes', 'loss_pi', 'loss_v', 'kl')
+        keys += ('accept_step', 'xHx') if a.alg in ('npg', 'trpo') else ('pi_iters',)
         for _ in range(a.epochs):
             row = pop.learn_one_epoch()
             for m in range(pop.P):
                 print(json.dumps({'epoch': row['epoch'], 'member': m, 'seed': a.seed + m, 'FPS': round(row['FPS'], 1),
                                   **{k: (round(row[k][m], 4) if isinstance(row[k][m], float) else row[k][m])
-                                     for k in ('EpRet', 'EpLen', 'episodes', 'loss_pi', 'loss_v', 'pi_iters', 'kl')}}),
+                                     for k in keys}}),
                       flush=True)
         return
     world = int(os.environ.get('WORLD_SIZE', '1'))

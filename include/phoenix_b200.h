@@ -448,6 +448,17 @@ int pdx_ppo_pi_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t r
 int pdx_ppo_v_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
                            const PdxMlp* v, const PdxMlpGrad* grad, float* loss, void* scratch, int64_t scratch_bytes,
                            void* stream);
+/* pdx_ppo_pi_fvp for P members in one launch, on the batch, index, active and scratch conventions of
+ * pdx_ppo_pi_grad_members (NPG passes every 4th member-local row as the index).  pi: stacked [P][out][in] / [P][out];
+ * log_std [P][4].  dir / out: the six tensors of member 0; member m's start vec_stride floats later, so one flat [P][F]
+ * vector per quantity (F = the actor's parameter count, in the order of the single entry point's flat views) serves
+ * with vec_stride = F.  An inactive member's out is not written.  PDX_ERR_INVALID before any device call for what
+ * pdx_ppo_pi_fvp rejects, members outside [1, 65535], rows < n without an index, vec_stride < F, a scratch
+ * smaller than P x one CTA's partials, and any overlap of out with dir over all members. */
+int pdx_ppo_pi_fvp_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                           const PdxMlp* pi, const float* log_std, const PdxMlp* dir, float scale, float damping,
+                           const PdxMlpGrad* out, int64_t vec_stride, void* scratch, int64_t scratch_bytes,
+                           void* stream);
 /* torch.optim.Adam (its foreach arithmetic: lerp_, mul_ / addcmul_, sqrt / bias correction, addcdiv_) on one parameter
  * tensor stacked over P members ([P][numel] param / grad / exp_avg / exp_avg_sq, float32): member m uses its own step
  * count steps[m] (float64, already incremented for this step) and is left untouched where active[m] == 0 (active

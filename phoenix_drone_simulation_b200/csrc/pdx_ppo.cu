@@ -3,7 +3,8 @@
 // pdx_ppo_pi_fvp: NPG / TRPO's Fisher-vector product (algs/npg/npg.py Fvp) on the same plan, with a tangent pass
 // along the direction between the forward and the backward pass (k_ppo_fvp).
 // pdx_ppo_{pi,v}_grad_members: the same for P members of a population in one launch (k_ppo_members, blockIdx.y =
-// member), bit-identical to the single-network launch on each member's slice; pdx_adam_members: their Adam step.
+// member), bit-identical to the single-network launch on each member's slice; pdx_ppo_pi_fvp_members: the Fisher-vector
+// product of P members likewise (k_ppo_fvp_members, k_ppo_fvp_reduce_members); pdx_adam_members: their Adam step.
 //
 // Design
 //   * persistent grid, fixed assignment of sample tiles to CTAs (tile t -> CTA t mod G); one thread per sample of a
@@ -432,6 +433,29 @@ __global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_members(const PpoArgs a, i
   ppo_body<KIND, GRAD, H>(b);
 }
 
+// k_ppo_fvp for P members: k_ppo_members' slicing of what the product reads, and member m's direction tensors start
+// m vec_stride floats after member 0's.  A kernel of its own rather than k_ppo_members<kFvp>: the stride is one more
+// argument, and one more parameter of k_ppo_members (a new name) or one more field of PpoArgs (even in its padding)
+// changes the code of the existing member kernels.
+template <int H>
+__global__ void __launch_bounds__(kPpoMaxBlock) k_ppo_fvp_members(const PpoArgs a, int64_t rows, const uint8_t* active,
+                                                                  int64_t vec_stride) {
+  const int m = blockIdx.y;
+  if (active && !active[m]) return;
+  PpoArgs b = a;
+  b.obs = a.obs + m * rows * a.D;
+  b.index = member_ptr(a.index, m * a.n);
+  const int in[3] = {a.D, a.h1, a.h2}, out[3] = {a.h1, a.h2, a.O};
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    b.w[k] = a.w[k] + (int64_t)m * out[k] * in[k]; b.b[k] = a.b[k] + (int64_t)m * out[k];
+    b.dw[k] = a.dw[k] + (int64_t)m * vec_stride; b.db[k] = a.db[k] + (int64_t)m * vec_stride;
+  }
+  b.log_std = a.log_std + 4 * m;
+  b.part = a.part + (int64_t)m * gridDim.x * a.E2;
+  ppo_body<kFvp, true, H>(b);
+}
+
 struct ReduceArgs {
   int32_t G, D, h1, h2, O, E2;
   double inv_n;
@@ -486,19 +510,32 @@ struct FvpReduceArgs {
   float* gw[3]; float* gb[3];
 };
 
+__device__ __forceinline__ void fvp_reduce_body(const FvpReduceArgs& a, const double* part, int64_t off);
+
 // k_ppo_reduce for the Fisher-vector product: out = scale / n * (sum of the CTA partials in CTA order) + damping * dir,
 // in float64, rounded once
-__global__ void k_ppo_fvp_reduce(const FvpReduceArgs a) {
+__global__ void k_ppo_fvp_reduce(const FvpReduceArgs a) { fvp_reduce_body(a, a.part, 0); }
+
+// k_ppo_fvp_reduce per member (blockIdx.y): partials [P][G][E2]; member m's dir and out tensors start m vec_stride
+// floats after member 0's
+__global__ void k_ppo_fvp_reduce_members(const FvpReduceArgs a, const uint8_t* active, int64_t vec_stride) {
+  const int m = blockIdx.y;
+  if (active && !active[m]) return;
+  fvp_reduce_body(a, a.part + (int64_t)m * a.G * a.E2, (int64_t)m * vec_stride);
+}
+
+// `part`: this launch's (member's) partials; `off`: floats from the tensors of a to the dir / out entries written
+__device__ __forceinline__ void fvp_reduce_body(const FvpReduceArgs& a, const double* part, int64_t off) {
   const int e = blockIdx.x * blockDim.x + threadIdx.x;
   if (e >= a.E2 - 2) return;
   double s = 0.0;
-  for (int g = 0; g < a.G; ++g) s += a.part[(int64_t)g * a.E2 + e];
+  for (int g = 0; g < a.G; ++g) s += part[(int64_t)g * a.E2 + e];
   int l = 0, in = a.D, k = e;
   if (k >= a.h1 * (a.D + 1)) { k -= a.h1 * (a.D + 1); l = 1; in = a.h1;
     if (k >= a.h2 * (a.h1 + 1)) { k -= a.h2 * (a.h1 + 1); l = 2; in = a.h2; } }
   const int r = k / (in + 1), c = k % (in + 1);
-  const float* d = c < in ? a.dw[l] + r * in + c : a.db[l] + r;
-  float* o = c < in ? a.gw[l] + r * in + c : a.gb[l] + r;
+  const float* d = (c < in ? a.dw[l] + r * in + c : a.db[l] + r) + off;
+  float* o = (c < in ? a.gw[l] + r * in + c : a.gb[l] + r) + off;
   *o = (float)(s * a.scale_n + a.damping * (double)*d);
 }
 
@@ -597,8 +634,14 @@ bool batch_ok(const PdxPpoBatch* b) {
 }
 
 template <int H>
-cudaError_t launch_kind_members(int kind, bool grad, const PpoArgs& a, int64_t rows, const uint8_t* active, int S,
-                                size_t smem, int G, int P, int dev, cudaStream_t st) {
+cudaError_t launch_kind_members(int kind, bool grad, const PpoArgs& a, int64_t rows, const uint8_t* active,
+                                int64_t vec_stride, int S, size_t smem, int G, int P, int dev, cudaStream_t st) {
+  if (kind == kFvp) {
+    const cudaError_t e = opt_in_smem(k_ppo_fvp_members<H>, dev, smem);
+    if (e != cudaSuccess) return e;
+    k_ppo_fvp_members<H><<<dim3(G, P), S, smem, st>>>(a, rows, active, vec_stride);
+    return cudaGetLastError();
+  }
   auto go = [&](auto kernel) {
     const cudaError_t e = opt_in_smem(kernel, dev, smem);
     if (e != cudaSuccess) return e;
@@ -612,15 +655,17 @@ cudaError_t launch_kind_members(int kind, bool grad, const PpoArgs& a, int64_t r
   }
 }
 
-// ppo_run for P members (k_ppo_members + k_ppo_reduce_members): each member gets the G of a single launch with
-// scratch_bytes / P bytes of scratch
+// ppo_run for P members (k_ppo_members + k_ppo_reduce_members, or k_ppo_fvp_reduce_members for kFvp): each member gets
+// the G of a single launch with scratch_bytes / P bytes of scratch.  kFvp: `grad` receives the product, dir / scale /
+// damping / vec_stride are used
 int ppo_run_members(const char* what, int kind, int P, const PdxPpoBatch* b, int64_t rows, const uint8_t* active,
                     const PdxMlp* net, const float* log_std, float clip_ratio, const PdxMlpGrad* grad, float* loss,
-                    float* mu, const float* mu_ref, float* kl, void* scratch, int64_t scratch_bytes, void* stream) {
-  const bool actor = kind != kCritic;
+                    float* mu, const float* mu_ref, float* kl, const PdxMlp* dir, float scale, float damping,
+                    int64_t vec_stride, void* scratch, int64_t scratch_bytes, void* stream) {
+  const bool actor = kind != kCritic, fvp = kind == kFvp;
   const int D = b->obs_dim, h1 = net->hidden[0], h2 = net->hidden[1], O = actor ? 4 : 1;
   const int H = (h1 <= 52 && h2 <= 52) ? 52 : 64;
-  const int S = ppo_tile(D, H, false);
+  const int S = ppo_tile(D, H, fvp);
   if (S == 0) return set_error(PDX_ERR_INVALID, "pdx_ppo_*_members: obs_dim too wide for the shared-memory plan");
   const int E2 = ppo_entries(D, h1, h2, O);
   const int64_t per_cta = (int64_t)E2 * sizeof(double);
@@ -636,7 +681,10 @@ int ppo_run_members(const char* what, int kind, int P, const PdxPpoBatch* b, int
   a.n = b->n; a.ntiles = (b->n + S - 1) / S;
   a.D = D; a.h1 = h1; a.h2 = h2; a.O = O; a.E2 = E2;
   a.obs = b->obs; a.index = b->index; a.act = b->act; a.adv = b->adv; a.logp_old = b->logp_old; a.target_v = b->target_v;
-  for (int k = 0; k < 3; ++k) { a.w[k] = net->weight[k]; a.b[k] = net->bias[k]; a.dw[k] = nullptr; a.db[k] = nullptr; }
+  for (int k = 0; k < 3; ++k) {
+    a.w[k] = net->weight[k]; a.b[k] = net->bias[k];
+    a.dw[k] = fvp ? dir->weight[k] : nullptr; a.db[k] = fvp ? dir->bias[k] : nullptr;
+  }
   a.log_std = log_std;
   a.lo = (float)(1.0 - (double)clip_ratio); a.hi = (float)(1.0 + (double)clip_ratio);
   a.mu = mu; a.mu_ref = mu_ref;
@@ -644,10 +692,19 @@ int ppo_run_members(const char* what, int kind, int P, const PdxPpoBatch* b, int
   int64_t G = a.ntiles < sms ? a.ntiles : sms;
   if (G > scratch_bytes / P / per_cta) G = scratch_bytes / P / per_cta;
   const cudaStream_t st = (cudaStream_t)stream;
-  const size_t smem = ppo_smem_bytes(S, D, H, false);
-  const cudaError_t e = H == 52 ? launch_kind_members<52>(kind, grad != nullptr, a, rows, active, S, smem, (int)G, P, dev, st)
-                                : launch_kind_members<64>(kind, grad != nullptr, a, rows, active, S, smem, (int)G, P, dev, st);
+  const size_t smem = ppo_smem_bytes(S, D, H, fvp);
+  const cudaError_t e =
+      H == 52 ? launch_kind_members<52>(kind, grad != nullptr, a, rows, active, vec_stride, S, smem, (int)G, P, dev, st)
+              : launch_kind_members<64>(kind, grad != nullptr, a, rows, active, vec_stride, S, smem, (int)G, P, dev, st);
   if (e != cudaSuccess) return cuda_error(what, e);
+  if (fvp) {
+    FvpReduceArgs r;
+    r.G = (int)G; r.D = D; r.h1 = h1; r.h2 = h2; r.E2 = E2; r.part = a.part;
+    r.scale_n = (double)scale / (double)b->n; r.damping = damping;
+    for (int k = 0; k < 3; ++k) { r.dw[k] = dir->weight[k]; r.db[k] = dir->bias[k]; r.gw[k] = grad->weight[k]; r.gb[k] = grad->bias[k]; }
+    k_ppo_fvp_reduce_members<<<dim3((E2 + 255) / 256, P), 256, 0, st>>>(r, active, vec_stride);
+    return cuda_error(what, cudaGetLastError());
+  }
   ReduceArgs r;
   r.G = (int)G; r.D = D; r.h1 = h1; r.h2 = h2; r.O = O; r.E2 = E2; r.inv_n = 1.0 / (double)b->n; r.part = a.part;
   for (int k = 0; k < 3; ++k) { r.gw[k] = grad ? grad->weight[k] : nullptr; r.gb[k] = grad ? grad->bias[k] : nullptr; }
@@ -755,7 +812,8 @@ extern "C" int pdx_ppo_pi_grad_members(int32_t members, const PdxPpoBatch* batch
   if (!loss || (grad && !grad_ok(grad)) || (!mu_ref) != (!kl))
     return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_grad_members: loss is required, a gradient with all six tensors, mu_ref and kl both or neither");
   return ppo_run_members("pdx_ppo_pi_grad_members", unclipped ? kUnclipped : kClipped, members, batch, rows, active, pi,
-                         log_std, clip_ratio, grad, loss, mu, mu_ref, kl, scratch, scratch_bytes, stream);
+                         log_std, clip_ratio, grad, loss, mu, mu_ref, kl, nullptr, 0.0f, 0.0f, 0, scratch, scratch_bytes,
+                         stream);
 }
 
 extern "C" int pdx_ppo_v_grad_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
@@ -771,7 +829,44 @@ extern "C" int pdx_ppo_v_grad_members(int32_t members, const PdxPpoBatch* batch,
   if (!loss || !grad || !grad_ok(grad))
     return set_error(PDX_ERR_INVALID, "pdx_ppo_v_grad_members: loss and a gradient with all six tensors are required");
   return ppo_run_members("pdx_ppo_v_grad_members", kCritic, members, batch, rows, active, v, nullptr, 0.0f, grad, loss,
-                         nullptr, nullptr, nullptr, scratch, scratch_bytes, stream);
+                         nullptr, nullptr, nullptr, nullptr, 0.0f, 0.0f, 0, scratch, scratch_bytes, stream);
+}
+
+extern "C" int pdx_ppo_pi_fvp_members(int32_t members, const PdxPpoBatch* batch, int64_t rows, const uint8_t* active,
+                                      const PdxMlp* pi, const float* log_std, const PdxMlp* dir, float scale,
+                                      float damping, const PdxMlpGrad* out, int64_t vec_stride, void* scratch,
+                                      int64_t scratch_bytes, void* stream) {
+  using namespace pdx;
+  if (!batch_ok(batch))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: batch needs n >= 1, 1 <= obs_dim <= 384 and obs");
+  if (!members_ok(members, batch, rows))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: members must be in [1, 65535] and rows >= n (>= 1 with an index)");
+  if (!mlp_ok(pi, 4) || !log_std)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: actor must have two hidden layers of <= 64 units, 4 outputs and log_std");
+  if (!mlp_ok(dir, 4) || dir->hidden[0] != pi->hidden[0] || dir->hidden[1] != pi->hidden[1])
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: dir must have the actor's shape and all six tensors");
+  if (!out || !grad_ok(out))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: out needs all six tensors");
+  const int64_t D = batch->obs_dim, h1 = pi->hidden[0], h2 = pi->hidden[1];
+  const int64_t F = h1 * (D + 1) + h2 * (h1 + 1) + 4 * (h2 + 1);
+  if (vec_stride < F || vec_stride > INT64_MAX / 4 / members)
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: vec_stride must be >= the actor's parameter count");
+  // no member's out may overlap any member's dir: k_ppo_fvp_reduce_members reads dir while it writes out.  Tensor k
+  // of all members spans (members - 1) vec_stride floats plus its own size from member 0's address.
+  const int64_t nrows[3] = {h1, h2, 4}, ncols[3] = {D, h1, h2};
+  const uintptr_t span = 4 * (uintptr_t)(members - 1) * (uintptr_t)vec_stride;
+  for (int i = 0; i < 6; ++i)
+    for (int j = 0; j < 6; ++j) {
+      const uintptr_t o = (uintptr_t)(i < 3 ? (const void*)out->weight[i] : (const void*)out->bias[i - 3]);
+      const uintptr_t d = (uintptr_t)(j < 3 ? (const void*)dir->weight[j] : (const void*)dir->bias[j - 3]);
+      const uintptr_t no = span + 4 * (uintptr_t)(i < 3 ? nrows[i] * ncols[i] : nrows[i - 3]);
+      const uintptr_t nd = span + 4 * (uintptr_t)(j < 3 ? nrows[j] * ncols[j] : nrows[j - 3]);
+      if (o < d + nd && d < o + no) return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: out must not overlap dir over the members");
+    }
+  if (!std::isfinite(scale) || !(damping >= 0.0f) || !std::isfinite(damping))
+    return set_error(PDX_ERR_INVALID, "pdx_ppo_pi_fvp_members: scale must be finite, damping finite and >= 0");
+  return ppo_run_members("pdx_ppo_pi_fvp_members", kFvp, members, batch, rows, active, pi, log_std, 0.0f, out, nullptr,
+                         nullptr, nullptr, nullptr, dir, scale, damping, vec_stride, scratch, scratch_bytes, stream);
 }
 
 // Adam (torch.optim.Adam's foreach arithmetic) on one parameter tensor stacked over P members, numel entries per

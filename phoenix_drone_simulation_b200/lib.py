@@ -183,6 +183,9 @@ def load():
                                             C.c_void_p, C.c_int64, C.c_void_p]
     lib.pdx_ppo_v_grad_members.argtypes = [C.c_int32, P(PdxPpoBatch), C.c_int64, C.c_void_p, P(PdxMlp), P(PdxMlpGrad),
                                            C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]
+    lib.pdx_ppo_pi_fvp_members.argtypes = [C.c_int32, P(PdxPpoBatch), C.c_int64, C.c_void_p, P(PdxMlp), C.c_void_p,
+                                           P(PdxMlp), C.c_float, C.c_float, P(PdxMlpGrad), C.c_int64, C.c_void_p,
+                                           C.c_int64, C.c_void_p]
     lib.pdx_adam_members.argtypes = [C.c_int32, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                      C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_float, C.c_void_p]
     if lib.pdx_abi_version() != ABI_VERSION:
@@ -207,5 +210,5 @@ EXPORTED_SYMBOLS = [
     'pdx_policy_step_tc', 'pdx_policy_tc_pack', 'pdx_policy_tc_pack_words', 'pdx_collect', 'pdx_collect_scratch_bytes', 'pdx_oms_update',
     'pdx_evaluate', 'pdx_ppo_scratch_bytes', 'pdx_ppo_pi_grad', 'pdx_ppo_v_grad', 'pdx_ppo_pi_fvp',
     'pdx_policy_step_members', 'pdx_gae_members', 'pdx_moments_members', 'pdx_ppo_pi_grad_members',
-    'pdx_ppo_v_grad_members', 'pdx_adam_members',
+    'pdx_ppo_v_grad_members', 'pdx_adam_members', 'pdx_ppo_pi_fvp_members',
 ]

@@ -10,6 +10,10 @@ Every per-member step of ppo.PPO becomes one launch for all members: the policy 
 GAE (pdx_gae_members), the observation moments (pdx_moments_members) and, with update_kernel='cuda', the losses and
 gradients (pdx_ppo_pi_grad_members / pdx_ppo_v_grad_members).  update_kernel='torch' computes the same update with
 batched matrix products and autograd over the stacked parameters; it is the reference the kernels are tested against.
+
+PopulationNPG / PopulationTRPO do the same for npg.NPG / trpo.TRPO: one surrogate-gradient launch, one Fisher-vector
+product launch per conjugate-gradient iteration (pdx_ppo_pi_fvp_members) and one forward launch per line-search
+candidate for all members, each member following the single agent's algorithm step for step.
 """
 import ctypes as C
 import math
@@ -18,6 +22,7 @@ import time
 import torch
 
 from . import lib as _lib
+from .npg import KL_SCALE
 from .ppo import UPDATE_KERNELS, check_update_kernel_plan
 from .rollout import ActorCritic, _world
 from .vec_env import VecEnv
@@ -455,6 +460,194 @@ class PopulationPPO:
             oms.mean.copy_(mean[m]), oms.std.copy_(std[m]), oms.count.copy_(count[m])
         ac._counter, ac.env_offset = self._counter, self.env.env_offset + m * self.N
         return ac
+
+
+def conjugate_gradients_members(Avp, b, nsteps, residual_tol=1e-10, eps=1e-6):
+    """npg.conjugate_gradients for P independent systems at once: b [P, F], Avp(p, active) -> A_m p_m for every member
+    m where active[m] ([P] bool device tensor; rows of inactive members may be left unwritten).  Member m takes exactly
+    the single loop's steps (the dot products are row sums, so it agrees to rounding): a member whose residual drops
+    below residual_tol keeps that iteration's x and r and drops out, where the single loop breaks, and is inactive in
+    the later products.  One host read-back per iteration: whether any member still runs."""
+    x = torch.zeros_like(b)
+    r = b.clone()
+    p = r.clone()
+    rdotr = (r * r).sum(1)
+    running = torch.ones(b.shape[0], dtype=torch.bool, device=b.device)
+    for _ in range(nsteps):
+        z = Avp(p, running)
+        alpha = (rdotr / ((p * z).sum(1) + eps)).unsqueeze(1)
+        live = running.unsqueeze(1)
+        x = torch.where(live, x + alpha * p, x)
+        r = torch.where(live, r - alpha * z, r)
+        new_rdotr = (r * r).sum(1)
+        running = running & ~(torch.sqrt(new_rdotr) < residual_tol)
+        if not bool(running.any()):
+            break
+        mu = (new_rdotr / (rdotr + eps)).unsqueeze(1)
+        p = torch.where(running.unsqueeze(1), r + mu * p, p)
+        rdotr = torch.where(running, new_rdotr, rdotr)
+    return x
+
+
+def line_search_members(evaluate, step, theta_old, target_kl, total_steps=15, decay=0.8):
+    """trpo.line_search for P members at once.  step / theta_old [P, F]; evaluate(theta [P, F], active [P] bool device
+    tensor) -> (loss improvement [P], kl [P]) as host sequences, read for the active members only.  Candidate j moves
+    every member still searching to theta_old + decay^j step; each member accepts the first candidate whose improvement
+    is finite and >= 0 and whose kl is <= 1.5 target_kl.  Returns (step to add to theta_old [P, F], accept_step [P]):
+    accept_step j + 1 for candidate j, 0 (and a zero step) for a member that passes none.  The fraction is the single
+    search's Python float, rounded to float32 as its `frac * step` does."""
+    P = step.shape[0]
+    fracs, accept = [0.0] * P, [0] * P
+    searching = list(range(P))
+    frac = 1.0
+    for j in range(total_steps):
+        active = torch.zeros(P, dtype=torch.bool)
+        active[searching] = True
+        improve, kl = evaluate(theta_old + frac * step, active.to(step.device))
+        for m in list(searching):
+            if math.isfinite(improve[m]) and improve[m] >= 0 and kl[m] <= 1.5 * target_kl:
+                fracs[m], accept[m] = frac, j + 1
+                searching.remove(m)
+        if not searching:
+            break
+        frac *= decay
+    f = torch.tensor(fracs, dtype=step.dtype, device=step.device).unsqueeze(1)
+    return f * step, accept
+
+
+class PopulationNPG(PopulationPPO):
+    """npg.NPG for a population: PopulationPPO's rollout, value phase and running statistics, and per member exactly
+    npg.NPG.update_pi's conjugate-gradient policy step (surrogate gradient g on the full batch, x = CG(F, -g) with the
+    Fisher-vector product on every 4th member-local row, step = sqrt(2 target_kl / x^T F x) x).  The actor has no
+    optimiser and no learning-rate schedule.  update_kernel='cuda': the gradient is one pdx_ppo_pi_grad_members launch
+    and every Fisher-vector product one pdx_ppo_pi_fvp_members launch on the flat [P, F] CG vectors; 'torch': autograd,
+    the product being the reference's double backward over the stacked parameters."""
+
+    def __init__(self, env_id, cg_iters=10, cg_damping=0.1, target_kl=0.01, **kwargs):
+        super().__init__(env_id, target_kl=target_kl, **kwargs)
+        self.clip_ratio = None                               # the unclipped surrogate
+        self.cg_iters, self.cg_damping = cg_iters, cg_damping
+        self.pi_opt = None                                   # npg.py: no pi optimiser step
+        self.step_info = {}
+
+    def update(self, data):
+        info = super().update(data)
+        info.update(self.step_info)
+        return info
+
+    # ---- flat [P, F] parameter vectors, per member in the order of ppo.pi_net_params ----------------------------------
+    def _flat_views(self, flat):
+        out, k = [], 0
+        for p_ in self.pi_params:
+            n = p_[0].numel()
+            out.append(flat[:, k:k + n].view(p_.shape))
+            k += n
+        assert k == flat.shape[1], (k, flat.shape)
+        return out
+
+    def _flat_params(self):
+        return torch.cat([p_.detach().reshape(self.P, -1) for p_ in self.pi_params], 1)
+
+    @torch.no_grad()
+    def _set_flat_params(self, flat):
+        for p_, v in zip(self.pi_params, self._flat_views(flat)):
+            p_.copy_(v)
+
+    # ---- the pieces of the policy step ----------------------------------------------------------------------------------
+    def _surrogate_grad(self, obs, act, adv, logp_old):
+        """(loss [P], flat gradient [P, F]) of -(r A).mean() on every member's full batch."""
+        if self.update_kernel == 'cuda':
+            loss, _ = self.pi_loss_and_grad(obs, act, adv, logp_old)
+        else:
+            for p_ in self.pi_params:
+                p_.grad = None
+            loss = self._surrogate(obs, act, adv, logp_old)
+            loss.sum().backward()
+        return loss.detach(), torch.cat([p_.grad.reshape(self.P, -1) for p_ in self.pi_params], 1)
+
+    def _surrogate(self, obs, act, adv, logp_old):
+        _, _, logp = self._log_prob(obs, act)
+        loss = -(torch.exp(logp - logp_old) * adv).mean(1)
+        if self.entropy_coef:
+            loss = loss - self._entropy_term()
+        return loss
+
+    def _fvp(self, obs, idx, v, active=None):
+        """F_m v_m + cg_damping v_m of every member (npg.py Fvp with npg.KL_SCALE), v [P, F]; with update_kernel='cuda'
+        the rows of members inactive in `active` are not written."""
+        if self.update_kernel == 'cuda':
+            out = torch.empty_like(v)
+            b = self._batch(obs, idx)
+            d, g = _lib.PdxMlp(), _lib.PdxMlpGrad()
+            d.hidden[0], d.hidden[1], d.n_out = self.pi_hidden[0], self.pi_hidden[1], 4
+            for k, (dv, ov) in enumerate(zip(self._flat_views(v), self._flat_views(out))):
+                getattr(d, ('weight', 'bias')[k % 2])[k // 2] = dv.data_ptr()
+                getattr(g, ('weight', 'bias')[k % 2])[k // 2] = ov.data_ptr()
+            scratch = self._scratch(self.pi_params, 4)
+            p = lambda t: C.c_void_p(t.data_ptr()) if t is not None else None
+            _lib.check(_lib.load().pdx_ppo_pi_fvp_members(
+                self.P, C.byref(b), obs.shape[1], p(active), C.byref(self._mlp(self.pi_params, 4)), p(self.log_std),
+                C.byref(d), KL_SCALE, float(self.cg_damping), C.byref(g), v.shape[1], p(scratch), scratch.numel(),
+                self._stream()))
+            return out
+        o = obs[torch.arange(self.P, device=obs.device).unsqueeze(1), idx]
+        mu = self._forward(self.pi_params, o, torch.relu)
+        std = torch.exp(self.log_std).unsqueeze(1).to(mu.dtype)
+        q_dist = torch.distributions.Normal(mu, std)
+        with torch.no_grad():
+            p_dist = torch.distributions.Normal(mu.detach(), std)
+        # the per-member KL means summed: the Hessian is block-diagonal over the members
+        kl = (torch.distributions.kl.kl_divergence(p_dist, q_dist).mean((1, 2)) * (KL_SCALE * mu.shape[-1])).sum()
+        grads = torch.autograd.grad(kl, self.pi_params, create_graph=True)
+        flat_grad_kl = torch.cat([g.reshape(self.P, -1) for g in grads], 1)
+        grads = torch.autograd.grad((flat_grad_kl * v).sum(), self.pi_params)
+        return torch.cat([g.contiguous().reshape(self.P, -1) for g in grads], 1) + v * self.cg_damping
+
+    def _loss_kl(self, obs, act, adv, logp_old, mu_old, active=None):
+        """Forward only: (surrogate loss [P], reference-normalised KL to mu_old [P]) as device tensors; with
+        update_kernel='cuda' the entries of members inactive in `active` are not written."""
+        if self.update_kernel == 'cuda':
+            mu = torch.empty_like(mu_old)
+            loss, kl = self.pi_loss_and_grad(obs, act, adv, logp_old, grad=False, mu=mu, mu_ref=mu_old, active=active)
+            return loss, kl * KL_SCALE
+        with torch.no_grad():
+            return self._surrogate(obs, act, adv, logp_old), self._pi_forward(obs, act, adv, logp_old, mu_ref=mu_old)[1] * KL_SCALE
+
+    def search_step_size(self, step, theta_old, evaluate):
+        """NPG takes every member's whole natural-gradient step.  Returns (step to add [P, F], accept_step [P])."""
+        return step, [1] * self.P
+
+    def update_pi(self, obs, act, adv, logp_old):
+        """npg.py update_policy_net per member.  Returns (loss after the step [P], zeros, kl after the step [P])."""
+        P, n = obs.shape[:2]
+        fvp_idx = torch.arange(0, n, 4, device=obs.device).expand(P, -1).contiguous()
+        mu_old = self._pi_forward(obs, act, adv, logp_old)[0]
+        theta_old = self._flat_params()
+        loss_before, g = self._surrogate_grad(obs, act, adv, logp_old)
+        x = conjugate_gradients_members(lambda v, active: self._fvp(obs, fvp_idx, v, active), -g, self.cg_iters)
+        xHx = (x * self._fvp(obs, fvp_idx, x)).sum(1)
+        step = torch.sqrt(2 * self.target_kl / (xHx + 1e-8)).unsqueeze(1) * x
+
+        def evaluate(theta, active):
+            """(loss improvement [P], kl [P]) of every member's actor at theta, as host lists."""
+            self._set_flat_params(theta)
+            loss, kl = self._loss_kl(obs, act, adv, logp_old, mu_old, active)
+            t = torch.stack([loss_before - loss, kl]).tolist()
+            return t[0], t[1]
+
+        final_step, accept = self.search_step_size(step, theta_old, evaluate)
+        self._set_flat_params(theta_old + final_step)
+        loss, kl = self._loss_kl(obs, act, adv, logp_old, mu_old)
+        self.step_info = {'accept_step': accept, 'xHx': xHx.tolist()}
+        return loss, [0] * P, kl.tolist()
+
+
+class PopulationTRPO(PopulationNPG):
+    """trpo.TRPO for a population: each member's NPG step under trpo.line_search, batched (line_search_members): one
+    forward-only pdx_ppo_pi_grad_members launch per candidate for the members still searching."""
+
+    def search_step_size(self, step, theta_old, evaluate):
+        return line_search_members(evaluate, step, theta_old, self.target_kl)
 
 
 def learn(env_id, **kwargs):
